@@ -3,7 +3,7 @@
 search over the Tianchi-news-shaped catalog (364,047 items x 250-d fp32), 50,000 user queries
 per step (the search Retrieval.py:32 performs per user, in its north-star IndexFlatIP form).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 * our arm: one process per GPU (torchrun for N > 1). N = 1: the whole catalog on one B200.
   N > 1 ("strong" scaling: the job is fixed, value = queries of one step x steps /
@@ -196,6 +196,18 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons), "source": "nvidia-smi -lms 100"}
 
 
+def dump_outputs(path, arrays, rank=0, world=1):
+    """--dump-outputs: the arrays the last timed step returned, as DIR/<name>.npy; scores stay
+    float32, ids and query rows become float64 (exact below 2**53). The inputs are seeded, so two
+    builds run with the same arguments can be compared array for array. With N > 1 GPUs every rank
+    writes the rows it owns, as <name>.rank<r>.npy."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        np.save(os.path.join(path, (name if world == 1 else f"{name}.rank{rank}") + ".npy"), a)
+
+
 def use_all_host_threads() -> int:
     """torchrun exports OMP_NUM_THREADS=1; the CPU legs must use every host core they can."""
     cores = len(os.sched_getaffinity(0))
@@ -251,8 +263,10 @@ def run_reference(args):
         fo.knn_fast(xq[:n], xb, K, 0)
     t0 = time.perf_counter()
     for _ in range(steps):
-        fo.knn_fast(xq[:n], xb, K, 0)
+        Dr, Ir = fo.knn_fast(xq[:n], xb, K, 0)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"D": Dr, "I": Ir})
     v = n * steps / dt
     sample = (f"each step = first {n} of {NQ} queries against the full catalog; faiss is not installable here, "
               f"this is the faiss-equivalent oracle port on all {cores} host threads")
@@ -346,7 +360,7 @@ def run_ours(args):
             dist.barrier()
             torch.cuda.synchronize()
 
-    def measure(run, sampler=None):
+    def measure(run, sampler=None, keep_outputs=False):
         for _ in range(args.warmup):
             run["step_device"]()
         sync_all()
@@ -357,8 +371,11 @@ def run_ours(args):
         n0 = _lib.launch_count()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
-        for _ in range(args.steps):
+        # results are dropped at once so that every step reuses the same output blocks; only the
+        # last step's are kept (for --dump-outputs)
+        for _ in range(args.steps - 1):
             run["step_device"]()
+        last = run["step_device"]()
         ev1.record()
         sync_all()
         ms = ev0.elapsed_time(ev1)
@@ -366,6 +383,13 @@ def run_ours(args):
         kern_ms, kern_n = _lib.profile_read()
         _lib.profile_enable(False)
         clocks = sampler.stop() if sampler is not None else None
+        outputs = None
+        if keep_outputs:  # copied before the end-to-end leg reuses the index
+            outputs = {"D": last[0].cpu().numpy(), "I": last[1].cpu().numpy()}
+            if world > 1:  # the rows of the batch this rank returns, as query indices
+                spans = last[2] if len(last) > 2 else [(0, run["hi"] - run["lo"])]
+                rows = [np.arange(a, b) for a, b in spans] or [np.empty(0, np.int64)]
+                outputs["query_rows"] = run["lo"] + np.concatenate(rows)
         t = torch.tensor([ms], device="cuda")
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -408,7 +432,7 @@ def run_ours(args):
                   "exact_ordered": f[3] / max(1.0, f[1]), "max_rel_score_err": float(worst.item()),
                   "checked_on": "every rank, rows it owns, vs the oracle port"}
         return dict(ms=ms, launches=launches, kern_ms=kern_ms, kern_n=kern_n, clocks=clocks,
-                    e2e_s=float(t.item()), parity=parity)
+                    e2e_s=float(t.item()), parity=parity, outputs=outputs)
 
     def describe(run):
         if world == 1:
@@ -428,7 +452,9 @@ def run_ours(args):
     # N > 1 (N = 2: the box is one group); a 10M-row catalog -> one group of N shards.
     S_main = args.shards if args.shards > 0 else default_shards(world, NB)
     run = build(S_main)
-    res = measure(run, ClockSampler(local) if rank == 0 else None)
+    res = measure(run, ClockSampler(local) if rank == 0 else None, keep_outputs=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res["outputs"], rank, world)
     ms, launches, kern_ms, kern_n, clocks, e2e_s = (res[k] for k in ("ms", "launches", "kern_ms", "kern_n", "clocks", "e2e_s"))
     main_desc = describe(run)
     run = {k: v for k, v in run.items() if not callable(v)}  # drop the index (frees HBM)
@@ -538,7 +564,7 @@ class _StdoutGuard:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--shards", type=int, default=0,
@@ -555,7 +581,12 @@ def main():
     ap.add_argument("--path", default="auto", choices=["auto", "tc", "tc1", "tc16"],
                     help="auto/tc16 = fp16 filter + exact fp32 refine (default), tc1 = the same with the 1xTF32 "
                          "filter, tc = 3xTF32")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the (D, I) results of the last timed step as DIR/<name>.npy "
+                         "(30 MB for the default job)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.out = _StdoutGuard()
     if args.impl == "reference":

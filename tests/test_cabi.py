@@ -181,14 +181,12 @@ def test_flat_planner_invariants_and_known_plans():
 
 def test_reference_script_fixtures_are_byte_identical():
     """tests/fixtures/reference_scripts holds test DATA: copies of three reference scripts that the
-    GPU suite runs unmodified. They must match the recorded sha256 and, where /root/reference is
-    present (this container), the originals."""
+    GPU suite runs unmodified. They must match the sha256 and size recorded from the originals."""
     import hashlib
     import json
     d = os.path.join(ROOT, "tests", "fixtures", "reference_scripts")
     prov = json.load(open(os.path.join(d, "PROVENANCE.json")))
+    assert sorted(prov["files"]) == ["Retrieval.py", "finialize_retrieval.py", "utils.py"]
     for name, meta in prov["files"].items():
         b = open(os.path.join(d, name), "rb").read()
         assert hashlib.sha256(b).hexdigest() == meta["sha256"] and len(b) == meta["bytes"]
-        if os.path.exists(meta["source"]):
-            assert open(meta["source"], "rb").read() == b

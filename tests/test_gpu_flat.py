@@ -1,15 +1,13 @@
 """GPU parity tests of the exact top-k path (K0 pack, K2 distance+selection, select) against the
 oracle, through the faiss-compatible surface and the C-ABI. Bit-exact ids outside sub-1e-5 gaps,
 scores within 1e-4 relative (tolerances of BASELINE.json's north_star, see parity.py)."""
-import os
-
 import numpy as np
 import pytest
 
+import golden_inputs
 from newsrecommend_b200.parity import compare_topk
 
 pytestmark = pytest.mark.gpu
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 PATHS = {"tc": 2, "simt": 1, "tc1": 3, "tc16": 4, "auto": 0}
 
 
@@ -77,7 +75,7 @@ def test_pack_rows_h16_scales(nf):
 @pytest.mark.parametrize("path", ["tc", "simt", "tc1", "tc16", "auto"])
 @pytest.mark.parametrize("metric", [0, 1])
 def test_golden_fixture(nf, path, metric):
-    g = np.load(os.path.join(GOLDEN, "flat_small.npz"))
+    g = golden_inputs.load("flat_small")
     D, I = _search(nf, g["xb"], g["xq"], 10, metric, path)
     assert D.dtype == np.float32 and I.dtype == np.int64 and D.shape == (48, 10)
     rep = compare_topk(D, I, g[f"D{metric}"], g[f"I{metric}"], metric)

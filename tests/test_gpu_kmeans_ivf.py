@@ -2,15 +2,13 @@
 search (K3) against the oracle. k-means is chaotic under ulp-level changes (SURVEY Appendix
 B-E5), so bit-level parity is checked teacher-forced per iteration; free-running runs are
 compared on their objective."""
-import os
-
 import numpy as np
 import pytest
 
+import golden_inputs
 from newsrecommend_b200.parity import compare_topk
 
 pytestmark = pytest.mark.gpu
-GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def test_kmeans_update_matches_sequential_fp32(nf, oracle):
@@ -52,7 +50,7 @@ def test_kmeans_teacher_forced_against_golden(nf):
     """Each recorded oracle iteration: same input centroids -> same assignments (modulo the gap
     rule) and new centroids within 1e-6 relative."""
     import torch
-    g = np.load(os.path.join(GOLDEN, "kmeans_small.npz"))
+    g = golden_inputs.load("kmeans_small")
     x = g["xs"]  # the rows the oracle iterated on (rand_perm subsample of g["x"])
     assert np.array_equal(x, g["x"][nf.rand_perm(g["x"].shape[0], 1234)[: x.shape[0]]])
     p = nf.PackedMatrix.from_tensor(torch.from_numpy(x).cuda())
@@ -280,8 +278,7 @@ def test_ivf_lists_split_into_several_units(nf, oracle, path, monkeypatch):
 def test_ivf_golden_fixture(nf, metric, path):
     """tests/golden/ivf_small.npz (written by the oracle): with the fixture's centroids in the coarse
     quantizer the GPU index builds lists of the same sizes and returns the fixture's (D, I)."""
-    import os
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "ivf_small.npz"))
+    g = golden_inputs.load("ivf_small")
     quant = nf.IndexFlatIP(64) if metric == 0 else nf.IndexFlatL2(64)
     quant.add(g[f"cent{metric}"])
     ivf = nf.IndexIVFFlat(quant, 64, 16, metric)

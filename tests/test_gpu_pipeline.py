@@ -37,14 +37,14 @@ def test_batched_stage_equals_reference_script(tmp_path):
     out = pipeline.retrieve_candidates(aids, emb, prof, num_clusters=300, niter=80)
     off, cand = out["offsets"].cpu().numpy(), out["candidates"].cpu().numpy()
     assert off[-1] == cand.shape[0] and int(out["list_sizes"].sum()) == len(ids)
-    ref = "/root/reference/Retrieval.py"
-    if os.path.exists(ref):
-        env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "shim") + os.pathsep + ROOT)
-        subprocess.check_call([sys.executable, ref], cwd=tmp_path, env=env)
-        u2, off2, cand2 = pipeline.load_recommendations(news / "test_user_recommendations.npy")
-        assert np.array_equal(u2, uids) and np.array_equal(off2, off) and np.array_equal(cand2, cand)
-    # The GPU box has no /root/reference, so the same call sequence the script makes
-    # (Retrieval.py:11-34) is replayed here against the shim, per-user loop included.
+    # the unmodified script (tests/fixtures/reference_scripts, sha256-pinned) with `import faiss` -> the shim
+    ref = os.path.join(ROOT, "tests", "fixtures", "reference_scripts", "Retrieval.py")
+    env = dict(os.environ, PYTHONPATH=os.path.join(ROOT, "shim") + os.pathsep + ROOT)
+    subprocess.check_call([sys.executable, ref], cwd=tmp_path, env=env)
+    u2, off2, cand2 = pipeline.load_recommendations(news / "test_user_recommendations.npy")
+    assert np.array_equal(u2, uids) and np.array_equal(off2, off) and np.array_equal(cand2, cand)
+    # The same call sequence the script makes (Retrieval.py:11-34), replayed in this process against
+    # the shim, per-user loop included.
     sys.path.insert(0, os.path.join(ROOT, "shim"))
     try:
         import faiss

@@ -5,6 +5,7 @@ import os
 import numpy as np
 import pytest
 
+import golden_inputs
 from newsrecommend_b200.parity import compare_topk
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
@@ -166,7 +167,7 @@ def test_ivf_full_probe_equals_flat(oracle, metric):
 
 
 def test_golden_flat(oracle):
-    g = np.load(os.path.join(GOLDEN, "flat_small.npz"))
+    g = golden_inputs.load("flat_small")
     for metric in (0, 1):
         D, I = oracle.knn(g["xq"], g["xb"], 10, metric)
         assert np.array_equal(I, g[f"I{metric}"])
@@ -178,7 +179,7 @@ def test_golden_flat(oracle):
 def test_golden_ivf(oracle):
     """IVF-Flat fixture: the oracle retrains to the same centroids (deterministic k-means: mt19937
     subsample / init, sequential fp32 sums), builds the same lists and returns the same (D, I)."""
-    g = np.load(os.path.join(GOLDEN, "ivf_small.npz"))
+    g = golden_inputs.load("ivf_small")
     for metric, qcls in ((0, oracle.IndexFlatIP), (1, oracle.IndexFlatL2)):
         quant = qcls(64)
         ivf = oracle.IndexIVFFlat(quant, 64, 16, metric)
@@ -216,7 +217,7 @@ GOLD = os.path.join(os.path.dirname(__file__), "golden")
 def test_golden_flat_against_torch_mkl_and_sklearn(metric):
     import torch
     from newsrecommend_b200.parity import compare_topk
-    g = np.load(os.path.join(GOLD, "flat_small.npz"))
+    g = golden_inputs.load("flat_small")
     xb, xq = torch.from_numpy(g["xb"]), torch.from_numpy(g["xq"])
     ip = xq @ xb.T  # MKL sgemm: a different BLAS from the OpenBLAS behind the oracle's numpy blocks
     if metric == 0:
@@ -256,7 +257,7 @@ def test_golden_kmeans_iteration_against_sklearn_lloyd():
     """One teacher-forced Lloyd iteration of the golden k-means trace reproduced by scikit-learn
     (init = the recorded input centroids, max_iter = 1): same assignment, same means."""
     from sklearn.cluster import KMeans
-    g = np.load(os.path.join(GOLD, "kmeans_small.npz"))
+    g = golden_inputs.load("kmeans_small")
     xs = g["xs"].astype(np.float64)
     for it in range(g["cin"].shape[0]):
         cin = g["cin"][it].astype(np.float64)
@@ -280,7 +281,7 @@ def test_golden_ivf_against_fp64_rederivation(metric):
     """IndexIVFFlat semantics re-derived in vectorised fp64 numpy from the fixture's centroids:
     items go to their nearest centroid, a query scans the nprobe = 4 best lists, top-10 by score."""
     from newsrecommend_b200.parity import compare_topk
-    g = np.load(os.path.join(GOLD, "ivf_small.npz"))
+    g = golden_inputs.load("ivf_small")
     xb, xq, cent = g["xb"].astype(np.float64), g["xq"].astype(np.float64), g[f"cent{metric}"].astype(np.float64)
 
     def coarse(x):  # larger is better

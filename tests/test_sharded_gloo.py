@@ -136,16 +136,34 @@ def test_chunk_ownership_partitions_the_batch():
                 assert sum(c1 - c0 for c0, c1, _ in chunk_slices(nq, world, chunk)) == nq
 
 
-def test_bench_default_layout():
-    """bench.py's default multi-GPU layout: shards of >= 180,000 rows, at least 2 per replica group, a
-    divisor of the world size (config 1 -> groups of 2; a 10M-row catalog -> one group of N)."""
+def _bench():
     import importlib.util
-    import os
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     spec = importlib.util.spec_from_file_location("_bench", os.path.join(root, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_default_layout():
+    """bench.py's default multi-GPU layout: shards of >= 180,000 rows, at least 2 per replica group, a
+    divisor of the world size (config 1 -> groups of 2; a 10M-row catalog -> one group of N)."""
+    bench = _bench()
     assert [bench.default_shards(w, 364_047) for w in (1, 2, 4, 8)] == [1, 2, 2, 2]
     assert [bench.default_shards(w, 10_000_000) for w in (1, 2, 4, 8)] == [1, 2, 4, 8]
     assert bench.default_shards(3, 364_047) == 1 and bench.default_shards(6, 364_047) == 2
     assert bench.default_shards(8, 1_000) == 2
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: float32 scores stay float32, int64 ids become float64 with the same
+    values, one <name>.npy per array (per rank with N > 1)."""
+    bench = _bench()
+    D = np.arange(6, dtype=np.float32).reshape(2, 3) / 7
+    I = np.array([[364_046, 0, -1], [5, 4, 3]], dtype=np.int64)
+    bench.dump_outputs(str(tmp_path / "one"), {"D": D, "I": I})
+    d, i = np.load(tmp_path / "one" / "D.npy"), np.load(tmp_path / "one" / "I.npy")
+    assert d.dtype == np.float32 and np.array_equal(d, D)
+    assert i.dtype == np.float64 and np.array_equal(i.astype(np.int64), I)
+    bench.dump_outputs(str(tmp_path / "two"), {"D": D, "I": I, "query_rows": np.arange(2)}, rank=1, world=2)
+    assert sorted(os.listdir(tmp_path / "two")) == ["D.rank1.npy", "I.rank1.npy", "query_rows.rank1.npy"]
