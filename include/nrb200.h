@@ -74,9 +74,6 @@ int nrb_device_info(int* sm_count, int* cc_major, int* cc_minor);
 /* Number of kernel launches issued by this library since load (bench.py's gpu_launches). */
 int64_t nrb_launch_count(void);
 
-/* Selects the tcgen05 kernel variant: 2 = CTA pairs (cta_group::2, default), 1 = single CTA.
- * Same results; kept for cross-checks and A/B timing. Also settable with NRB_TC_VARIANT=1. */
-int nrb_set_tc_variant(int v);
 /* Device-side timing of the dominant (distance + selection) kernel: when enabled, every such
  * launch is bracketed by CUDA events on its stream; nrb_profile_read() synchronises, returns the
  * summed milliseconds and the launch count since the last read, and resets. */
@@ -122,20 +119,6 @@ size_t nrb_search_flat_workspace(int64_t nq, int64_t nb, int32_t k, int32_t kp);
 int nrb_search_flat(const nrb_matrix* q, const nrb_matrix* b, int32_t metric, int32_t k,
                     int64_t id_base, float* D, int64_t* I, void* workspace,
                     size_t workspace_bytes, int32_t path, void* stream);
-
-/* nrb_search_flat with per-query bounds the caller already knows: seed_kth f32[nq] (device) holds,
- * in D's domain (a score for IP, a squared distance for L2), a value that at least k items of the
- * WHOLE catalog the caller is searching reach -- e.g. the k-th best over a row sample, or over
- * another shard. The kernel's shared running bounds start there instead of at -inf, so every unit
- * skips the append-heavy warm-up of its first tiles; +-FLT_MAX / NaN = no bound for that query.
- * Results: every item of b that scores at least the bound is found exactly as nrb_search_flat finds
- * it; a query may come back with fewer than k results from THIS matrix (the rest padded with -1)
- * when the bound came from elsewhere -- the k-way merge over the shards restores the global top-k
- * (sharded.py). Honoured by the filter paths (their margin absorbs the estimate error of the bounding
- * item); the 3xTF32 paths ignore it. No reference analogue: faiss keeps one heap per query. */
-int nrb_search_flat_seeded(const nrb_matrix* q, const nrb_matrix* b, int32_t metric, int32_t k,
-                           int64_t id_base, float* D, int64_t* I, void* workspace,
-                           size_t workspace_bytes, int32_t path, const float* seed_kth, void* stream);
 
 /* Queries that NRB_PATH_TC1 had to recompute with the 3xTF32 kernel since the library was loaded
  * (candidate slots exhausted inside the error margin, or an estimate outside its bound). */

@@ -22,9 +22,9 @@ SMALL_MAX_NQ = 64  # NRB_SMALL_MAX_NQ
 # every symbol include/nrb200.h declares (tests check the library exports all of them)
 SYMBOLS = [
     "nrb_version", "nrb_last_error", "nrb_device_info", "nrb_launch_count",
-    "nrb_profile_enable", "nrb_profile_read", "nrb_set_tc_variant",
+    "nrb_profile_enable", "nrb_profile_read",
     "nrb_pack_rows", "nrb_pack_rows_h16", "nrb_gather_rows", "nrb_gather_i64", "nrb_normalize_l2",
-    "nrb_search_flat_workspace", "nrb_search_flat", "nrb_search_flat_seeded", "nrb_fallback_query_count", "nrb_plan_flat_describe",
+    "nrb_search_flat_workspace", "nrb_search_flat", "nrb_fallback_query_count", "nrb_plan_flat_describe",
     "nrb_kmeans_update_workspace", "nrb_kmeans_update", "nrb_kmeans_partial_sums", "nrb_kmeans_means",
     "nrb_rand_perm_host", "nrb_split_clusters_host", "nrb_split_clusters",
     "nrb_kmeans_train_workspace", "nrb_kmeans_train",
@@ -59,7 +59,6 @@ lib.nrb_last_error.argtypes = [C.c_char_p, C.c_int]
 lib.nrb_device_info.argtypes = [C.POINTER(C.c_int)] * 3
 lib.nrb_launch_count.restype = _i64
 lib.nrb_profile_enable.argtypes = [C.c_int]
-lib.nrb_set_tc_variant.argtypes = [C.c_int]
 lib.nrb_profile_read.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_int)]
 lib.nrb_pack_rows.argtypes = [_vp, _i64, _i32, _i64, _i32, _vp, _vp, _vp, _vp, _vp]
 lib.nrb_pack_rows_h16.argtypes = [_vp, _i64, _i32, _i64, _i32, C.c_float, _vp, _vp, _vp]
@@ -69,7 +68,6 @@ lib.nrb_normalize_l2.argtypes = [_vp, _i64, _i32, _i64, _vp]
 lib.nrb_search_flat_workspace.restype = _sz
 lib.nrb_search_flat_workspace.argtypes = [_i64, _i64, _i32, _i32]
 lib.nrb_search_flat.argtypes = [_mp, _mp, _i32, _i32, _i64, _vp, _vp, _vp, _sz, _i32, _vp]
-lib.nrb_search_flat_seeded.argtypes = [_mp, _mp, _i32, _i32, _i64, _vp, _vp, _vp, _sz, _i32, _vp, _vp]
 lib.nrb_fallback_query_count.restype = _i64
 lib.nrb_plan_flat_describe.argtypes = [_i64, _i64, _i32, _i32, _vp]
 lib.nrb_kmeans_update_workspace.restype = _sz

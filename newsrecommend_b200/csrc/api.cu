@@ -108,16 +108,15 @@ static FlatPlan plan_flat(int64_t nq, int64_t nb, int k, int path) {
     if (nbt < 1) nbt = 1;
     p.full_pairs = (p.npairs / C) * C;
     p.tail_pairs = p.npairs - p.full_pairs;
+    // cost of a plan = waves x (chunk length + per-unit overhead), in catalogs per CTA pair (or CTA);
+    // a unit costs about 200 tiles of MMA time on top of its item rows (query-tile load, the
+    // append-heavy threshold warm-up and its prunes, 32 final sorts per warp; measured by sweeping
+    // that overhead on config 1), which is what stops small batches from being cut into dozens of
+    // slivers
+    const double ov = 200.0 / nbt;
     int best = 1;
     if (p.tail_pairs > 0) {
         int max_split = nbt < 64 ? nbt : 64;
-        // cost of a plan = waves x (chunk length + per-unit overhead), in catalogs per CTA pair;
-        // a unit costs about 200 tiles of MMA time on top of its item rows (query-tile load, the
-        // append-heavy threshold warm-up and its prunes, 32 final sorts per warp; measured by
-        // sweeping NRB_FLAT_OV_TILES on config 1), which is what stops small batches from being
-        // cut into dozens of slivers
-        static const double ov_tiles = getenv("NRB_FLAT_OV_TILES") ? atof(getenv("NRB_FLAT_OV_TILES")) : 200.0;
-        const double ov = ov_tiles / nbt;
         double best_cost = 1e30;
         for (int s = 1; s <= max_split; s++) {
             const double waves = (double)(((int64_t)p.tail_pairs * s + C - 1) / C);
@@ -134,10 +133,8 @@ static FlatPlan plan_flat(int64_t nq, int64_t nb, int k, int path) {
     // 49 tiles x 3 chunks = 147 units where 25 pairs stop at 2 chunks. CTA pairs halve the L2
     // traffic per unit of work, so they stay unless the single-CTA plan is clearly shorter.
     // (catalogs of one tile -- coarse quantizers -- go to the CTA-pair short-unit kernel instead)
-    if (path == NRB_PATH_TC16 && p.full_pairs == 0 && p.nqt <= sm_count() && nb > 256 && !getenv("NRB_NO_SINGLE_CTA")) {
+    if (path == NRB_PATH_TC16 && p.full_pairs == 0 && p.nqt <= sm_count() && nb > 256) {
         const int C1 = sm_count();
-        static const double ov_tiles1 = getenv("NRB_FLAT_OV_TILES") ? atof(getenv("NRB_FLAT_OV_TILES")) : 200.0;
-        const double ov = ov_tiles1 / nbt;
         const int max_split = nbt < 64 ? nbt : 64;
         const double pair_cost = (double)(((int64_t)p.tail_pairs * best + C - 1) / C) * (1.0 / best + ov);
         int best1 = 1;
@@ -404,7 +401,7 @@ static IvfPlan plan_ivf(int64_t nq, int nprobe, int nlist, int max_list_len, int
     }
     p.S = nprobe * p.maxsplit * p.wgs;
     // the SIMT kernels keep no shared running bounds: one phase
-    p.nph = (nprobe > 1 && path != NRB_PATH_SIMT && !getenv("NRB_IVF_ONE_PHASE")) ? 2 : 1;
+    p.nph = (nprobe > 1 && path != NRB_PATH_SIMT) ? 2 : 1;
     p.total_units = 0;
     for (int i = 0; i < p.nph; i++) {
         IvfPhase& f = p.ph[i];
@@ -522,12 +519,6 @@ extern "C" int nrb_device_info(int* sms, int* cc_major, int* cc_minor) {
     return NRB_OK;
 }
 
-extern "C" int nrb_set_tc_variant(int v) {
-    NRB_REQUIRE(v == 1 || v == 2, "set_tc_variant: 1 (single CTA) or 2 (CTA pair)");
-    tc_set_variant(v);
-    return NRB_OK;
-}
-
 extern "C" int nrb_profile_enable(int on) {
     g_profile = on != 0;
     return NRB_OK;
@@ -570,19 +561,9 @@ extern "C" size_t nrb_search_flat_workspace(int64_t nq, int64_t nb, int32_t k, i
 
 namespace nrb {
 
-// gthr[i] = ordered-uint key of seed[i] (a score for IP, a squared distance for L2): a lower bound of
-// query i's k-th best key that the caller already knows; +-FLT_MAX / non-finite = no bound.
-__global__ void seed_bounds_kernel(const float* __restrict__ seed, int64_t nq, int l2, unsigned* __restrict__ gthr) {
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nq; i += (int64_t)gridDim.x * blockDim.x) {
-        const float v = seed[i];
-        const bool ok = fabsf(v) < 3.0e38f;  // false for NaN, inf and the FLT_MAX padding of a short result row
-        gthr[i] = ok ? ordered_u32(l2 ? -v : v) : 0u;
-    }
-}
-
 static int search_flat_impl(const nrb_matrix* q, const nrb_matrix* b, int metric, int k, int64_t id_base,
                             float* D, int64_t* I, void* workspace, size_t workspace_bytes, int path,
-                            cudaStream_t st, const float* seed_kth = nullptr) {
+                            cudaStream_t st) {
     if (path == NRB_PATH_AUTO)
         path = tc16_eligible(q, b, k) ? NRB_PATH_TC16 : tc1_eligible(q, b, k) ? NRB_PATH_TC1 : NRB_PATH_TC;
     if (path == NRB_PATH_TC1 && !tc1_eligible(q, b, k)) {
@@ -610,16 +591,7 @@ static int search_flat_impl(const nrb_matrix* q, const nrb_matrix* b, int metric
         rc = launch_fill_flat_units(w.units, w.n_units, w.src, q->n, b->n, p.nqt, p.full_pairs, p.tail_pairs, p.tsplit,
                                     p.chunk_rows, p.wgs, st);
     if (rc) return rc;
-    // Seeded bounds are honoured by the filter paths only: their margin absorbs the difference between
-    // the caller's exact score of the bounding item and this kernel's estimate of the same item; the
-    // 3xTF32 kernels compare with no margin and start cold.
-    const bool seeded = seed_kth && filt && w.gthr;
-    if (seeded) {
-        int64_t blocks = (q->n + 255) / 256;
-        if (blocks > 148 * 8) blocks = 148 * 8;
-        seed_bounds_kernel<<<(unsigned)blocks, 256, 0, st>>>(seed_kth, q->n, metric == NRB_METRIC_L2 ? 1 : 0, w.gthr);
-        NRB_LAUNCH_CHECK();
-    } else if (w.gthr) {
+    if (w.gthr) {
         NRB_CUDA_CHECK(cudaMemsetAsync(w.gthr, 0, (size_t)q->n * sizeof(unsigned), st));
     }
     if (!filt) {
@@ -642,8 +614,8 @@ static int search_flat_impl(const nrb_matrix* q, const nrb_matrix* b, int metric
         ProfScope prof(st);
         rc = launch_topk_tc1_dev(q, b, w.units, w.n_units, p.grid, metric, k, pw, 2.f * eps_xmax, w.part_key,
                                  w.part_idx, w.part_cnt, w.flags, w.scratch, w.scratch_bytes, w.gthr, nullptr, 1,
-                                 path == NRB_PATH_TC16, p.single, (!p.single && b->n <= 256) ? 1 : 0, st,
-                                 seeded ? 1 : 0);  // <= 256 items: every unit is one tile (coarse search, nearest centroid) -> the short-unit kernel
+                                 path == NRB_PATH_TC16, p.single, (!p.single && b->n <= 256) ? 1 : 0,
+                                 st);  // <= 256 items: every unit is one tile (coarse search, nearest centroid) -> the short-unit kernel
     }
     if (rc) return rc;
     if ((rc = launch_gather_refine(w.part_key, w.part_idx, w.part_cnt, w.src, p.S, q->n, k, pw, metric, q, b, eps_xmax,
@@ -716,21 +688,6 @@ extern "C" int nrb_search_flat(const nrb_matrix* q, const nrb_matrix* b, int32_t
     return search_flat_impl(q, b, metric, k, id_base, D, I, workspace, workspace_bytes, path, (cudaStream_t)stream);
 }
 
-extern "C" int nrb_search_flat_seeded(const nrb_matrix* q, const nrb_matrix* b, int32_t metric, int32_t k,
-                                      int64_t id_base, float* D, int64_t* I, void* workspace,
-                                      size_t workspace_bytes, int32_t path, const float* seed_kth, void* stream) {
-    NRB_REQUIRE(q && b && D && I, "search_flat_seeded: null argument");
-    NRB_REQUIRE(metric == NRB_METRIC_INNER_PRODUCT || metric == NRB_METRIC_L2, "search_flat_seeded: bad metric %d", metric);
-    NRB_REQUIRE(k >= 1 && k <= NRB_MAX_K, "search_flat_seeded: k=%d out of range [1,%d]", k, NRB_MAX_K);
-    NRB_REQUIRE(q->d == b->d && q->kp == b->kp, "search_flat_seeded: dimension mismatch");
-    NRB_REQUIRE(q->n >= 0 && b->n >= 0 && b->n < (1LL << 31) - 4096 && q->n < (1LL << 31), "search_flat_seeded: sizes out of range");
-    NRB_REQUIRE(path >= NRB_PATH_AUTO && path <= NRB_PATH_TC16, "search_flat_seeded: bad path %d", path);
-    if (q->n == 0) return NRB_OK;
-    int rc = require_device();
-    if (rc) return rc;
-    return search_flat_impl(q, b, metric, k, id_base, D, I, workspace, workspace_bytes, path, (cudaStream_t)stream, seed_kth);
-}
-
 extern "C" int64_t nrb_fallback_query_count(void) { return (int64_t)g_fallback_queries.load(); }
 
 extern "C" int nrb_plan_flat_describe(int64_t nq, int64_t nb, int32_t k, int32_t path, int32_t* out10) {
@@ -759,11 +716,7 @@ extern "C" size_t nrb_ivf_search_workspace(int64_t nq, int32_t nprobe, int32_t k
 namespace nrb {
 
 // phase A (or a single-phase scan): cold rows; phase B: rows start from their query's shared bound
-static inline int ivf_mode_of(int nph, int i) {
-    static const int force = getenv("NRB_IVF_MODE") ? atoi(getenv("NRB_IVF_MODE")) : -1;  // A/B measurements
-    if (force >= 0) return force;
-    return (nph > 1 && i == 1) ? 2 : 1;
-}
+static inline int ivf_mode_of(int nph, int i) { return (nph > 1 && i == 1) ? 2 : 1; }
 
 // dst[i, :] = src[list[i], :] for rows of `width` 64-bit ids (coarse assignments of flagged queries)
 __global__ void gather_i64_rows_kernel(const int64_t* __restrict__ src, int width, const int* __restrict__ list,

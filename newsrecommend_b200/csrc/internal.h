@@ -1,6 +1,5 @@
 // Internal C++ interfaces between the translation units of libnrb200.
 #pragma once
-#include <cstdlib>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -26,7 +25,6 @@ constexpr int UNIT_ROWS = 128;
 int tc_available();  // 1 when the current device is sm_100
 size_t tc_scratch_bytes(int grid);
 int tc_grid(int n_units_upper);
-void tc_set_variant(int v);  // 1 = single-CTA kernel, 2 = CTA-pair kernel (default)
 // gthr (optional): zero-initialised per-query shared bounds; row_map/row_div map query-side rows
 // to queries (null = identity).
 int launch_topk_tc_dev(const nrb_matrix* a, const nrb_matrix* b, const Unit* units,
@@ -41,12 +39,8 @@ constexpr int TC1_EXTRA = 32;      // margin slots per row when they fit (IVF sc
 constexpr int TC1_EXTRA_FLAT = 96; // ... flat searches: as many as the 128-entry exact stage of the refine can take
 constexpr int TC1_MIN_EXTRA = 16;  // ... never fewer than this (partial rows are at most 128 wide)
 constexpr int TC1_MAX_PW = 128;
-static inline int tc1_extra() {  // NRB_TC1_EXTRA overrides the margin slots (A/B runs: scripts/bench_robustness.py)
-    static const int v = getenv("NRB_TC1_EXTRA") ? atoi(getenv("NRB_TC1_EXTRA")) : TC1_EXTRA;
-    return v < TC1_MIN_EXTRA ? TC1_MIN_EXTRA : v;
-}
 static inline int tc1_pw(int k, bool flat = false) {
-    const int extra = (flat && !getenv("NRB_TC1_EXTRA")) ? TC1_EXTRA_FLAT : tc1_extra();
+    const int extra = flat ? TC1_EXTRA_FLAT : TC1_EXTRA;
     return k + extra <= TC1_MAX_PW ? k + extra : TC1_MAX_PW;
 }
 static inline int tc1_k_ok(int k) { return k + TC1_MIN_EXTRA <= TC1_MAX_PW; }
@@ -59,10 +53,10 @@ int launch_topk_tc1_dev(const nrb_matrix* a, const nrb_matrix* b, const Unit* un
                         const int* n_units_dev, int grid, int metric, int k, int pw, float margin_scale,
                         float* part_key, int* part_idx, int* part_cnt, int* row_flags, void* scratch,
                         size_t scratch_bytes, unsigned* gthr, const int* row_map, int row_div, int f16,
-                        int single, int ivf_mode, cudaStream_t st, int seeded = 0);
+                        int single, int ivf_mode, cudaStream_t st);
 // ivf_mode: 0 = flat search; 1 = IVF list scan, cold rows (two resident query tiles: units are short);
-// 2 = IVF phase B, every row starts from its query's shared bound (also: no scheduled prunes in units
-// under 16 tiles, no union prune at the end of a unit)
+// 2 = IVF phase B, every row starts from its query's shared bound (also: no scheduled prunes, no union
+// prune at the end of a unit)
 
 // ---- topk_simt.cu: fp32 CUDA-core distance + selection over the same Unit list
 size_t simt_scratch_bytes(int grid);

@@ -31,8 +31,7 @@
 //   topk_tc2_kernel             3xTF32: per K step lo*hi, hi*lo, hi*hi into one accumulator, CTA
 //                 pairs; each CTA stages its own 128 query rows and HALF of the 256-row item
 //                 tile, so the item stream is read from L2 once per 256 queries. 3 x 64 KB stages.
-//   topk_tc_kernel              3xTF32, one CTA per unit, 2 x 96 KB stages; the simpler
-//                 cross-check (nrb_set_tc_variant(1)).
+//                 The exact path (NRB_PATH_TC) and the recompute of queries the filter flags.
 #include <cuda.h>
 
 #include <cstdlib>
@@ -49,8 +48,8 @@ constexpr int BM = 128;   // query rows per CTA tile (= TMEM lanes)
 constexpr int BN = 256;   // item rows per tile (= TMEM columns per accumulator)
 constexpr int KC = 32;    // fp32 elements per K chunk (128-byte swizzle span)
 constexpr int A_BYTES = BM * KC * 4;        // 16 KB: 128 rows x 128 B
-constexpr int BH_BYTES = (BN / 2) * KC * 4; // 16 KB: half item tile (v2)
-constexpr int B_BYTES = BN * KC * 4;        // 32 KB: full item tile (v1)
+constexpr int BH_BYTES = (BN / 2) * KC * 4; // 16 KB: half item tile (CTA pairs)
+constexpr int B_BYTES = BN * KC * 4;        // 32 KB: full item tile (single CTA)
 // Warps 0-3: control warpgroup (warp 0 TMA producer, warp 1 MMA issuer, warps 2-3 idle); warps
 // 4-7 and 8-11: the two selection warpgroups. Roles are aligned to hardware warpgroups so that
 // setmaxnreg can move registers from the control warps to the selection warps.
@@ -60,8 +59,6 @@ constexpr int EPI_WGS = 2;
 constexpr int HALF_N = BN / EPI_WGS;  // columns of every tile handled by one warpgroup
 constexpr int TMEM_COLS = 512;
 
-constexpr int V1_STAGES = 2;
-constexpr int V1_STAGE_BYTES = 2 * A_BYTES + 2 * B_BYTES;  // 96 KB
 constexpr int V2_STAGES = 3;
 constexpr int V2_STAGE_BYTES = 2 * A_BYTES + 2 * BH_BYTES;  // 64 KB
 
@@ -91,7 +88,6 @@ struct TcShared {
     XchgShared xchg;
 };
 
-constexpr size_t V1_SMEM = (size_t)V1_STAGES * V1_STAGE_BYTES + sizeof(TcShared<V1_STAGES>) + 1024;
 constexpr size_t V2_SMEM = (size_t)V2_STAGES * V2_STAGE_BYTES + sizeof(TcShared<V2_STAGES>) + 1024;
 
 // ---------------------------------------------------------------------------- timeline trace
@@ -267,19 +263,13 @@ __device__ __forceinline__ void epi_chunk(const uint32_t (&v)[32], int c0, int v
         if (!FULL && c0 + i >= valid) x = NEG_INF;
         f[i] = x;
     }
-#ifndef NRB_HIT_GROUP
-#define NRB_HIT_GROUP 8
-#endif
-    constexpr int GW = NRB_HIT_GROUP;  // columns per hit group (8; 4 measured: see DESIGN)
+    constexpr int GW = 8;  // columns per hit group (4 was measured slower: see DESIGN)
     constexpr int NG = 32 / GW;
     float g[NG];
 #pragma unroll
     for (int j = 0; j < NG; j++) {
         const float* e = f + GW * j;
-        if (GW == 8)
-            g[j] = fmaxf(fmaxf(fmaxf(fmaxf(e[0], e[1]), e[2]), fmaxf(fmaxf(e[3], e[4]), e[5])), fmaxf(e[6], e[GW - 1]));
-        else
-            g[j] = fmaxf(fmaxf(fmaxf(e[0], e[1]), e[2]), e[3]);
+        g[j] = fmaxf(fmaxf(fmaxf(fmaxf(e[0], e[1]), e[2]), fmaxf(fmaxf(e[3], e[4]), e[5])), fmaxf(e[6], e[7]));
     }
     float cmax = g[0];
 #pragma unroll
@@ -391,10 +381,7 @@ __device__ __forceinline__ void epi_unit_end_unsorted(int n, const uint2* cb, in
 // with more than 128 entries (possible only after heavy ties) are first brought down by the
 // single-buffer prune.
 constexpr int UT_SLACK = 3;
-#ifndef NRB_UT_ROWS
-#define NRB_UT_ROWS 2
-#endif
-constexpr int UT_ROWS = NRB_UT_ROWS;  // rows of a scheduled prune in flight together (2; 4 measured: flat +0 %, IVF -17 %)
+constexpr int UT_ROWS = 2;  // rows of a scheduled prune in flight together (4 was measured: flat +0 %, IVF -17 %)
 // min_new > 0 (units that share running bounds with other units of the same query: IVF lists):
 // a row pair is pruned only once min_new new candidates have arrived in one of its rows -- rows
 // whose threshold was already hot when the unit started are left alone and the scheduled prune
@@ -693,7 +680,7 @@ __device__ __forceinline__ void epi_stage_norms(float* nrm, const float* b_norms
     }
 }
 
-// The selection epilogue shared by the three kernels. Executed by warps 2..9; warpgroup
+// The selection epilogue shared by every kernel of this file. Executed by warps 2..9; warpgroup
 // g = (warp-2)/4 handles the tiles whose running index (over all units of this CTA) has parity
 // g, i.e. TMEM accumulator g. PAIR: units are taken in CTA pairs and the accumulator is handed
 // back with a cluster-scope arrive on the leader's barrier.
@@ -718,22 +705,13 @@ struct EpiArgs {
     // fp16 filter: accumulator = a_row_scale[row] * b_scale * (q . x), powers of two (null / 1: unscaled)
     const float* a_row_scale;
     float b_scale;
-    // IVF phase B (every row starts from the bound its query's closest list established): units shorter
-    // than HOT_MIN_TILES skip the scheduled prunes, and a unit ends without the pairwise union prune
-    // (rows over pw entries are tightened one by one; the in-tile overflow guard stays)
+    // IVF phase B (every row starts from the bound its query's closest list established): units run
+    // no scheduled prunes, and a unit ends without the pairwise union prune. Their rows collect what
+    // beats the bound of phase A -- ~9 candidates per (query, list) pair on average, ~110 in the
+    // longest lists -- and the few rows that outgrow a buffer are tightened one by one by the in-tile
+    // overflow guard and at the unit's end.
     int hot;
-    int one_shot_ok;  // 1: one-tile units take epi_single_tile (0 only for A/B measurements: NRB_NO_ONE_SHOT)
-    int seeded;       // 1: the shared bounds were seeded by the caller (nrb_search_flat_seeded)
-    int first_shot_ok;  // 1: the first tile of a cold multi-tile unit takes single_tile_call (0: NRB_NO_FIRST_SHOT, A/B)
 };
-#ifndef NRB_HOT_MIN_TILES
-#define NRB_HOT_MIN_TILES (1 << 30)
-#endif
-// Hot units run NO scheduled prunes at all (the value was 16 tiles until the end of round 2): their rows
-// collect what beats the bound of phase A -- ~9 candidates per (query, list) pair on average, ~110 in
-// the longest lists -- and the few rows that outgrow a buffer are tightened one by one by the in-tile
-// overflow guard and at the unit's end.
-constexpr int HOT_MIN_TILES = NRB_HOT_MIN_TILES;
 
 // IVFX compiles in the short-unit machinery (hot rows, one-tile units): only the double-buffered
 // kernel (topk_tc3d_kernel) carries it, so the flat search kernels keep their exact code.
@@ -778,7 +756,11 @@ __device__ __forceinline__ void epilogue_run(const EpiArgs& A, uint64_t* tfull, 
         if (A.gthr && live) st.gslot = A.gthr + (A.row_map ? A.row_map[ar] / A.row_div : (int)ar);
         // filter kernels, one-tile unit, cold rows: per-thread bisection in registers (epi_single_tile)
         const bool hot = IVFX && A.hot;
-        const bool one_shot = IVFX && NEED_QN && !hot && ntiles == 1 && A.one_shot_ok;
+        const bool one_shot = IVFX && NEED_QN && !hot && ntiles == 1;
+        // the unit's end (below) is chosen here, ahead of the tile loop: tested after the loop, the
+        // condition let the compiler reshape the whole loop around ntiles == 1 (more spills, IVF scan
+        // with inner products ~2 % slower on a B200)
+        const bool short_end = IVFX && NEED_QN && (hot || one_shot);
         // Cold multi-tile units (flat search: full-catalog and first-round tail units; IVF phase A): the
         // generic path appends the whole first tile (every key beats -inf: 256 entries per row, 112k
         // cycles) and then prunes 256 entries per row (58k). Their first tile takes the in-register
@@ -787,7 +769,7 @@ __device__ __forceinline__ void epilogue_run(const EpiArgs& A, uint64_t* tfull, 
         // lane quarter must take the same path (barriers inside): they agree through shared memory on
         // whether ANY of their 32 rows already holds a bound from another unit of its query.
         bool first_shot = false;
-        if (NEED_QN && !hot && ntiles > 1 && A.first_shot_ok && !A.seeded) {
+        if (NEED_QN && !hot && ntiles > 1) {
             unsigned g0 = 0u;
             if (st.gslot) g0 = *(volatile unsigned*)st.gslot;
             if (wg == 0)
@@ -882,7 +864,7 @@ __device__ __forceinline__ void epilogue_run(const EpiArgs& A, uint64_t* tfull, 
             // prunes and ~25 % more appends (scan kernels 9.2 -> 8.8 ms; the flat kernel is indifferent: 8.0 / 8.3
             // vs 8.05 ms, so it keeps the schedule its buffers were sized for)
             const bool sched = (tp & (tp - 1u)) == 0u && (!IVFX || tp == 1u || ((__ffs(tp) - 1) & 1) == 1);
-            if (sched && t + 1 < ntiles && !(hot && ntiles < HOT_MIN_TILES) && !(first_shot && t == 0)) {
+            if (sched && t + 1 < ntiles && !hot && !(first_shot && t == 0)) {
                 xs->cnt[wg][row] = st.cnt;
                 xs->fresh[wg][row] = st.cnt - st.base;
                 xs->thr[wg][row] = st.thr;
@@ -891,7 +873,7 @@ __device__ __forceinline__ void epilogue_run(const EpiArgs& A, uint64_t* tfull, 
                 ptx::named_bar_sync(3 + quad, 64);
                 NRB_TRP(warp - EPI_WARP0 + 1, 1);
                 union_tighten_rows(xs, A.cand_buf + (int64_t)blockIdx.x * EPI_WGS * BM * CAND_CAP, quad, wg, A.k, A.pw,
-                                   (A.row_map || A.seeded) ? max(4, A.k >> 2) : 0);
+                                   A.row_map ? max(4, A.k >> 2) : 0);
                 NRB_TRP(warp - EPI_WARP0 + 1, 2);
                 ptx::named_bar_sync(3 + quad, 64);
                 NRB_TRP(warp - EPI_WARP0 + 1, 3);
@@ -907,7 +889,7 @@ __device__ __forceinline__ void epilogue_run(const EpiArgs& A, uint64_t* tfull, 
                 }
             }
         }
-        if (IVFX && NEED_QN && (hot || one_shot)) {
+        if (short_end) {
             // hot units: rows hold a handful of entries; only rows over pw are tightened, each on its own
             // (no exchange with the partner warp, no barriers), then the rows leave unsorted
             const unsigned need = __ballot_sync(0xffffffffu, st.cnt > A.pw);
@@ -943,142 +925,6 @@ __device__ __forceinline__ void epilogue_run(const EpiArgs& A, uint64_t* tfull, 
             epi_unit_end(st, cb, ((int64_t)u * EPI_WGS + wg) * UNIT_ROWS + quad * 32, A.k, A.pw, A.part_key, A.part_idx, lane);
         }
         if (NEED_QN && st.flag && live) A.row_flags[A.row_map ? A.row_map[ar] / A.row_div : (int)ar] = 1;  // per QUERY
-    }
-}
-
-// ---------------------------------------------------------------------------- v1: one CTA
-template <bool L2>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-topk_tc_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constant__ CUtensorMap map_al,
-               const __grid_constant__ CUtensorMap map_bh, const __grid_constant__ CUtensorMap map_bl,
-               const Unit* __restrict__ units, const int* __restrict__ n_units_p, int nkc, int k,
-               const float* __restrict__ a_norms, const float* __restrict__ b_norms,
-               int64_t a_total, int64_t b_total, float* __restrict__ part_key,
-               int* __restrict__ part_idx, float* __restrict__ cand_key_buf,
-               int* __restrict__ cand_idx_buf, unsigned* __restrict__ gthr, const int* __restrict__ row_map,
-               int row_div) {
-    constexpr int STAGES = V1_STAGES, STAGE_BYTES = V1_STAGE_BYTES;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-    TcShared<STAGES>* sh = reinterpret_cast<TcShared<STAGES>*>(smem + (size_t)STAGES * STAGE_BYTES);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int n_units = *n_units_p;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < STAGES; s++) {
-            ptx::mbar_init(&sh->full[s], 1);
-            ptx::mbar_init(&sh->empty[s], 1);
-        }
-        for (int a = 0; a < 2; a++) {
-            ptx::mbar_init(&sh->tfull[a], 1);
-            ptx::mbar_init(&sh->tempty[a], 8);  // both warpgroups (8 warps) read every accumulator
-        }
-        ptx::fence_barrier_init();
-        ptx::prefetch_tensormap(&map_ah);
-        ptx::prefetch_tensormap(&map_al);
-        ptx::prefetch_tensormap(&map_bh);
-        ptx::prefetch_tensormap(&map_bl);
-    }
-    if (warp == 1) {
-        ptx::tmem_alloc(&sh->tmem_base, TMEM_COLS);
-        ptx::tmem_relinquish();
-    }
-    ptx::tcgen05_fence_before();
-    __syncthreads();
-    ptx::tcgen05_fence_after();
-    const uint32_t tmem_base = sh->tmem_base;
-    if (warp < EPI_WARP0) ptx::setmaxnreg_dec<40>();
-
-    // Producer and MMA warps run their loops with all 32 lanes (warp-uniform control flow), and
-    // only the instruction with side effects is issued by one elected lane: issued from divergent
-    // code, every UTMALDG / UTCHMMA gets wrapped by ptxas in a waterfall loop that moves its
-    // operands to uniform registers one by one, which made the MMA-issuing thread the bottleneck.
-    if (warp == 0) {
-        // ------------------------------------------------------------------ TMA producer
-        int stage = 0;
-        uint32_t phase = 0;
-        for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
-            const Unit un = units[u];
-            const int ntiles = un.a_rows > 0 ? (un.b_rows + BN - 1) / BN : 0;
-            for (int t = 0; t < ntiles; t++) {
-                const int brow = un.b_row0 + t * BN;
-                for (int kc = 0; kc < nkc; kc++) {
-                    ptx::mbar_wait<64>(&sh->empty[stage], phase ^ 1);
-                    uint8_t* st = smem + (size_t)stage * STAGE_BYTES;
-                    if (ptx::elect_one()) {
-                        ptx::mbar_arrive_expect_tx(&sh->full[stage], STAGE_BYTES);
-                        ptx::tma_load_2d(st, &map_ah, &sh->full[stage], kc * KC, un.a_row0);
-                        ptx::tma_load_2d(st + A_BYTES, &map_al, &sh->full[stage], kc * KC, un.a_row0);
-                        ptx::tma_load_2d(st + 2 * A_BYTES, &map_bh, &sh->full[stage], kc * KC, brow);
-                        ptx::tma_load_2d(st + 2 * A_BYTES + B_BYTES, &map_bl, &sh->full[stage], kc * KC, brow);
-                    }
-                    __syncwarp();
-                    if (++stage == STAGES) {
-                        stage = 0;
-                        phase ^= 1;
-                    }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------------------------------------------ MMA issuer
-        constexpr uint32_t idesc = ptx::umma_idesc_tf32(BM, BN);
-        const uint32_t lo0 = ptx::umma_desc_lo(ptx::smem_u32(smem));
-        int stage = 0;
-        uint32_t phase = 0;
-        int acc = 0;
-        uint32_t acc_phase = 0;
-        for (int u = blockIdx.x; u < n_units; u += gridDim.x) {
-            const Unit un = units[u];
-            const int ntiles = un.a_rows > 0 ? (un.b_rows + BN - 1) / BN : 0;
-            for (int t = 0; t < ntiles; t++) {
-                ptx::mbar_wait(&sh->tempty[acc], acc_phase ^ 1);
-                ptx::tcgen05_fence_after();
-                const uint32_t d_tmem = tmem_base + (uint32_t)(acc * BN);
-                for (int kc = 0; kc < nkc; kc++) {
-                    ptx::mbar_wait(&sh->full[stage], phase);
-                    ptx::tcgen05_fence_after();
-                    // descriptor low words advance by bytes/16: stage base, then 32 B per K step
-                    const uint32_t l_ah = lo0 + (uint32_t)(stage * STAGE_BYTES) / 16;
-                    const uint32_t l_al = l_ah + A_BYTES / 16, l_bh = l_ah + 2 * A_BYTES / 16,
-                                   l_bl = l_ah + (2 * A_BYTES + B_BYTES) / 16;
-                    if (ptx::elect_one()) {
-#pragma unroll
-                        for (int ks = 0; ks < KC / 8; ks++) {
-                            const uint64_t d_ah = ptx::umma_desc_join(l_ah + 2 * ks), d_al = ptx::umma_desc_join(l_al + 2 * ks);
-                            const uint64_t d_bh = ptx::umma_desc_join(l_bh + 2 * ks), d_bl = ptx::umma_desc_join(l_bl + 2 * ks);
-                            ptx::umma_tf32(d_tmem, d_al, d_bh, idesc, (kc | ks) != 0);
-                            ptx::umma_tf32(d_tmem, d_ah, d_bl, idesc, 1);
-                            ptx::umma_tf32(d_tmem, d_ah, d_bh, idesc, 1);
-                        }
-                        ptx::umma_commit(&sh->empty[stage]);  // frees the smem stage when the MMAs retire
-                    }
-                    __syncwarp();
-                    if (++stage == STAGES) {
-                        stage = 0;
-                        phase ^= 1;
-                    }
-                }
-                if (ptx::elect_one()) ptx::umma_commit(&sh->tfull[acc]);  // accumulator complete
-                __syncwarp();
-                acc ^= 1;
-                if (acc == 0) acc_phase ^= 1;
-            }
-        }
-    } else if (warp >= EPI_WARP0) {
-        // ------------------------------------------------------------------ selection epilogue
-        ptx::setmaxnreg_inc<232>();
-        EpiArgs ea{units, n_units, k, k, 0.f, a_norms, b_norms, a_total, b_total, part_key, part_idx, nullptr, nullptr,
-                   reinterpret_cast<uint2*>(cand_key_buf), gthr, row_map, row_div, nullptr, 1.f, 0, 0, 0, 0};
-        epilogue_run<L2, false, false>(ea, sh->tfull, sh->tempty, sh->nrm, &sh->xchg, tmem_base, warp, lane, 0);
-    }
-
-    ptx::tcgen05_fence_before();
-    __syncthreads();
-    if (warp == 1) {
-        ptx::tcgen05_fence_after();
-        ptx::tmem_dealloc(tmem_base, TMEM_COLS);
     }
 }
 
@@ -1210,7 +1056,7 @@ topk_tc2_kernel(const __grid_constant__ CUtensorMap map_ah, const __grid_constan
         // ------------------------------------------------------------------ selection epilogue (both CTAs)
         ptx::setmaxnreg_inc<232>();
         EpiArgs ea{units, *n_units_p, k, k, 0.f, a_norms, b_norms, a_total, b_total, part_key, part_idx, nullptr, nullptr,
-                   reinterpret_cast<uint2*>(cand_key_buf), gthr, row_map, row_div, nullptr, 1.f, 0, 0, 0, 0};
+                   reinterpret_cast<uint2*>(cand_key_buf), gthr, row_map, row_div, nullptr, 1.f, 0};
         epilogue_run<L2, true, false>(ea, sh->tfull, sh->tempty, sh->nrm, &sh->xchg, tmem_base, warp, lane, rank);
     }
 
@@ -1484,7 +1330,7 @@ __device__ __forceinline__ void tc3_body(const CUtensorMap& map_ah, const CUtens
         // ------------------------------------------------------------------ filter epilogue (every CTA)
         ptx::setmaxnreg_inc<232>();
         EpiArgs ea{units, *n_units_p, k, pw, margin_scale, a_norms, b_norms, a_total, b_total, part_key, part_idx,
-                   part_cnt, row_flags, reinterpret_cast<uint2*>(cand_key_buf), gthr, row_map, row_div, a_row_scale, b_scale, hot & 1, (hot & 2) ? 0 : 1, (hot & 4) ? 1 : 0, (hot & 8) ? 0 : 1};
+                   part_cnt, row_flags, reinterpret_cast<uint2*>(cand_key_buf), gthr, row_map, row_div, a_row_scale, b_scale, hot};
         epilogue_run<L2, PAIR, true, A2>(ea, sh->tfull, sh->tempty, sh->nrm, &sh->xchg, tmem_base, warp, lane, rank);
     }
 
@@ -1595,16 +1441,6 @@ int make_plane_map_h16(CUtensorMap* m, const void* base, int64_t rows, int kp, i
     return NRB_OK;
 }
 
-int g_variant = 0;  // 0 = not yet read from the environment
-
-int variant() {
-    if (g_variant == 0) {
-        const char* e = getenv("NRB_TC_VARIANT");
-        g_variant = (e && e[0] == '1') ? 1 : 2;
-    }
-    return g_variant;
-}
-
 }  // namespace
 
 int tc_available() {
@@ -1618,8 +1454,6 @@ int tc_available() {
     if (dev >= 0 && dev < 64) cached[dev] = major == 10 ? 1 : -1;
     return major == 10 ? 1 : 0;
 }
-
-void tc_set_variant(int v) { g_variant = (v == 1) ? 1 : 2; }
 
 int tc_grid(int n_units) {
     int g = sm_count() & ~1;  // whole CTA pairs
@@ -1645,13 +1479,12 @@ int launch_topk_tc_dev(const nrb_matrix* a, const nrb_matrix* b, const Unit* uni
         set_error("tc: scratch too small");
         return NRB_ERR_WORKSPACE;
     }
-    const int v = variant();
     CUtensorMap mah, mal, mbh, mbl;
     int rc;
     if ((rc = make_plane_map(&mah, a->hi, a->n, a->kp, BM))) return rc;
     if ((rc = make_plane_map(&mal, a->lo, a->n, a->kp, BM))) return rc;
-    if ((rc = make_plane_map(&mbh, b->hi, b->n, b->kp, v == 1 ? BN : BN / 2))) return rc;
-    if ((rc = make_plane_map(&mbl, b->lo, b->n, b->kp, v == 1 ? BN : BN / 2))) return rc;
+    if ((rc = make_plane_map(&mbh, b->hi, b->n, b->kp, BN / 2))) return rc;
+    if ((rc = make_plane_map(&mbl, b->lo, b->n, b->kp, BN / 2))) return rc;
     float* ck = (float*)scratch;
     int* ci = (int*)((char*)scratch + (size_t)grid * EPI_WGS * BM * CAND_CAP * sizeof(float));
     const int nkc = a->kp / KC;
@@ -1662,17 +1495,10 @@ int launch_topk_tc_dev(const nrb_matrix* a, const nrb_matrix* b, const Unit* uni
                                                 b->norms, a->n, b->n, part_key, part_idx, ck, ci, gthr,     \
                                                 row_map, row_div);                                           \
     } while (0)
-    if (v == 1) {
-        if (metric == NRB_METRIC_L2)
-            NRB_TC_LAUNCH(topk_tc_kernel<true>, V1_SMEM);
-        else
-            NRB_TC_LAUNCH(topk_tc_kernel<false>, V1_SMEM);
-    } else {
-        if (metric == NRB_METRIC_L2)
-            NRB_TC_LAUNCH(topk_tc2_kernel<true>, V2_SMEM);
-        else
-            NRB_TC_LAUNCH(topk_tc2_kernel<false>, V2_SMEM);
-    }
+    if (metric == NRB_METRIC_L2)
+        NRB_TC_LAUNCH(topk_tc2_kernel<true>, V2_SMEM);
+    else
+        NRB_TC_LAUNCH(topk_tc2_kernel<false>, V2_SMEM);
 #undef NRB_TC_LAUNCH
     NRB_LAUNCH_CHECK();
     return NRB_OK;
@@ -1692,12 +1518,8 @@ int launch_topk_tc1_dev(const nrb_matrix* a, const nrb_matrix* b, const Unit* un
                         const int* n_units_dev, int grid, int metric, int k, int pw, float margin_scale,
                         float* part_key, int* part_idx, int* part_cnt, int* row_flags, void* scratch,
                         size_t scratch_bytes, unsigned* gthr, const int* row_map, int row_div, int f16,
-                        int single, int ivf_mode, cudaStream_t st, int seeded) {
-    static const int no_one_shot = (getenv("NRB_NO_ONE_SHOT") ? 2 : 0) | (getenv("NRB_NO_FIRST_SHOT") ? 8 : 0);  // A/B measurements only
-    // bit 0: hot rows (IVF phase B); bit 1: disable epi_single_tile for one-tile units; bit 2: gthr was
-    // seeded by the caller (rows start from a known bound: scheduled prunes skip rows with few new
-    // candidates); bit 3: disable the in-register first tile of cold multi-tile units
-    const int hot = (ivf_mode == 2 ? 1 : 0) | no_one_shot | (seeded ? 4 : 0);
+                        int single, int ivf_mode, cudaStream_t st) {
+    const int hot = ivf_mode == 2 ? 1 : 0;  // IVF phase B: rows start from their query's shared bound
     NRB_REQUIRE(part_cnt, "tc1: part_cnt required (the filter kernels write unsorted partial rows)");
     NRB_REQUIRE(!single || f16, "tc1: the single-CTA form exists for the fp16 planes only");
     // what the KERNEL reads (the raw planes are the refine stage's business: *_eligible)

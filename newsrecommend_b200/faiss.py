@@ -208,17 +208,16 @@ class PackedMatrix:
         self.max_norm = 0.0
         self.h16_scale = 0.0
 
-    def struct(self, row0: int = 0, rows: int | None = None) -> Matrix:
-        rows = self.n - row0 if rows is None else rows
+    def struct(self) -> Matrix:
         m = Matrix()
-        m.raw = _ptr(self.raw[row0:]) if self.raw is not None else None
-        m.hi = _ptr(self.hi[row0:]) if self.hi is not None else None
-        m.lo = _ptr(self.lo[row0:]) if self.lo is not None else None
-        m.norms = _ptr(self.norms[row0:]) if self.norms is not None else None
-        m.h16 = _ptr(self.h16[row0:]) if self.h16 is not None else None
-        m.h16_row_scale = _ptr(self.row_scale[row0:]) if self.row_scale is not None else None
+        m.raw = _ptr(self.raw) if self.raw is not None else None
+        m.hi = _ptr(self.hi) if self.hi is not None else None
+        m.lo = _ptr(self.lo) if self.lo is not None else None
+        m.norms = _ptr(self.norms) if self.norms is not None else None
+        m.h16 = _ptr(self.h16) if self.h16 is not None else None
+        m.h16_row_scale = _ptr(self.row_scale) if self.row_scale is not None else None
         m.h16_scale = self.h16_scale if self.h16 is not None else 0.0
-        m.n, m.d, m.kp = rows, self.d, self.kp
+        m.n, m.d, m.kp = self.n, self.d, self.kp
         m.max_norm = self.max_norm if self.track_max_norm else 0.0
         return m
 
@@ -230,26 +229,18 @@ class PackedMatrix:
 
 
 def _search_flat_dev(q: PackedMatrix, b: PackedMatrix, metric: int, k: int, id_base: int = 0,
-                     path: int = PATH_AUTO, seed: torch.Tensor | None = None, rows: int | None = None,
-                     qrange: tuple[int, int] | None = None):
-    """nrb_search_flat on packed matrices -> (D f32[nq,k], I i64[nq,k]) CUDA tensors. seed f32[nq]:
-    per-query bounds for nrb_search_flat_seeded; rows: search only the first `rows` rows of b;
-    qrange = (row0, n): only these rows of q."""
-    q0, nq = qrange if qrange is not None else (0, q.n)
+                     path: int = PATH_AUTO):
+    """nrb_search_flat on packed matrices -> (D f32[nq,k], I i64[nq,k]) CUDA tensors."""
+    nq = q.n
     D = torch.empty((nq, k), dtype=torch.float32, device=q.device)
     I = torch.empty((nq, k), dtype=torch.int64, device=q.device)
     if nq == 0:
         return D, I
     wsb = lib.nrb_search_flat_workspace(nq, b.n, k, q.kp)
     ws = torch.empty(wsb, dtype=torch.uint8, device=q.device)
-    qs, bs = q.struct(q0, nq), b.struct(0, rows)
-    if seed is not None:
-        assert seed.dtype == torch.float32 and seed.numel() == nq and seed.is_contiguous()
-        check(lib.nrb_search_flat_seeded(C.byref(qs), C.byref(bs), metric, k, id_base, D.data_ptr(), I.data_ptr(),
-                                         ws.data_ptr(), wsb, path, seed.data_ptr(), _stream()), "search_flat_seeded")
-    else:
-        check(lib.nrb_search_flat(C.byref(qs), C.byref(bs), metric, k, id_base, D.data_ptr(), I.data_ptr(),
-                                  ws.data_ptr(), wsb, path, _stream()), "search_flat")
+    qs, bs = q.struct(), b.struct()
+    check(lib.nrb_search_flat(C.byref(qs), C.byref(bs), metric, k, id_base, D.data_ptr(), I.data_ptr(),
+                              ws.data_ptr(), wsb, path, _stream()), "search_flat")
     return D, I
 
 
@@ -330,17 +321,14 @@ class IndexFlat:
             self._xb = PackedMatrix(self.d, planes=_INDEX_PLANES, track_max_norm=True)
         return self._xb
 
-    def search_packed(self, q: PackedMatrix, k: int, id_base: int = 0, seed=None, rows: int | None = None,
-                      qrange: tuple[int, int] | None = None):
-        """seed / rows / qrange: see _search_flat_dev (bounds known to the caller; a row prefix as the
-        sample; a slice of the packed query batch)."""
+    def search_packed(self, q: PackedMatrix, k: int, id_base: int = 0):
         if self.ntotal == 0:
             # faiss on an empty index: I = -1, D = +/-FLT_MAX (also what an empty catalog shard returns)
-            nq = qrange[1] if qrange is not None else q.n
+            nq = q.n
             D = torch.full((nq, k), _FLT_MAX if self.metric_type == METRIC_L2 else -_FLT_MAX,
                            dtype=torch.float32, device=q.device)
             return D, torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
-        return _search_flat_dev(q, self._packed(), self.metric_type, k, id_base, self.path, seed, rows, qrange)
+        return _search_flat_dev(q, self._packed(), self.metric_type, k, id_base, self.path)
 
     def search(self, x, k: int, D=None, I=None):
         """(D, I) = search(x, k). Like faiss, optional preallocated numpy outputs D f32[nq,k],

@@ -21,19 +21,11 @@ the same code runs under gloo on CPU with the oracle index and numpy stand-ins (
 """
 from __future__ import annotations
 
-import os
-
 import numpy as np
 import torch
 import torch.distributed as dist
 
 CHUNK_WAVES = 7  # queries per chunk = CHUNK_WAVES full waves of the search kernel (7 x 18,944)
-# Rows of the sample pass that seeds every shard's running bounds. OFF by default: measured on 2 B200
-# (profiles/r02_seed_n2_*.json) the sample pass costs what it saves -- a cold 32-tile unit is ~0.5 M
-# cycles whether it runs as the sample or as the head of the shard scan, so only the G-fold reuse
-# pays, and at G = 2 the extra launches + the all-gather make it a net loss (6.19 vs 5.74 ms / step).
-# NRB_SEED_ROWS=8192 turns it on (A/B runs, larger G).
-SEED_SAMPLE_ROWS = int(os.environ.get("NRB_SEED_ROWS", "0"))
 
 
 def shard_range(nb: int, world: int, rank: int) -> tuple[int, int]:
@@ -135,9 +127,8 @@ class _ShardedSearch:
         return 1 << 17
 
     # ------------------------------------------------------------------ search pieces
-    def search_local(self, xq, k: int, per: int | None = None):
-        """Per-shard top-k of a raw query chunk with GLOBAL ids: (D f32[n,k], I i64[n,k]) tensors.
-        per: rows of the chunk each rank owns in the exchange (rank r: [r*per, (r+1)*per))."""
+    def search_local(self, xq, k: int):
+        """Per-shard top-k of a raw query chunk with GLOBAL ids: (D f32[n,k], I i64[n,k]) tensors."""
         raise NotImplementedError
 
     def _exchange_start(self, P: torch.Tensor, per: int):
@@ -176,7 +167,7 @@ class _ShardedSearch:
             parts.append(self.codec.merge(recv, self._bases(), self.metric_type))
 
         for c0, c1, per in chunk_slices(nq, G, chunk):
-            D, I = self.search_local(xq[c0:c1], k, per)
+            D, I = self.search_local(xq[c0:c1], k)
             P = self.codec.pack(D, I, self.id_base)
             nxt = self._exchange_start(P, per)
             if pending is not None:
@@ -262,7 +253,7 @@ class _ShardedSearch:
                 dist.all_gather_into_tensor(full, mine, group=self.group)
             else:
                 full = mine
-            D, I = self.search_local(full[: c1 - c0], k, per)
+            D, I = self.search_local(full[: c1 - c0], k)
             P = self.codec.pack(D, I, self.id_base)
             recv, work = self._exchange_start(P, per)
             if pending is not None:
@@ -285,7 +276,6 @@ class ShardedIndexFlat(_ShardedSearch):
             from .faiss import IndexFlat
             make_index = IndexFlat
         self.local = make_index(d, metric)
-        self.seed_sample_rows = SEED_SAMPLE_ROWS
 
     # ------------------------------------------------------------------ build
     def add_global(self, x):
@@ -307,37 +297,11 @@ class ShardedIndexFlat(_ShardedSearch):
         self.ntotal = int(ntotal)
         self._set_bases_gathered()
 
-    def _sample_bounds(self, q, k: int, per: int):
-        """Seeds for the shard searches of one chunk. A shard that starts cold spends its first tiles
-        appending nearly everything (the running top-k threshold warms up once per shard: G times
-        per query instead of once). So every rank first searches ITS rows of the chunk (the ones it
-        will merge) against the first seed_sample_rows rows of its shard -- 1/G of the queries x a
-        small sample -- and the ranks all-gather the k-th best scores (4 bytes per query). At least k
-        items of the catalog reach that score, so it is a valid lower bound of the query's global
-        k-th best, and every shard's kernel starts from it (nrb_search_flat_seeded). Returns f32[cn]
-        or None. The decision uses only rank-independent quantities (it guards a collective)."""
-        G, m = self.world, int(self.seed_sample_rows or 0)
-        from .faiss import PATH_AUTO, PATH_TC1, PATH_TC16, _round_kp
-        if G == 1 or m <= 0 or self.ntotal // G < 4 * m or k > 112 or _round_kp(self.d) > 256 or \
-                self.local.path not in (PATH_AUTO, PATH_TC1, PATH_TC16):
-            return None
-        cn, r = q.n, self.rank
-        lo, hi = min(cn, r * per), min(cn, (r + 1) * per)
-        none = 3.4028234663852886e38 if self.metric_type == 1 else -3.4028234663852886e38
-        mine = torch.full((per,), none, dtype=torch.float32, device=q.device)
-        if hi > lo:
-            Ds, _ = self.local.search_packed(q, k, 0, rows=m, qrange=(lo, hi - lo))
-            mine[: hi - lo] = Ds[:, k - 1]
-        full = torch.empty(G * per, dtype=torch.float32, device=q.device)
-        dist.all_gather_into_tensor(full, mine, group=self.group)
-        return full[:cn].contiguous()
-
-    def search_local(self, xq, k: int, per: int | None = None):
+    def search_local(self, xq, k: int):
         if self._cuda_index:
             from .faiss import PackedMatrix
             q = PackedMatrix.from_tensor(xq, planes=self.local._query_planes(k))  # K0 on the fresh chunk
-            seed = self._sample_bounds(q, k, per) if per is not None else None
-            return self.local.search_packed(q, k, self.id_base, seed=seed)
+            return self.local.search_packed(q, k, self.id_base)
         D, I = self.local.search(np.ascontiguousarray(xq), k)
         I = torch.as_tensor(I)
         return torch.as_tensor(D), torch.where(I >= 0, I + self.id_base, I)
@@ -567,7 +531,7 @@ class ShardedIndexIVFFlat(_ShardedSearch):
         self.ntotal = int(ntotal)
         self._set_bases_gathered()
 
-    def search_local(self, xq, k: int, per: int | None = None):
+    def search_local(self, xq, k: int):
         self.local.nprobe = self.nprobe
         if self._cuda_index:
             D, I = self.local.search(xq, k)  # ids = local insertion rows

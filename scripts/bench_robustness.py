@@ -7,7 +7,7 @@ queries/s, fallback queries, parity sample vs the oracle.
   * dup x m       near-duplicate-heavy catalog (news reposts): 364,047 / m base articles, each present m
                   times with relative noise 1e-4 -- inside the filter's error margin (2 * 1.07e-3 * |q| * max|x|),
                   so every copy of an article near the k-th rank lands in the margin set
-One JSON line. NRB_TC1_EXTRA=<slots> overrides the margin slots per partial row (default 32)."""
+One JSON line."""
 import json
 import os
 import sys
@@ -74,4 +74,4 @@ for m in [int(a) for a in os.environ.get("NRB_DUPS", "4,16,64").split(",")]:
         + 1e-4 * np.linalg.norm(base[rep_rows], axis=1, keepdims=True) / np.sqrt(D) * rng.standard_normal((NB, D), dtype=np.float32)
     xd = np.ascontiguousarray(xd.astype(np.float32))
     out.append(run("dup x %d (relative noise 1e-4)" % m, xd, xq))
-print(json.dumps(dict(shape=[NB, D, NQ, K], margin_slots=int(os.environ.get("NRB_TC1_EXTRA", "32")), cases=out)))
+print(json.dumps(dict(shape=[NB, D, NQ, K], cases=out)))

@@ -210,24 +210,18 @@ def test_item_item_cosine_self_match(nf):
     assert np.allclose(D[:, 0], 1.0, atol=1e-5)
 
 
-@pytest.mark.parametrize("variant", [1, 2])
 @pytest.mark.parametrize("metric", [0, 1])
-def test_tc_kernel_variants(nf, oracle, variant, metric):
-    """Both tcgen05 kernels (1 = single CTA, 2 = CTA pair / cta_group::2) against the oracle on
-    shapes with odd query-tile counts, partial item tiles and several item chunks."""
-    from newsrecommend_b200._lib import lib
+def test_tc_kernel_variants(nf, oracle, metric):
+    """The 3xTF32 tcgen05 kernel (CTA pairs, cta_group::2) against the oracle on shapes with odd
+    query-tile counts, partial item tiles and several item chunks."""
     rng = np.random.default_rng(77 + metric)
-    try:
-        assert lib.nrb_set_tc_variant(variant) == 0
-        for nq, nb, d, k in ((48, 2000, 250, 10), (385, 30011, 250, 50), (1, 70000, 96, 7), (129, 513, 32, 128)):
-            xb = rng.standard_normal((nb, d), dtype=np.float32)
-            xq = rng.standard_normal((nq, d), dtype=np.float32)
-            D, I = _search(nf, xb, xq, k, metric, "tc")
-            Do, Io = oracle.knn_fast(xq, xb, k, metric)
-            rep = compare_topk(D, I, Do, Io, metric, scale=_l2_scale(xq, xb) if metric == 1 else None)
-            assert rep["ok"], (variant, nq, nb, d, k, rep)
-    finally:
-        lib.nrb_set_tc_variant(2)
+    for nq, nb, d, k in ((48, 2000, 250, 10), (385, 30011, 250, 50), (1, 70000, 96, 7), (129, 513, 32, 128)):
+        xb = rng.standard_normal((nb, d), dtype=np.float32)
+        xq = rng.standard_normal((nq, d), dtype=np.float32)
+        D, I = _search(nf, xb, xq, k, metric, "tc")
+        Do, Io = oracle.knn_fast(xq, xb, k, metric)
+        rep = compare_topk(D, I, Do, Io, metric, scale=_l2_scale(xq, xb) if metric == 1 else None)
+        assert rep["ok"], (nq, nb, d, k, rep)
 
 
 @pytest.mark.parametrize("filt", ["tc1", "tc16"])
@@ -346,57 +340,3 @@ def test_single_cta_filter_kernel(nf, oracle, metric, monkeypatch):
         Do, Io = oracle.knn_fast(xq, xb, k, metric)
         rep = compare_topk(D, I, Do, Io, metric, scale=_l2_scale(xq, xb) if metric == 1 else None)
         assert rep["ok"], (nq, nb, d, k, rep)
-
-
-@pytest.mark.parametrize("metric", [0, 1])
-@pytest.mark.parametrize("path", ["auto", "tc1"])
-def test_seeded_search(nf, oracle, metric, path):
-    """nrb_search_flat_seeded: bounds the caller knows (k-th best of a row sample, of the whole
-    catalog, of another shard) change nothing about what is found above them."""
-    import torch
-    from newsrecommend_b200 import synth
-    nb, d, nq, k, m = 30_011, 250, 1_111, 50, 2_048
-    xb, topics = synth.g_skew(nb, d, 3, return_topics=True)
-    xq = synth.user_profiles(xb, topics, nq, 4)
-    index = nf.IndexFlat(d, metric)
-    index.path = PATHS[path]
-    index.add(xb)
-    q = nf.PackedMatrix.from_tensor(torch.from_numpy(xq).cuda(), planes=index._query_planes(k))
-    D0, I0 = index.search_packed(q, k)
-    Do, Io = oracle.knn_fast(xq, xb, k, metric)
-    assert compare_topk(D0.cpu().numpy(), I0.cpu().numpy(), Do, Io, metric)["ok"]
-    # (1) seeds = k-th best over the first m rows (the sample pass of the sharded search)
-    Ds, _ = index.search_packed(q, k, rows=m)
-    Dm, Im = oracle.knn_fast(xq, xb[:m], k, metric)
-    assert compare_topk(Ds.cpu().numpy(), _.cpu().numpy(), Dm, Im, metric)["ok"]
-    D1, I1 = index.search_packed(q, k, seed=Ds[:, k - 1].contiguous())
-    assert torch.equal(I1, I0) and torch.equal(D1, D0)
-    # (2) the tightest valid bound: the exact k-th best of the whole catalog; rows without a bound mixed in
-    seed = D0[:, k - 1].clone()
-    seed[::7] = 3.4028234663852886e38 if metric == 1 else -3.4028234663852886e38
-    seed[3::7] = float("nan")
-    D2, I2 = index.search_packed(q, k, seed=seed)
-    assert compare_topk(D2.cpu().numpy(), I2.cpu().numpy(), D0.cpu().numpy(), I0.cpu().numpy(), metric)["ok"]
-    # (3) a bound from ANOTHER shard: this shard returns exactly its items that reach it (up to k)
-    half = nb // 2
-    other = nf.IndexFlat(d, metric)
-    other.path = PATHS[path]
-    other.add(xb[half:])
-    Dg, Ig = other.search_packed(q, k, half)
-    mine = nf.IndexFlat(d, metric)
-    mine.path = PATHS[path]
-    mine.add(xb[:half])
-    Dl, Il = mine.search_packed(q, k, 0, seed=Dg[:, k - 1].contiguous())
-    Df, If = mine.search_packed(q, k, 0)  # the shard's full top-k
-    Dl_h, Il_h, Df_h, If_h, bound = (t.cpu().numpy() for t in (Dl, Il, Df, If, Dg[:, k - 1]))
-    for i in range(nq):
-        reach = (Df_h[i] >= bound[i]) if metric == 0 else (Df_h[i] <= bound[i])
-        want = If_h[i][reach]  # local items at least as good as the other shard's k-th best
-        got = Il_h[i][Il_h[i] >= 0]
-        assert np.isin(want, got).all(), (i, want.size, got.size)
-        assert np.isin(got, If_h[i]).all()
-    # merged with the other shard: the global top-k
-    from newsrecommend_b200.sharded import GpuCodec
-    P = torch.stack([GpuCodec.pack(Dl, Il, 0), GpuCodec.pack(Dg, Ig, half)])
-    Dmg, Img = GpuCodec.merge(P, torch.tensor([0, half], dtype=torch.int64, device="cuda"), metric)
-    assert compare_topk(Dmg.cpu().numpy(), Img.cpu().numpy(), Do, Io, metric)["ok"]
