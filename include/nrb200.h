@@ -263,6 +263,24 @@ int nrb_ivf_scan_small(const float* xq, int64_t ldq, int32_t nq, int32_t d, cons
  * the article id (news/article_table.npy) -> emb f32[n, width-1] C-contiguous, ids i64[n]. */
 int nrb_split_table_f64(const double* table, int64_t n, int32_t width, float* emb, int64_t* ids, void* stream);
 
+/* ---- external ids (faiss IndexIDMap, IndexIVF::add_with_ids / remove_ids) -------------------
+ * The reference keeps the article ids in an array beside the index and translates row positions
+ * by hand (Retrieval.py:7 splits article_ids off the table, Retrieval.py:23 maps rows to ids);
+ * these entry points let the index carry the ids and drop rows by id.
+ * nrb_id_select: faiss IDSelectorBatch / IDSelectorRange over n ids: member[i] = 1 if ids[i] is
+ * selected, else 0. ids == NULL: the id of row i is i (IndexFlat without an id map). batch == NULL:
+ * range, imin <= id < imax (empty when imin >= imax). Otherwise a set of nbatch ids (any int64
+ * value, duplicates allowed; nbatch == 0 selects nothing), built in the workspace as an
+ * open-addressing hash table (64-bit atomicCAS inserts, then one probe per id); the empty-slot
+ * sentinel (-1) is tracked by a separate flag word, so a batch may contain it. member is i64 so it
+ * feeds nrb_ivf_build_lists(member, n, 2, ...) directly: a stable keep / remove partition,
+ * offsets[1] = rows kept. Workspace: nrb_id_select_workspace(nbatch) bytes (0 for a range). */
+size_t nrb_id_select_workspace(int64_t nbatch);
+int nrb_id_select(const int64_t* ids, int64_t n, const int64_t* batch, int64_t nbatch, int64_t imin,
+                  int64_t imax, int64_t* member, void* workspace, size_t workspace_bytes, void* stream);
+/* IndexIDMap::search's label translation, in place: I[i] = I[i] < 0 ? I[i] : id_map[I[i]]. */
+int nrb_map_ids(const int64_t* id_map, int64_t* I, int64_t n, void* stream);
+
 /* Wire format of the all-to-all by query range (the exchange step of the catalog-sharded search):
  * P[i] = (fp32 bits of D[i]) << 32 | uint32(I[i] - id_base), 0xffffffff in the low word when
  * I[i] < 0. 8 bytes per candidate, one collective instead of two. n = nq * k elements. */

@@ -34,6 +34,7 @@ SYMBOLS = [
     "nrb_pack_topk", "nrb_merge_topk_packed",
     "nrb_search_small_workspace", "nrb_search_small", "nrb_search_small_host",
     "nrb_ivf_scan_small_workspace", "nrb_ivf_scan_small", "nrb_split_table_f64",
+    "nrb_id_select_workspace", "nrb_id_select", "nrb_map_ids",
 ]
 
 
@@ -102,6 +103,10 @@ lib.nrb_ivf_scan_small.argtypes = [_vp, _i64, _i32, _i32, _mp, _vp, _i32, _i32, 
 lib.nrb_split_table_f64.argtypes = [_vp, _i64, _i32, _vp, _vp, _vp]
 lib.nrb_expand_lists.argtypes = [_vp, _vp, _vp, _vp, _i64, _vp, _vp]
 lib.nrb_csr_contains.argtypes = [_vp, _vp, _vp, _i64, _vp, _vp]
+lib.nrb_id_select_workspace.restype = _sz
+lib.nrb_id_select_workspace.argtypes = [_i64]
+lib.nrb_id_select.argtypes = [_vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _sz, _vp]
+lib.nrb_map_ids.argtypes = [_vp, _vp, _i64, _vp]
 
 
 def last_error() -> str:

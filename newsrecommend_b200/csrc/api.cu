@@ -39,7 +39,7 @@ int sm_count() {
     return cached;
 }
 
-static int require_device() {
+int require_device() {
     static int n = -1;
     if (n <= 0 && (cudaGetDeviceCount(&n) != cudaSuccess || n == 0)) {
         n = 0;

@@ -108,5 +108,7 @@ int launch_exact_k1_fallback(const nrb_matrix* q, const nrb_matrix* b, int metri
                              const int* count, float* D, int64_t* I, cudaStream_t st);
 
 int sm_count();
+// NRB_OK, or NRB_ERR_NO_DEVICE (with the message set) when there is no sm_100 device
+int require_device();
 
 }  // namespace nrb

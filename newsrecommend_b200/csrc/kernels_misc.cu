@@ -1503,3 +1503,129 @@ extern "C" int nrb_csr_contains(const int64_t* off, const int64_t* ids, const in
     NRB_LAUNCH_CHECK();
     return NRB_OK;
 }
+
+// ------------------------------------------------------------------- id selectors (faiss IDSelector*)
+// Retrieval.py:7,23 keep the article ids in a second array beside the index; these two entry points
+// let the index carry them (IndexIDMap, IndexIVFFlat.add_with_ids) and drop rows by id (remove_ids).
+// IDSelectorBatch is an open-addressing hash table with linear probing in the workspace: a power-of-two
+// capacity of at least twice the batch (load factor <= 1/2), empty slots hold ID_EMPTY, and a batch
+// entry equal to ID_EMPTY sets the flag word instead of occupying a slot.
+constexpr int64_t ID_EMPTY = -1;  // workspace is cleared with cudaMemsetAsync(0xff)
+
+static int64_t id_table_cap(int64_t nbatch) {
+    int64_t cap = 64;
+    while (cap < 2 * nbatch) cap <<= 1;
+    return cap;
+}
+
+__device__ __forceinline__ uint64_t id_hash(int64_t v) {  // splitmix64 finaliser
+    uint64_t z = (uint64_t)v;
+    z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+    z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+    return z ^ (z >> 31);
+}
+
+__global__ void id_insert_kernel(const int64_t* __restrict__ batch, int64_t nbatch, unsigned long long* table,
+                                 uint64_t mask, int* has_empty) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nbatch; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t v = batch[i];
+        if (v == ID_EMPTY) {
+            *has_empty = 1;
+            continue;
+        }
+        for (uint64_t s = id_hash(v) & mask;; s = (s + 1) & mask) {
+            const unsigned long long prev = atomicCAS(table + s, (unsigned long long)ID_EMPTY, (unsigned long long)v);
+            if (prev == (unsigned long long)ID_EMPTY || prev == (unsigned long long)v) break;
+        }
+    }
+}
+
+// member[i] = 1 if the id of row i (ids[i], or i when ids == NULL) is selected. table == NULL: range.
+__global__ void id_member_kernel(const int64_t* __restrict__ ids, int64_t n, const int64_t* __restrict__ table,
+                                 uint64_t mask, const int* __restrict__ has_empty, int64_t imin, int64_t imax,
+                                 int64_t* __restrict__ member) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t v = ids ? ids[i] : i;
+        int64_t m;
+        if (!table) {
+            m = imin <= v && v < imax;
+        } else if (v == ID_EMPTY) {
+            m = *has_empty;
+        } else {
+            m = 0;
+            for (uint64_t s = id_hash(v) & mask;; s = (s + 1) & mask) {
+                const int64_t t = table[s];
+                if (t == v) { m = 1; break; }
+                if (t == ID_EMPTY) break;
+            }
+        }
+        member[i] = m;
+    }
+}
+
+__global__ void map_ids_kernel(const int64_t* __restrict__ id_map, int64_t* __restrict__ I, int64_t n) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t v = I[i];
+        if (v >= 0) I[i] = id_map[v];
+    }
+}
+
+extern "C" size_t nrb_id_select_workspace(int64_t nbatch) {
+    if (nbatch <= 0) return 0;
+    return 256 + (size_t)id_table_cap(nbatch) * sizeof(int64_t);
+}
+
+extern "C" int nrb_id_select(const int64_t* ids, int64_t n, const int64_t* batch, int64_t nbatch, int64_t imin,
+                             int64_t imax, int64_t* member, void* workspace, size_t workspace_bytes, void* stream) {
+    NRB_REQUIRE(n >= 0 && nbatch >= 0 && nbatch < (1LL << 40), "id_select: bad sizes n=%lld nbatch=%lld",
+                (long long)n, (long long)nbatch);
+    NRB_REQUIRE(batch || nbatch == 0, "id_select: nbatch=%lld with no batch", (long long)nbatch);
+    NRB_REQUIRE(n == 0 || member, "id_select: null member");
+    if (batch && nbatch == 0) {  // an empty batch selects nothing: the empty range
+        batch = nullptr;
+        imin = imax = 0;
+    }
+    const size_t need = batch ? nrb_id_select_workspace(nbatch) : 0;
+    if (workspace_bytes < need || (need && !workspace)) {
+        set_error("id_select: workspace %zu < %zu", workspace_bytes, need);
+        return NRB_ERR_WORKSPACE;
+    }
+    if (n == 0) return NRB_OK;
+    int rc = require_device();
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t* table = nullptr;
+    const int* has_empty = nullptr;
+    uint64_t mask = 0;
+    if (batch) {
+        const int64_t cap = id_table_cap(nbatch);
+        int* flag = (int*)workspace;
+        unsigned long long* tab = (unsigned long long*)((char*)workspace + 256);
+        NRB_CUDA_CHECK(cudaMemsetAsync(flag, 0, sizeof(int), st));
+        NRB_CUDA_CHECK(cudaMemsetAsync(tab, 0xff, (size_t)cap * sizeof(int64_t), st));
+        mask = (uint64_t)cap - 1;
+        int64_t blocks = (nbatch + 255) / 256;
+        if (blocks > 148 * 16) blocks = 148 * 16;
+        id_insert_kernel<<<(unsigned)blocks, 256, 0, st>>>(batch, nbatch, tab, mask, flag);
+        NRB_LAUNCH_CHECK();
+        table = (const int64_t*)tab;
+        has_empty = flag;
+    }
+    int64_t blocks = (n + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    id_member_kernel<<<(unsigned)blocks, 256, 0, st>>>(ids, n, table, mask, has_empty, imin, imax, member);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}
+
+extern "C" int nrb_map_ids(const int64_t* id_map, int64_t* I, int64_t n, void* stream) {
+    NRB_REQUIRE(n >= 0 && (n == 0 || (id_map && I)), "map_ids: bad arguments");
+    if (n == 0) return NRB_OK;
+    int rc = require_device();
+    if (rc) return rc;
+    int64_t blocks = (n + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    map_ids_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(id_map, I, n);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}

@@ -3,7 +3,9 @@
 Mirrors exactly the symbols /root/reference/Retrieval.py uses (Retrieval.py:12-32: Clustering,
 IndexHNSWFlat, IndexFlatL2, vector_float_to_array, index.search) plus the index surface
 BASELINE.json's north_star names (IndexFlatIP, IndexIVFFlat with train/add/search, nlist /
-nprobe / k semantics, METRIC_*, normalize_L2). Semantics follow SURVEY.md section 8b.
+nprobe / k semantics, METRIC_*, normalize_L2). Semantics follow SURVEY.md section 8b. External
+ids (IndexIDMap, IndexIVFFlat.add_with_ids, remove_ids with IDSelectorBatch / IDSelectorRange) stand
+in for the article-id array that Retrieval.py:7,23 keeps beside the index.
 
 Host code only: every array lives in HBM as torch tensors and all arithmetic is done by
 libnrb200.so (hand-written sm_100a CUDA) through the C-ABI in include/nrb200.h. numpy in ->
@@ -26,7 +28,8 @@ from ._lib import (METRIC_INNER_PRODUCT, METRIC_L2, PATH_AUTO, PATH_SIMT, PATH_T
 
 __all__ = [
     "METRIC_INNER_PRODUCT", "METRIC_L2", "IndexFlat", "IndexFlatL2", "IndexFlatIP", "IndexHNSWFlat",
-    "IndexIVFFlat", "Clustering", "ClusteringParameters", "vector_float_to_array", "normalize_L2",
+    "IndexIVFFlat", "IndexIDMap", "IDSelectorBatch", "IDSelectorRange", "Clustering", "ClusteringParameters",
+    "vector_float_to_array", "normalize_L2",
 ]
 
 _FLT_MAX = 3.4028234663852886e38
@@ -247,6 +250,122 @@ def _search_flat_dev(q: PackedMatrix, b: PackedMatrix, metric: int, k: int, id_b
 _INDEX_PLANES = ("raw", "hi", "lo", "norms", "h16")
 
 
+# ------------------------------------------------------------------------------------ ids
+class IDSelectorRange:
+    """faiss.IDSelectorRange: selects imin <= id < imax. A host-side description that remove_ids
+    hands to nrb_id_select; assume_sorted is accepted for faiss compatibility and changes nothing."""
+
+    def __init__(self, imin: int, imax: int, assume_sorted: bool = False):
+        self.imin, self.imax, self.assume_sorted = int(imin), int(imax), bool(assume_sorted)
+
+    def is_member(self, i: int) -> bool:
+        return self.imin <= i < self.imax
+
+
+class IDSelectorBatch:
+    """faiss.IDSelectorBatch: selects the ids of a set (duplicates allowed). IDSelectorBatch(ids),
+    or faiss's SWIG form IDSelectorBatch(n, ids) with a numpy array in place of the pointer (the
+    first n entries count)."""
+
+    def __init__(self, *args):
+        if len(args) == 2:
+            n, ids = int(args[0]), _int64_ids(args[1], "IDSelectorBatch")
+            if not 0 <= n <= ids.shape[0]:
+                raise ValueError(f"IDSelectorBatch: n={n} but {ids.shape[0]} ids given")
+            ids = ids[:n]
+        elif len(args) == 1:
+            ids = _int64_ids(args[0], "IDSelectorBatch")
+        else:
+            raise TypeError("IDSelectorBatch(ids) or IDSelectorBatch(n, ids)")
+        self.ids = np.ascontiguousarray(ids)
+
+    def is_member(self, i: int) -> bool:
+        return bool(np.any(self.ids == i))
+
+
+def _int64_ids(a, what: str) -> np.ndarray:
+    """A 1-D host array of integer ids as int64 (floats are refused, not truncated)."""
+    if isinstance(a, torch.Tensor):
+        a = a.detach().cpu().numpy()
+    a = np.asarray(a)
+    if a.ndim != 1 or not (np.issubdtype(a.dtype, np.integer) or a.size == 0):
+        raise TypeError(f"{what}: expected a 1-D integer id array, got {a.dtype} of shape {a.shape}")
+    return a.astype(np.int64, copy=False)
+
+
+def _selector(sel):
+    """remove_ids' argument: an IDSelector, or an id array wrapped in IDSelectorBatch (faiss's
+    Python layer does the same)."""
+    if isinstance(sel, (IDSelectorBatch, IDSelectorRange)):
+        return sel
+    if isinstance(sel, (np.ndarray, torch.Tensor)):
+        return IDSelectorBatch(sel)
+    raise TypeError(f"remove_ids takes an IDSelectorBatch, an IDSelectorRange or an int64 id array, not {type(sel)}")
+
+
+def _keep_partition(sel, ids, n: int, dev):
+    """Stable keep / remove partition of n rows whose ids are ids (i64 CUDA tensor) or, when ids
+    is None, the row positions: nrb_id_select marks the selected rows, nrb_ivf_build_lists with two
+    buckets puts the rest first in their old order. Returns (order i32 CUDA tensor of the kept rows,
+    number of removed rows); reads one count back, so it synchronises the stream."""
+    member = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+    if isinstance(sel, IDSelectorRange):
+        batch, nb, imin, imax = None, 0, sel.imin, sel.imax
+    else:
+        batch = torch.from_numpy(sel.ids).to(dev) if sel.ids.size else None
+        nb, imin, imax = sel.ids.size, 0, 0
+    wsb = lib.nrb_id_select_workspace(nb)
+    ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device=dev)
+    check(lib.nrb_id_select(_ptr(ids), n, _ptr(batch), nb, imin, imax, member.data_ptr(), ws.data_ptr(), wsb,
+                            _stream()), "id_select")
+    offsets = torch.empty(3, dtype=torch.int32, device=dev)
+    order = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
+    wsb = lib.nrb_ivf_build_lists_workspace(n, 2)
+    ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
+    check(lib.nrb_ivf_build_lists(member.data_ptr(), n, 2, offsets.data_ptr(), order.data_ptr(), ws.data_ptr(), wsb,
+                                  _stream()), "ivf_build_lists")
+    nkeep = int(_to_host(offsets[1:2])[0])
+    return order[:nkeep], n - nkeep
+
+
+def _gather_i64(src: torch.Tensor, order: torch.Tensor) -> torch.Tensor:
+    dst = torch.empty(order.shape[0], dtype=torch.int64, device=src.device)
+    check(lib.nrb_gather_i64(src.data_ptr(), order.data_ptr(), order.shape[0], dst.data_ptr(), _stream()),
+          "gather_i64")
+    return dst
+
+
+def _gather_packed(p: PackedMatrix, order: torch.Tensor) -> PackedMatrix:
+    """The rows order[:] of p's raw plane appended to a fresh PackedMatrix with p's planes: every
+    plane, max_norm and h16_scale come out as if those rows had been added in one call."""
+    n = order.shape[0]
+    raw = torch.empty((n, p.kp), dtype=torch.float32, device=p.device)
+    check(lib.nrb_gather_rows(p.raw.data_ptr(), p.kp, order.data_ptr(), n, raw.data_ptr(), _stream()), "gather_rows")
+    out = PackedMatrix(p.d, p.device, planes=p.planes, track_max_norm=p.track_max_norm)
+    out.append(raw[:, : p.d])
+    return out
+
+
+def _ids_arg(ids, n: int, dev) -> torch.Tensor:
+    """add_with_ids' ids: an int64 numpy array or torch tensor of length n -> i64 CUDA tensor."""
+    if isinstance(ids, np.ndarray):
+        ok = ids.dtype == np.int64
+        t = torch.from_numpy(np.ascontiguousarray(ids)) if ok else None
+    elif isinstance(ids, torch.Tensor):
+        ok, t = ids.dtype == torch.int64, ids
+    else:
+        ok = False
+    if not ok or t.dim() != 1 or t.shape[0] != n:
+        raise TypeError(f"add_with_ids: ids must be an int64 numpy array or tensor of length {n}")
+    return t.to(dev, non_blocking=True).contiguous()
+
+
+def _map_ids(id_map: torch.Tensor | None, I: torch.Tensor):
+    """IndexIDMap's label translation on the current stream, in place: I = id_map[I] where I >= 0."""
+    if id_map is not None and id_map.numel():
+        check(lib.nrb_map_ids(id_map.data_ptr(), I.data_ptr(), I.numel(), _stream()), "map_ids")
+
+
 # ------------------------------------------------------------------------------------ flat
 class IndexFlat:
     """IndexFlatL2 / IndexFlatIP (Retrieval.py:25-26,32; SURVEY 8b). add() copies into HBM."""
@@ -330,9 +449,33 @@ class IndexFlat:
             return D, torch.full((nq, k), -1, dtype=torch.int64, device=q.device)
         return _search_flat_dev(q, self._packed(), self.metric_type, k, id_base, self.path)
 
+    def add_with_ids(self, x, ids):
+        raise RuntimeError("add_with_ids not implemented for this type of index")
+
+    def remove_ids(self, sel) -> int:
+        """faiss IndexFlatCodes::remove_ids: `sel` selects row positions. The rows after each removed
+        row move up (a stable compaction), and the storage is rebuilt as one add() of the survivors,
+        so max_norm and the fp16 scale shrink with them. Returns the number of rows removed."""
+        n = self.ntotal
+        if n == 0:
+            _selector(sel)
+            return 0
+        order, removed = _keep_partition(_selector(sel), None, n, self._xb.device)
+        if removed:
+            self._keep_rows(order)
+        return removed
+
+    def _keep_rows(self, order: torch.Tensor):
+        self._xb = _gather_packed(self._xb, order)
+        self._struct_cache = None
+
     def search(self, x, k: int, D=None, I=None):
         """(D, I) = search(x, k). Like faiss, optional preallocated numpy outputs D f32[nq,k],
         I i64[nq,k] are filled and returned (page-locked buffers avoid a staging copy)."""
+        return self._search(x, k, D, I, None)
+
+    def _search(self, x, k: int, D, I, id_map: torch.Tensor | None):
+        """search(); id_map (IndexIDMap): labels are translated on the device before any copy back."""
         assert k > 0
         if k > _lib.MAX_K:
             raise RuntimeError(f"k={k} > {_lib.MAX_K} is not supported by the selection stage")
@@ -340,24 +483,26 @@ class IndexFlat:
         if not isinstance(x, torch.Tensor) and torch.cuda.is_available():
             a = np.ascontiguousarray(x, dtype=np.float32)
             assert a.ndim == 2 and a.shape[1] == self.d
-            if small and 0 < a.shape[0] < self.small_nq:
+            if small and 0 < a.shape[0] < self.small_nq and id_map is None:
                 return self._search_small_host(a, int(k), D, I)
             if a.shape[0] >= 2 * _wave_rows():
-                return self._search_host_pipelined(a, int(k), D, I)
+                return self._search_host_pipelined(a, int(k), D, I, id_map)
         t, from_np = _to_device_f32(x)
         assert t.shape[1] == self.d
         if small and 0 < t.shape[0] < self.small_nq:
             Dd, Id = self._search_small_dev(t, int(k))
+            _map_ids(id_map, Id)
             if from_np or D is not None or I is not None:
                 return _to_host_pair(Dd, Id, D, I)
             return Dd, Id
         q = PackedMatrix.from_tensor(t, planes=self._query_planes(int(k)))
         Dd, Id = self.search_packed(q, int(k))
+        _map_ids(id_map, Id)
         if from_np or D is not None or I is not None:
             return _to_host_pair(Dd, Id, D, I)
         return Dd, Id
 
-    def _search_host_pipelined(self, a: np.ndarray, k: int, D=None, I=None):
+    def _search_host_pipelined(self, a: np.ndarray, k: int, D=None, I=None, id_map=None):
         """Host arrays in, host arrays out, for batches of at least two waves: the batch is cut at
         wave boundaries (one wave = one 256-query unit pair per CTA pair, so the cuts cost the
         kernel nothing), all host-to-device copies are queued on a copy stream up front, and each
@@ -394,6 +539,7 @@ class IndexFlat:
             xd.record_stream(cur)
             q = PackedMatrix.from_tensor(xd, planes=planes)
             Dd, Id = self.search_packed(q, k)
+            _map_ids(id_map, Id)
             done = torch.cuda.Event()
             done.record(cur)
             with torch.cuda.stream(d2h):
@@ -434,6 +580,64 @@ class IndexFlatL2(IndexFlat):
 class IndexFlatIP(IndexFlat):
     def __init__(self, d: int):
         super().__init__(d, METRIC_INNER_PRODUCT)
+
+
+class IndexIDMap:
+    """faiss.IndexIDMap over an empty IndexFlat (or subclass): rows carry caller-given int64 ids, such
+    as the article ids that Retrieval.py:7 splits off the embedding table and Retrieval.py:23 maps
+    rows back to by hand. The ids live on the device beside the rows; search() runs the inner
+    index's own route (the same D on every path) and translates labels with nrb_map_ids on the
+    current stream before any copy back; -1 stays -1. Numpy batches of fewer than 20 queries cannot
+    take the single-call host route (its kernels write straight into host memory), so they run the
+    device route, the translation and one copy back: a few microseconds more per call than the plain
+    index. IndexIVFFlat carries ids of its own (add_with_ids) and is not wrapped."""
+
+    def __init__(self, index):
+        if not isinstance(index, IndexFlat):
+            raise TypeError(f"IndexIDMap wraps an IndexFlat (IndexFlatIP, IndexFlatL2); {type(index).__name__} "
+                            "is not supported (IndexIVFFlat has add_with_ids of its own)")
+        if index.ntotal != 0:
+            raise RuntimeError("index must be empty on input")
+        self.index = index
+        self.id_map: torch.Tensor | None = None  # i64[ntotal] on the device, row order
+
+    ntotal = property(lambda self: self.index.ntotal)
+    d = property(lambda self: self.index.d)
+    metric_type = property(lambda self: self.index.metric_type)
+    is_trained = property(lambda self: self.index.is_trained)
+
+    def train(self, x):
+        self.index.train(x)
+
+    def add(self, x):
+        raise RuntimeError("add does not make sense with IndexIDMap, use add_with_ids")
+
+    def add_with_ids(self, x, ids):
+        t, _ = _to_device_f32(x)
+        assert t.shape[1] == self.d
+        ids_d = _ids_arg(ids, t.shape[0], t.device)
+        self.index.add(t)
+        self.id_map = ids_d if self.id_map is None or self.id_map.numel() == 0 else torch.cat([self.id_map, ids_d])
+
+    def search(self, x, k: int, D=None, I=None):
+        return self.index._search(x, k, D, I, self.id_map if self.ntotal else None)
+
+    def remove_ids(self, sel) -> int:
+        """faiss IndexIDMapTemplate::remove_ids: selects on the external ids, compacts the inner
+        index and the id map with the same stable partition. Returns the number of rows removed."""
+        sel = _selector(sel)
+        n = self.ntotal
+        if n == 0:
+            return 0
+        order, removed = _keep_partition(sel, self.id_map, n, self.id_map.device)
+        if removed:
+            self.index._keep_rows(order)
+            self.id_map = _gather_i64(self.id_map, order)
+        return removed
+
+    def reset(self):
+        self.index.reset()
+        self.id_map = None
 
 
 class IndexHNSWFlat(IndexFlatL2):
@@ -609,7 +813,12 @@ class IndexIVFFlat:
     """IndexIVFFlat(quantizer, d, nlist, metric): train = k-means on the quantizer (cp.niter =
     10), add = nearest centroid + list-contiguous layout, search = coarse top-nprobe + list
     scan (SURVEY 3.3). In the reference this is the hand-rolled k-means -> cluster_to_articles
-    -> nearest-centroid pipeline of Retrieval.py:11-34."""
+    -> nearest-centroid pipeline of Retrieval.py:11-34.
+
+    Every row carries an int64 id: add() numbers rows ntotal, ntotal+1, ... as faiss does (also after
+    removals), add_with_ids() stores the ids given, remove_ids() drops rows by id. The lists keep
+    rows in insertion order, so with arbitrary ids exact score ties come out in list-position
+    order, where faiss orders them by id."""
 
     def __init__(self, quantizer: IndexFlat, d: int, nlist: int, metric: int = METRIC_L2):
         self.quantizer = quantizer
@@ -625,6 +834,7 @@ class IndexIVFFlat:
         self.clustering = None
         self._x: PackedMatrix | None = None   # rows in insertion order (raw plane only)
         self._assign = None                   # i64[ntotal] list of every row
+        self._ids = None                      # i64[ntotal] id of every row
         self._lists = None                    # dict built lazily: packed planes in list order
 
     @property
@@ -643,23 +853,48 @@ class IndexIVFFlat:
         self.is_trained = True
 
     def add(self, x):
+        self.add_with_ids(x, None)
+
+    def add_with_ids(self, x, ids):
+        """ids: int64 numpy array or tensor of length n; None numbers the rows from ntotal."""
         if not self.is_trained:
             raise RuntimeError("Error: 'is_trained' failed")
         t, _ = _to_device_f32(x)
         assert t.shape[1] == self.d
+        n0 = self.ntotal
+        ids = torch.arange(n0, n0 + t.shape[0], dtype=torch.int64, device=t.device) if ids is None else \
+            _ids_arg(ids, t.shape[0], t.device)
         if self._x is None:
             self._x = PackedMatrix(self.d, t.device, planes=("raw",))
         q = PackedMatrix.from_tensor(t, planes=self.quantizer._query_planes(1))
         _, a = self.quantizer.search_packed(q, 1)
         a = a.reshape(-1)
-        self._assign = a if self._assign is None or self._x.n == 0 else torch.cat([self._assign, a])
+        self._assign = a if self._assign is None or n0 == 0 else torch.cat([self._assign, a])
+        self._ids = ids if self._ids is None or n0 == 0 else torch.cat([self._ids, ids])
         self._x.append(t)
         self._lists = None
+
+    def remove_ids(self, sel) -> int:
+        """faiss IndexIVF::remove_ids: selects on the row ids; the rows, their lists and their ids are
+        compacted with one stable partition and the lists are rebuilt on the next search, as after
+        add(). Returns the number of rows removed."""
+        sel = _selector(sel)
+        n = self.ntotal
+        if n == 0:
+            return 0
+        order, removed = _keep_partition(sel, self._ids, n, self._x.device)
+        if removed:
+            self._x = _gather_packed(self._x, order)
+            self._assign = _gather_i64(self._assign, order)
+            self._ids = _gather_i64(self._ids, order)
+            self._lists = None
+        return removed
 
     def reset(self):
         if self._x is not None:
             self._x.clear()
         self._assign = None
+        self._ids = None
         self._lists = None
 
     def _build_lists(self):
@@ -691,7 +926,7 @@ class IndexIVFFlat:
                 packed.h16_scale = _h16_scale_for(packed.max_norm)
                 check(lib.nrb_pack_rows_h16(raw.data_ptr(), n, self.d, kp, kp, packed.h16_scale,
                                             packed.h16.data_ptr(), 0, _stream()), "pack_rows_h16")
-        ids = order[:n].to(torch.int64)  # ids are sequential: id = insertion row
+        ids = _gather_i64(self._ids, order[:n])
         off_h = _to_host(offsets).astype(np.int64)
         sizes = np.diff(off_h)
         self._lists = dict(packed=packed, ids=ids, offsets=offsets, offsets_host=off_h,

@@ -4,4 +4,5 @@ can never shadow a real faiss that is used as an oracle."""
 from newsrecommend_b200.faiss import *  # noqa: F401,F403
 from newsrecommend_b200.faiss import (METRIC_INNER_PRODUCT, METRIC_L2, Clustering,  # noqa: F401
                                       ClusteringParameters, IndexFlat, IndexFlatIP, IndexFlatL2,
-                                      IndexHNSWFlat, IndexIVFFlat, normalize_L2, vector_float_to_array)
+                                      IndexHNSWFlat, IndexIDMap, IndexIVFFlat, IDSelectorBatch, IDSelectorRange,
+                                      normalize_L2, vector_float_to_array)
