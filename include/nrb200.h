@@ -258,6 +258,26 @@ int nrb_ivf_scan_small(const float* xq, int64_t ldq, int32_t nq, int32_t d, cons
                        const int32_t* offsets, int32_t nlist, int32_t max_list_len, const int64_t* ids,
                        const int64_t* coarse, int32_t nprobe, int32_t metric, int32_t k, float* D, int64_t* I,
                        void* workspace, size_t workspace_bytes, void* stream);
+/* Search-time ID selectors (faiss SearchParameters::sel) on the three routes above: the same calls
+ * with two more arguments, member i64 (device; nrb_id_select's output) and keep. Only the rows with
+ * member[row] == keep take part; keep = 0 evaluates faiss's IDSelectorNot of the selector that
+ * produced member, with no extra pass. member is indexed like the plane the kernel scans: catalog
+ * rows (b) for the flat forms, packed list rows (lists, the order of ids) for the IVF scan. A warp
+ * skips the row load of an unselected row, and the selection treats such rows as absent, not as low
+ * scores: when fewer than k rows qualify, the result is padded exactly as for k > n (I = -1,
+ * D = -FLT_MAX / +FLT_MAX).
+ * Workspaces as for the unfiltered calls; nrb_search_small_host_sel stays one synchronous call and
+ * runs after the kernel that wrote member when both are queued on `stream`. */
+int nrb_search_small_sel(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* b, int32_t metric,
+                         int32_t k, int64_t id_base, float* D, int64_t* I, void* workspace, size_t workspace_bytes,
+                         void* stream, const int64_t* member, int64_t keep);
+int nrb_search_small_host_sel(const nrb_matrix* b, const float* xq_host, int32_t nq, int32_t d, int32_t metric, int32_t k,
+                              int64_t id_base, float* D_host, int64_t* I_host, void* stream, const int64_t* member,
+                              int64_t keep);
+int nrb_ivf_scan_small_sel(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* lists,
+                           const int32_t* offsets, int32_t nlist, int32_t max_list_len, const int64_t* ids,
+                           const int64_t* coarse, int32_t nprobe, int32_t metric, int32_t k, float* D, int64_t* I,
+                           void* workspace, size_t workspace_bytes, void* stream, const int64_t* member, int64_t keep);
 
 /* Retrieval.py:6-8 on the device (SURVEY 8f row 1): table f64[n, width] = embedding values followed by
  * the article id (news/article_table.npy) -> emb f32[n, width-1] C-contiguous, ids i64[n]. */
@@ -280,6 +300,12 @@ int nrb_id_select(const int64_t* ids, int64_t n, const int64_t* batch, int64_t n
                   int64_t imax, int64_t* member, void* workspace, size_t workspace_bytes, void* stream);
 /* IndexIDMap::search's label translation, in place: I[i] = I[i] < 0 ? I[i] : id_map[I[i]]. */
 int nrb_map_ids(const int64_t* id_map, int64_t* I, int64_t n, void* stream);
+/* Bucket keys of a filtered IVF scan: out[i] = member[i] == keep ? key[i] : drop. With key = the
+ * list of every row and drop = nlist, nrb_ivf_build_lists(out, n, nlist + 1, ...) lays out the lists
+ * of the selected rows only (in the same order as the unfiltered lists) and puts the rest in bucket
+ * nlist, which the scan never reads. */
+int nrb_sel_keys(const int64_t* member, int64_t keep, const int64_t* key, int64_t n, int64_t drop, int64_t* out,
+                 void* stream);
 
 /* Wire format of the all-to-all by query range (the exchange step of the catalog-sharded search):
  * P[i] = (fp32 bits of D[i]) << 32 | uint32(I[i] - id_base), 0xffffffff in the low word when

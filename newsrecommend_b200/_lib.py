@@ -35,6 +35,7 @@ SYMBOLS = [
     "nrb_search_small_workspace", "nrb_search_small", "nrb_search_small_host",
     "nrb_ivf_scan_small_workspace", "nrb_ivf_scan_small", "nrb_split_table_f64",
     "nrb_id_select_workspace", "nrb_id_select", "nrb_map_ids",
+    "nrb_search_small_sel", "nrb_search_small_host_sel", "nrb_ivf_scan_small_sel", "nrb_sel_keys",
 ]
 
 
@@ -107,6 +108,10 @@ lib.nrb_id_select_workspace.restype = _sz
 lib.nrb_id_select_workspace.argtypes = [_i64]
 lib.nrb_id_select.argtypes = [_vp, _i64, _vp, _i64, _i64, _i64, _vp, _vp, _sz, _vp]
 lib.nrb_map_ids.argtypes = [_vp, _vp, _i64, _vp]
+lib.nrb_search_small_sel.argtypes = lib.nrb_search_small.argtypes + [_vp, _i64]
+lib.nrb_search_small_host_sel.argtypes = lib.nrb_search_small_host.argtypes + [_vp, _i64]
+lib.nrb_ivf_scan_small_sel.argtypes = lib.nrb_ivf_scan_small.argtypes + [_vp, _i64]
+lib.nrb_sel_keys.argtypes = [_vp, _i64, _vp, _i64, _i64, _vp, _vp]
 
 
 def last_error() -> str:

@@ -1570,6 +1570,13 @@ __global__ void map_ids_kernel(const int64_t* __restrict__ id_map, int64_t* __re
     }
 }
 
+// out[i] = member[i] == keep ? key[i] : drop: the list of every selected row, and bucket `drop` for the rest
+__global__ void sel_keys_kernel(const int64_t* __restrict__ member, int64_t keep, const int64_t* __restrict__ key,
+                                int64_t n, int64_t drop, int64_t* __restrict__ out) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
+        out[i] = member[i] == keep ? key[i] : drop;
+}
+
 extern "C" size_t nrb_id_select_workspace(int64_t nbatch) {
     if (nbatch <= 0) return 0;
     return 256 + (size_t)id_table_cap(nbatch) * sizeof(int64_t);
@@ -1626,6 +1633,19 @@ extern "C" int nrb_map_ids(const int64_t* id_map, int64_t* I, int64_t n, void* s
     int64_t blocks = (n + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
     map_ids_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(id_map, I, n);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}
+
+extern "C" int nrb_sel_keys(const int64_t* member, int64_t keep, const int64_t* key, int64_t n, int64_t drop, int64_t* out,
+                            void* stream) {
+    NRB_REQUIRE(n >= 0 && (n == 0 || (member && key && out)), "sel_keys: bad arguments");
+    if (n == 0) return NRB_OK;
+    int rc = require_device();
+    if (rc) return rc;
+    int64_t blocks = (n + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    sel_keys_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(member, keep, key, n, drop, out);
     NRB_LAUNCH_CHECK();
     return NRB_OK;
 }

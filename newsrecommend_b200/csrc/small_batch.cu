@@ -17,9 +17,17 @@
 //
 // Algorithmic bytes: flat n * kp * 4 per group of <= 16 queries; IVF sum over (query, probed list)
 // of |list| * kp * 4 (SURVEY 8d "small nq: HBM").
+//
+// Search-time ID selectors (faiss SearchParameters::sel): the MASKED instantiations take a row mask
+// member i64[n] (nrb_id_select's output, in the order of the plane the kernel scans) and a keep value.
+// A warp reads member[row] first and skips the row load of an unselected row; its score slot gets
+// absent_score(), which the masked selection sources map to the ordered key 0, below every real key
+// (even -inf). Absent rows therefore sort after every selected row, and the result writers turn a
+// candidate with ordered key 0 into padding (I = -1), so an unselected row never appears in a result.
 #include <float.h>
 #include <mutex>
 #include <string.h>
+#include <type_traits>
 
 #include "common.cuh"
 #include "internal.h"
@@ -61,9 +69,10 @@ __device__ __forceinline__ float warp_reduce_multi(float (&acc)[QG], int lane) {
 // R rows (one per pointer) against QG queries held in shared memory (qs[q * kp + c]); kp % 32 == 0.
 // Lane l owns columns [c*128 + 4l, c*128 + 4l + 4) of every 128-column chunk c. The loads of all R
 // rows are issued before any arithmetic: R x 16 bytes in flight per lane and chunk.
-template <int QG, bool L2, int R>
+// MASKED: only the rows whose bit is set in `use` are loaded (the others contribute zeros).
+template <int QG, bool L2, int R, bool MASKED = false>
 __device__ __forceinline__ void rows_scores(const float* const (&row)[R], const float* qs, int kp, int lane,
-                                            float (&out)[R]) {
+                                            float (&out)[R], unsigned use = ~0u) {
     float acc[R][QG];
 #pragma unroll
     for (int r = 0; r < R; r++)
@@ -74,7 +83,9 @@ __device__ __forceinline__ void rows_scores(const float* const (&row)[R], const 
         if (col < kp) {
             float4 x[R];
 #pragma unroll
-            for (int r = 0; r < R; r++) x[r] = __ldg(reinterpret_cast<const float4*>(row[r] + col));
+            for (int r = 0; r < R; r++)
+                x[r] = (!MASKED || ((use >> r) & 1u)) ? __ldg(reinterpret_cast<const float4*>(row[r] + col))
+                                                      : make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
             for (int q = 0; q < QG; q++) {
                 const float4 y = *reinterpret_cast<const float4*>(qs + q * kp + col);
@@ -118,6 +129,14 @@ __device__ __forceinline__ void stage_queries(const float* __restrict__ xq, int6
         qs[t] = (q0 + q < nq && c < d) ? xq[(int64_t)(q0 + q) * ldq + c] : 0.f;
     }
 }
+
+// Score of a row a MASKED kernel skipped: the NaN bit pattern 0xffffffff, which fp32 arithmetic never
+// produces (it yields the canonical NaN 0x7fffffff). MaskedScoreSrc tests these bits before any
+// arithmetic (negating a NaN leaves its sign unspecified) and returns them as the key: ordered_u32 == 0.
+constexpr unsigned ABSENT_BITS = 0xffffffffu;
+__device__ __forceinline__ float absent_score() { return __uint_as_float(ABSENT_BITS); }
+// a sorted candidate that stands for an absent row (packed key word 0)
+__device__ __forceinline__ bool absent_cand(unsigned long long c) { return (c >> 32) == 0; }
 
 // ------------------------------------------------------------------ block-wide exact top-k
 // Keys are "larger is better" (score, or -distance). Radix select over the ordered-uint image of
@@ -246,6 +265,19 @@ struct ScoreSrc {
     __device__ __forceinline__ float key(int i) const { const float v = p[i]; return l2 ? -v : v; }
     __device__ __forceinline__ int pos(int i) const { return base + i; }
 };
+// the same for the score rows of the MASKED kernels: an absent row keeps the key ABSENT_BITS
+struct MaskedScoreSrc {
+    const float* p;
+    int base;
+    bool l2;
+    __device__ __forceinline__ float key(int i) const {
+        const float v = p[i];
+        return __float_as_uint(v) == ABSENT_BITS ? __uint_as_float(ABSENT_BITS) : (l2 ? -v : v);
+    }
+    __device__ __forceinline__ int pos(int i) const { return base + i; }
+};
+template <bool MASKED>
+using ScoreSrcT = typename std::conditional<MASKED, MaskedScoreSrc, ScoreSrc>::type;
 // packed-candidate source (second level of the two-level selection)
 struct CandSrc {
     const unsigned long long* c;
@@ -254,10 +286,10 @@ struct CandSrc {
 };
 
 // ------------------------------------------------------------------ flat
-template <int QG, bool L2, int R>
+template <int QG, bool L2, int R, bool MASKED>
 __global__ void __launch_bounds__(SMALL_THREADS)
 small_scores_kernel(const float* __restrict__ xq, int64_t ldq, int nq, int d, const float* __restrict__ xb, int64_t nb,
-                    int kp, float* __restrict__ scores) {
+                    int kp, float* __restrict__ scores, const int64_t* __restrict__ member, int64_t keep) {
     extern __shared__ __align__(16) float qs[];
     const int q0 = blockIdx.y * QG;
     stage_queries<QG>(xq, ldq, d, kp, q0, nq, qs);
@@ -269,26 +301,35 @@ small_scores_kernel(const float* __restrict__ xq, int64_t ldq, int nq, int d, co
     const bool writer = (lane % LPQ) == 0 && q0 + q < nq;
     for (int64_t r = (int64_t)blockIdx.x * (SMALL_THREADS / 32) + (threadIdx.x >> 5); r < nb; r += warps * R) {
         const float* rows[R];
+        unsigned use = 0;
 #pragma unroll
         for (int j = 0; j < R; j++) {
             const int64_t rj = r + j * warps;
             rows[j] = xb + (rj < nb ? rj : r) * kp;
+            if (MASKED && rj < nb && member[rj] == keep) use |= 1u << j;
         }
         float out[R];
-        rows_scores<QG, L2, R>(rows, qs, kp, lane, out);
+        if (MASKED && use == 0) {
+#pragma unroll
+            for (int j = 0; j < R; j++) out[j] = 0.f;
+        } else {
+            rows_scores<QG, L2, R, MASKED>(rows, qs, kp, lane, out, use);
+        }
 #pragma unroll
         for (int j = 0; j < R; j++) {
             const int64_t rj = r + j * warps;
-            if (writer && rj < nb) scores[(int64_t)(q0 + q) * nb + rj] = out[j];
+            if (writer && rj < nb)
+                scores[(int64_t)(q0 + q) * nb + rj] = (!MASKED || ((use >> j) & 1u)) ? out[j] : absent_score();
         }
     }
 }
 
-// results of one query from the sorted candidates in S.cand
+// results of one query from the sorted candidates in S.cand (MASKED: absent rows become padding)
+template <bool MASKED>
 __device__ __forceinline__ void write_flat_results(const SelectShared& S, int kk, int k, bool l2, int64_t id_base,
                                                    float* __restrict__ Dq, int64_t* __restrict__ Iq) {
     for (int e = threadIdx.x; e < k; e += blockDim.x) {
-        const int ps = e < kk ? cand_idx(S.cand[e]) : -1;
+        const int ps = e < kk && !(MASKED && absent_cand(S.cand[e])) ? cand_idx(S.cand[e]) : -1;
         const float key = cand_key(S.cand[e < kk ? e : 0]);
         Dq[e] = ps < 0 ? (l2 ? FLT_MAX : -FLT_MAX) : (l2 ? -key : key);
         Iq[e] = ps < 0 ? -1 : id_base + ps;
@@ -296,18 +337,20 @@ __device__ __forceinline__ void write_flat_results(const SelectShared& S, int kk
 }
 
 // one level: block per query over the whole score row
+template <bool MASKED>
 __global__ void __launch_bounds__(1024)
 small_select_kernel(const float* __restrict__ scores, int64_t ld, int n, int k, int l2, int64_t id_base,
                     float* __restrict__ D, int64_t* __restrict__ I) {
     __shared__ SelectShared S;
     const int q = blockIdx.x;
-    ScoreSrc src{scores + (int64_t)q * ld, 0, l2 != 0};
+    ScoreSrcT<MASKED> src{scores + (int64_t)q * ld, 0, l2 != 0};
     const int kk = block_select(src, n, k, S);
-    write_flat_results(S, kk, k, l2 != 0, id_base, D + (int64_t)q * k, I + (int64_t)q * k);
+    write_flat_results<MASKED>(S, kk, k, l2 != 0, id_base, D + (int64_t)q * k, I + (int64_t)q * k);
 }
 
 // two levels for long rows: block (b, q) selects the top-k of slice b of query q's scores into
 // cands[q][b][k] (padded with empty candidates); small_select2_kernel then selects among the B*k.
+template <bool MASKED>
 __global__ void __launch_bounds__(1024)
 small_select1_kernel(const float* __restrict__ scores, int64_t ld, int n, int k, int l2,
                      unsigned long long* __restrict__ cands) {
@@ -315,12 +358,13 @@ small_select1_kernel(const float* __restrict__ scores, int64_t ld, int n, int k,
     const int q = blockIdx.y, b = blockIdx.x, B = gridDim.x;
     const int per = (n + B - 1) / B;
     const int lo = min(n, b * per), hi = min(n, lo + per);
-    ScoreSrc src{scores + (int64_t)q * ld + lo, lo, l2 != 0};
+    ScoreSrcT<MASKED> src{scores + (int64_t)q * ld + lo, lo, l2 != 0};
     const int kk = block_select(src, hi - lo, k, S);
     unsigned long long* out = cands + ((int64_t)q * B + b) * k;
     for (int e = threadIdx.x; e < k; e += blockDim.x) out[e] = e < kk ? S.cand[e] : empty_cand();
 }
 
+template <bool MASKED>
 __global__ void __launch_bounds__(1024)
 small_select2_kernel(const unsigned long long* __restrict__ cands, int B, int k, int l2, int64_t id_base,
                      float* __restrict__ D, int64_t* __restrict__ I) {
@@ -328,14 +372,15 @@ small_select2_kernel(const unsigned long long* __restrict__ cands, int B, int k,
     const int q = blockIdx.x;
     CandSrc src{cands + (int64_t)q * B * k};
     const int kk = block_select(src, B * k, k, S);
-    write_flat_results(S, kk, k, l2 != 0, id_base, D + (int64_t)q * k, I + (int64_t)q * k);
+    write_flat_results<MASKED>(S, kk, k, l2 != 0, id_base, D + (int64_t)q * k, I + (int64_t)q * k);
 }
 
 // n <= FUSED_MAX_ROWS: one block per query computes the scores into shared memory and selects.
-template <bool L2>
+template <bool L2, bool MASKED>
 __global__ void __launch_bounds__(SMALL_THREADS)
 small_fused_kernel(const float* __restrict__ xq, int64_t ldq, int nq, int d, const float* __restrict__ xb, int n, int kp,
-                   int k, int64_t id_base, float* __restrict__ D, int64_t* __restrict__ I) {
+                   int k, int64_t id_base, float* __restrict__ D, int64_t* __restrict__ I,
+                   const int64_t* __restrict__ member, int64_t keep) {
     extern __shared__ __align__(16) float sm[];
     float* qs = sm;            // [kp]
     float* sc = sm + kp;       // [n]
@@ -347,18 +392,27 @@ small_fused_kernel(const float* __restrict__ xq, int64_t ldq, int nq, int d, con
     constexpr int W = SMALL_THREADS / 32, R = 4;
     for (int r = threadIdx.x >> 5; r < n; r += W * R) {
         const float* rows[R];
+        unsigned use = 0;
 #pragma unroll
-        for (int j = 0; j < R; j++) rows[j] = xb + (int64_t)(r + j * W < n ? r + j * W : r) * kp;
+        for (int j = 0; j < R; j++) {
+            rows[j] = xb + (int64_t)(r + j * W < n ? r + j * W : r) * kp;
+            if (MASKED && r + j * W < n && member[r + j * W] == keep) use |= 1u << j;
+        }
         float out[R];
-        rows_scores<1, L2, R>(rows, qs, kp, lane, out);
+        if (MASKED && use == 0) {
+#pragma unroll
+            for (int j = 0; j < R; j++) out[j] = 0.f;
+        } else {
+            rows_scores<1, L2, R, MASKED>(rows, qs, kp, lane, out, use);
+        }
 #pragma unroll
         for (int j = 0; j < R; j++)
-            if (lane == 0 && r + j * W < n) sc[r + j * W] = out[j];
+            if (lane == 0 && r + j * W < n) sc[r + j * W] = (!MASKED || ((use >> j) & 1u)) ? out[j] : absent_score();
     }
     __syncthreads();
-    ScoreSrc src{sc, 0, L2};
+    ScoreSrcT<MASKED> src{sc, 0, L2};
     const int kk = block_select(src, n, k, S);
-    write_flat_results(S, kk, k, L2, id_base, D + (int64_t)q * k, I + (int64_t)q * k);
+    write_flat_results<MASKED>(S, kk, k, L2, id_base, D + (int64_t)q * k, I + (int64_t)q * k);
 }
 
 // ------------------------------------------------------------------ IVF (HBM-regime list scan)
@@ -367,11 +421,11 @@ small_fused_kernel(const float* __restrict__ xq, int64_t ldq, int nq, int d, con
 // 128-bit loads of the list-contiguous raw plane; scores[q*ld + prefix(q, p) + r].
 constexpr int IVF_CHUNK = 256;
 
-template <bool L2>
+template <bool L2, bool MASKED>
 __global__ void __launch_bounds__(SMALL_THREADS)
 ivf_small_scores_kernel(const float* __restrict__ xq, int64_t ldq, int d, const float* __restrict__ xb, int kp,
                         const int* __restrict__ offsets, const int64_t* __restrict__ coarse, int nprobe,
-                        float* __restrict__ scores, int64_t ld) {
+                        float* __restrict__ scores, int64_t ld, const int64_t* __restrict__ member, int64_t keep) {
     extern __shared__ __align__(16) float qs[];
     const int q = blockIdx.y / nprobe, p = blockIdx.y - q * nprobe;
     const int64_t l = coarse[(int64_t)q * nprobe + p];
@@ -391,13 +445,23 @@ ivf_small_scores_kernel(const float* __restrict__ xq, int64_t ldq, int d, const 
     constexpr int W = SMALL_THREADS / 32, R = 4;
     for (int r = c0 + (threadIdx.x >> 5); r < c1; r += W * R) {
         const float* rows[R];
+        unsigned use = 0;
 #pragma unroll
-        for (int j = 0; j < R; j++) rows[j] = xb + (int64_t)(row0 + (r + j * W < c1 ? r + j * W : r)) * kp;
+        for (int j = 0; j < R; j++) {
+            rows[j] = xb + (int64_t)(row0 + (r + j * W < c1 ? r + j * W : r)) * kp;
+            if (MASKED && r + j * W < c1 && member[row0 + r + j * W] == keep) use |= 1u << j;
+        }
         float out[R];
-        rows_scores<1, L2, R>(rows, qs, kp, lane, out);
+        if (MASKED && use == 0) {
+#pragma unroll
+            for (int j = 0; j < R; j++) out[j] = 0.f;
+        } else {
+            rows_scores<1, L2, R, MASKED>(rows, qs, kp, lane, out, use);
+        }
 #pragma unroll
         for (int j = 0; j < R; j++)
-            if (lane == 0 && r + j * W < c1) scores[(int64_t)q * ld + prefix + r + j * W] = out[j];
+            if (lane == 0 && r + j * W < c1)
+                scores[(int64_t)q * ld + prefix + r + j * W] = (!MASKED || ((use >> j) & 1u)) ? out[j] : absent_score();
     }
 }
 
@@ -418,11 +482,12 @@ __device__ __forceinline__ int ivf_segments(const int* __restrict__ offsets, con
     return seg_end[nprobe - 1];
 }
 
+template <bool MASKED>
 __device__ __forceinline__ void write_ivf_results(const SelectShared& S, int kk, int k, bool l2, const int* seg_end,
                                                   const int* seg_row0, const int64_t* __restrict__ ids,
                                                   float* __restrict__ Dq, int64_t* __restrict__ Iq) {
     for (int e = threadIdx.x; e < k; e += blockDim.x) {
-        const int ps = e < kk ? cand_idx(S.cand[e]) : -1;
+        const int ps = e < kk && !(MASKED && absent_cand(S.cand[e])) ? cand_idx(S.cand[e]) : -1;
         const float key = cand_key(S.cand[e < kk ? e : 0]);
         int64_t id = -1;
         if (ps >= 0) {
@@ -436,6 +501,7 @@ __device__ __forceinline__ void write_ivf_results(const SelectShared& S, int kk,
 }
 
 // level 1: block (b, q) selects over slice b of query q's concatenated list scores
+template <bool MASKED>
 __global__ void __launch_bounds__(1024)
 ivf_small_select1_kernel(const float* __restrict__ scores, int64_t ld, const int* __restrict__ offsets,
                          const int64_t* __restrict__ coarse, int nprobe, int k, int l2,
@@ -446,12 +512,13 @@ ivf_small_select1_kernel(const float* __restrict__ scores, int64_t ld, const int
     const int n = ivf_segments(offsets, coarse + (int64_t)q * nprobe, nprobe, seg_end, seg_row0);
     const int per = (n + B - 1) / B;
     const int lo = min(n, b * per), hi = min(n, lo + per);
-    ScoreSrc src{scores + (int64_t)q * ld + lo, lo, l2 != 0};
+    ScoreSrcT<MASKED> src{scores + (int64_t)q * ld + lo, lo, l2 != 0};
     const int kk = block_select(src, hi - lo, k, S);
     unsigned long long* out = cands + ((int64_t)q * B + b) * k;
     for (int e = threadIdx.x; e < k; e += blockDim.x) out[e] = e < kk ? S.cand[e] : empty_cand();
 }
 
+template <bool MASKED>
 __global__ void __launch_bounds__(1024)
 ivf_small_select2_kernel(const unsigned long long* __restrict__ cands, int B, const int* __restrict__ offsets,
                          const int64_t* __restrict__ coarse, int nprobe, const int64_t* __restrict__ ids, int k, int l2,
@@ -462,7 +529,7 @@ ivf_small_select2_kernel(const unsigned long long* __restrict__ cands, int B, co
     ivf_segments(offsets, coarse + (int64_t)q * nprobe, nprobe, seg_end, seg_row0);
     CandSrc src{cands + (int64_t)q * B * k};
     const int kk = block_select(src, B * k, k, S);
-    write_ivf_results(S, kk, k, l2 != 0, seg_end, seg_row0, ids, D + (int64_t)q * k, I + (int64_t)q * k);
+    write_ivf_results<MASKED>(S, kk, k, l2 != 0, seg_end, seg_row0, ids, D + (int64_t)q * k, I + (int64_t)q * k);
 }
 
 // ------------------------------------------------------------------ exact k = 1 fallback (no host round trip)
@@ -550,40 +617,63 @@ static SmallWs carve_small(void* ws, int64_t nq, int64_t ld, int B, int k) {
     return s;
 }
 
-template <bool L2>
+// member == nullptr: every row (the unmasked kernels); else the rows with member[row] == keep
+template <bool L2, bool MASKED>
 static int small_flat_launch(const float* xq, int64_t ldq, int nq, int d, const nrb_matrix* b, int k, int64_t id_base,
-                             void* workspace, float* D, int64_t* I, cudaStream_t st) {
+                             void* workspace, float* D, int64_t* I, const int64_t* member, int64_t keep, cudaStream_t st) {
     const int kp = b->kp;
     const int n = (int)b->n;
     if (b->n <= FUSED_MAX_ROWS) {
         const size_t sh = (size_t)(kp + n) * sizeof(float);
-        small_fused_kernel<L2><<<nq, SMALL_THREADS, sh, st>>>(xq, ldq, nq, d, b->raw, n, kp, k, id_base, D, I);
+        small_fused_kernel<L2, MASKED><<<nq, SMALL_THREADS, sh, st>>>(xq, ldq, nq, d, b->raw, n, kp, k, id_base, D, I,
+                                                                     member, keep);
         NRB_LAUNCH_CHECK();
         return NRB_OK;
     }
     const int B = select_slices(n);
     const SmallWs w = carve_small(workspace, nq, n, B, k);
     if (nq == 1) {
-        small_scores_kernel<1, L2, 4><<<dim3(small_grid_rows(n, 4), 1), SMALL_THREADS, kp * sizeof(float), st>>>(
-            xq, ldq, nq, d, b->raw, b->n, kp, w.scores);
+        small_scores_kernel<1, L2, 4, MASKED><<<dim3(small_grid_rows(n, 4), 1), SMALL_THREADS, kp * sizeof(float), st>>>(
+            xq, ldq, nq, d, b->raw, b->n, kp, w.scores, member, keep);
     } else if (nq <= 4) {
-        small_scores_kernel<4, L2, 4><<<dim3(small_grid_rows(n, 4), 1), SMALL_THREADS, 4 * kp * sizeof(float), st>>>(
-            xq, ldq, nq, d, b->raw, b->n, kp, w.scores);
+        small_scores_kernel<4, L2, 4, MASKED><<<dim3(small_grid_rows(n, 4), 1), SMALL_THREADS, 4 * kp * sizeof(float), st>>>(
+            xq, ldq, nq, d, b->raw, b->n, kp, w.scores, member, keep);
     } else {
-        small_scores_kernel<SMALL_QG, L2, 4><<<dim3(small_grid_rows(n, 4), (nq + SMALL_QG - 1) / SMALL_QG), SMALL_THREADS,
-                                               SMALL_QG * kp * sizeof(float), st>>>(xq, ldq, nq, d, b->raw, b->n, kp, w.scores);
+        small_scores_kernel<SMALL_QG, L2, 4, MASKED><<<dim3(small_grid_rows(n, 4), (nq + SMALL_QG - 1) / SMALL_QG),
+                                                       SMALL_THREADS, SMALL_QG * kp * sizeof(float), st>>>(
+            xq, ldq, nq, d, b->raw, b->n, kp, w.scores, member, keep);
     }
     NRB_LAUNCH_CHECK();
     if (B == 1) {
-        small_select_kernel<<<nq, n <= 4096 ? 256 : 1024, 0, st>>>(w.scores, n, n, k, L2 ? 1 : 0, id_base, D, I);
+        small_select_kernel<MASKED><<<nq, n <= 4096 ? 256 : 1024, 0, st>>>(w.scores, n, n, k, L2 ? 1 : 0, id_base, D, I);
         NRB_LAUNCH_CHECK();
     } else {
-        small_select1_kernel<<<dim3(B, nq), 1024, 0, st>>>(w.scores, n, n, k, L2 ? 1 : 0, w.cands);
+        small_select1_kernel<MASKED><<<dim3(B, nq), 1024, 0, st>>>(w.scores, n, n, k, L2 ? 1 : 0, w.cands);
         NRB_LAUNCH_CHECK();
-        small_select2_kernel<<<nq, B * k <= 2048 ? 256 : 1024, 0, st>>>(w.cands, B, k, L2 ? 1 : 0, id_base, D, I);
+        small_select2_kernel<MASKED><<<nq, B * k <= 2048 ? 256 : 1024, 0, st>>>(w.cands, B, k, L2 ? 1 : 0, id_base, D, I);
         NRB_LAUNCH_CHECK();
     }
     return NRB_OK;
+}
+
+static int search_small_impl(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* b, int32_t metric,
+                             int32_t k, int64_t id_base, float* D, int64_t* I, void* workspace, size_t workspace_bytes,
+                             const int64_t* member, int64_t keep, void* stream) {
+    NRB_REQUIRE(b && b->raw && b->n > 0 && b->n < (1LL << 31), "search_small: the item matrix needs its raw plane (0 < n < 2^31)");
+    NRB_REQUIRE(nq > 0 && nq <= NRB_SMALL_MAX_NQ && k > 0 && k <= SELECT_MAX_K && d == b->d && b->kp % 32 == 0 && b->kp <= 2048,
+                "search_small: bad sizes (nq <= %d, k <= %d)", NRB_SMALL_MAX_NQ, SELECT_MAX_K);
+    NRB_REQUIRE(xq && D && I && ldq >= d, "search_small: null argument");
+    NRB_REQUIRE(workspace_bytes >= nrb_search_small_workspace(nq, b->n, k) && (workspace || b->n <= FUSED_MAX_ROWS),
+                "search_small: workspace too small");
+    if (!tc_available()) return NRB_ERR_NO_DEVICE;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (member)
+        return metric == NRB_METRIC_L2
+                   ? small_flat_launch<true, true>(xq, ldq, nq, d, b, k, id_base, workspace, D, I, member, keep, st)
+                   : small_flat_launch<false, true>(xq, ldq, nq, d, b, k, id_base, workspace, D, I, member, keep, st);
+    return metric == NRB_METRIC_L2
+               ? small_flat_launch<true, false>(xq, ldq, nq, d, b, k, id_base, workspace, D, I, nullptr, 0, st)
+               : small_flat_launch<false, false>(xq, ldq, nq, d, b, k, id_base, workspace, D, I, nullptr, 0, st);
 }
 
 }  // namespace nrb
@@ -598,16 +688,14 @@ extern "C" size_t nrb_search_small_workspace(int64_t nq, int64_t nb, int32_t k) 
 extern "C" int nrb_search_small(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* b, int32_t metric,
                                 int32_t k, int64_t id_base, float* D, int64_t* I, void* workspace, size_t workspace_bytes,
                                 void* stream) {
-    NRB_REQUIRE(b && b->raw && b->n > 0 && b->n < (1LL << 31), "search_small: the item matrix needs its raw plane (0 < n < 2^31)");
-    NRB_REQUIRE(nq > 0 && nq <= NRB_SMALL_MAX_NQ && k > 0 && k <= SELECT_MAX_K && d == b->d && b->kp % 32 == 0 && b->kp <= 2048,
-                "search_small: bad sizes (nq <= %d, k <= %d)", NRB_SMALL_MAX_NQ, SELECT_MAX_K);
-    NRB_REQUIRE(xq && D && I && ldq >= d, "search_small: null argument");
-    NRB_REQUIRE(workspace_bytes >= nrb_search_small_workspace(nq, b->n, k) && (workspace || b->n <= FUSED_MAX_ROWS),
-                "search_small: workspace too small");
-    if (!tc_available()) return NRB_ERR_NO_DEVICE;
-    cudaStream_t st = (cudaStream_t)stream;
-    return metric == NRB_METRIC_L2 ? small_flat_launch<true>(xq, ldq, nq, d, b, k, id_base, workspace, D, I, st)
-                                   : small_flat_launch<false>(xq, ldq, nq, d, b, k, id_base, workspace, D, I, st);
+    return search_small_impl(xq, ldq, nq, d, b, metric, k, id_base, D, I, workspace, workspace_bytes, nullptr, 0, stream);
+}
+
+extern "C" int nrb_search_small_sel(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* b,
+                                    int32_t metric, int32_t k, int64_t id_base, float* D, int64_t* I, void* workspace,
+                                    size_t workspace_bytes, void* stream, const int64_t* member, int64_t keep) {
+    NRB_REQUIRE(member, "search_small_sel: null member");
+    return search_small_impl(xq, ldq, nq, d, b, metric, k, id_base, D, I, workspace, workspace_bytes, member, keep, stream);
 }
 
 // Host arrays in, host arrays out. The staging buffer is page-locked AND mapped into the device
@@ -627,8 +715,9 @@ SmallCache g_small[64];
 std::mutex g_small_mu;
 }  // namespace
 
-extern "C" int nrb_search_small_host(const nrb_matrix* b, const float* xq_host, int32_t nq, int32_t d, int32_t metric,
-                                     int32_t k, int64_t id_base, float* D_host, int64_t* I_host, void* stream) {
+static int search_small_host_impl(const nrb_matrix* b, const float* xq_host, int32_t nq, int32_t d, int32_t metric,
+                                  int32_t k, int64_t id_base, float* D_host, int64_t* I_host, const int64_t* member,
+                                  int64_t keep, void* stream) {
     NRB_REQUIRE(b && xq_host && D_host && I_host && nq > 0 && nq <= NRB_SMALL_MAX_NQ && k > 0 && k <= SELECT_MAX_K && d > 0,
                 "search_small_host: bad arguments");
     int dev = 0;
@@ -660,13 +749,25 @@ extern "C" int nrb_search_small_host(const nrb_matrix* b, const float* xq_host, 
     char* hp = (char*)c.pin;
     char* mp = (char*)c.pin_dev;
     memcpy(hp, xq_host, (size_t)nq * d * sizeof(float));
-    const int rc = nrb_search_small((const float*)mp, d, nq, d, b, metric, k, id_base, (float*)(mp + q_bytes + i_bytes),
-                                    (int64_t*)(mp + q_bytes), c.dev, c.dev_bytes, stream);
+    const int rc = search_small_impl((const float*)mp, d, nq, d, b, metric, k, id_base, (float*)(mp + q_bytes + i_bytes),
+                                     (int64_t*)(mp + q_bytes), c.dev, c.dev_bytes, member, keep, stream);
     if (rc != NRB_OK) return rc;
     NRB_CUDA_CHECK(cudaStreamSynchronize(st));
     memcpy(I_host, hp + q_bytes, (size_t)nq * k * sizeof(int64_t));
     memcpy(D_host, hp + q_bytes + i_bytes, (size_t)nq * k * sizeof(float));
     return NRB_OK;
+}
+
+extern "C" int nrb_search_small_host(const nrb_matrix* b, const float* xq_host, int32_t nq, int32_t d, int32_t metric,
+                                     int32_t k, int64_t id_base, float* D_host, int64_t* I_host, void* stream) {
+    return search_small_host_impl(b, xq_host, nq, d, metric, k, id_base, D_host, I_host, nullptr, 0, stream);
+}
+
+extern "C" int nrb_search_small_host_sel(const nrb_matrix* b, const float* xq_host, int32_t nq, int32_t d, int32_t metric,
+                                         int32_t k, int64_t id_base, float* D_host, int64_t* I_host, void* stream,
+                                         const int64_t* member, int64_t keep) {
+    NRB_REQUIRE(member, "search_small_host_sel: null member");
+    return search_small_host_impl(b, xq_host, nq, d, metric, k, id_base, D_host, I_host, member, keep, stream);
 }
 
 static int64_t ivf_small_ld(int32_t nprobe, int32_t max_list_len, int64_t ntotal) {
@@ -679,10 +780,33 @@ extern "C" size_t nrb_ivf_scan_small_workspace(int64_t nq, int32_t nprobe, int32
     return carve_small(nullptr, nq, ld, select_slices(ld), k).total;
 }
 
-extern "C" int nrb_ivf_scan_small(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* lists,
-                                  const int32_t* offsets, int32_t nlist, int32_t max_list_len, const int64_t* ids,
-                                  const int64_t* coarse, int32_t nprobe, int32_t metric, int32_t k, float* D, int64_t* I,
-                                  void* workspace, size_t workspace_bytes, void* stream) {
+template <bool MASKED>
+static int ivf_small_launch(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* lists,
+                             const int32_t* offsets, int32_t max_list_len, const int64_t* ids, const int64_t* coarse,
+                             int32_t nprobe, int l2, int32_t k, float* D, int64_t* I, const SmallWs& w, int64_t ld, int B,
+                             const int64_t* member, int64_t keep, cudaStream_t st) {
+    const dim3 grid((max_list_len + IVF_CHUNK - 1) / IVF_CHUNK, nq * nprobe);
+    const size_t sh = lists->kp * sizeof(float);
+    if (l2)
+        ivf_small_scores_kernel<true, MASKED><<<grid, SMALL_THREADS, sh, st>>>(xq, ldq, d, lists->raw, lists->kp, offsets,
+                                                                               coarse, nprobe, w.scores, ld, member, keep);
+    else
+        ivf_small_scores_kernel<false, MASKED><<<grid, SMALL_THREADS, sh, st>>>(xq, ldq, d, lists->raw, lists->kp, offsets,
+                                                                                coarse, nprobe, w.scores, ld, member, keep);
+    NRB_LAUNCH_CHECK();
+    ivf_small_select1_kernel<MASKED><<<dim3(B, nq), 1024, 0, st>>>(w.scores, ld, offsets, coarse, nprobe, k, l2, w.cands);
+    NRB_LAUNCH_CHECK();
+    ivf_small_select2_kernel<MASKED><<<nq, B * k <= 2048 ? 256 : 1024, 0, st>>>(w.cands, B, offsets, coarse, nprobe, ids, k,
+                                                                               l2, D, I);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}
+
+static int ivf_scan_small_impl(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* lists,
+                               const int32_t* offsets, int32_t nlist, int32_t max_list_len, const int64_t* ids,
+                               const int64_t* coarse, int32_t nprobe, int32_t metric, int32_t k, float* D, int64_t* I,
+                               void* workspace, size_t workspace_bytes, const int64_t* member, int64_t keep,
+                               void* stream) {
     NRB_REQUIRE(lists && lists->raw && lists->n > 0 && lists->n < (1LL << 31) && d == lists->d && lists->kp % 32 == 0 &&
                     lists->kp <= 2048, "ivf_scan_small: the list matrix needs its raw plane");
     NRB_REQUIRE(nq > 0 && nprobe > 0 && nprobe <= SELECT_MAX_K && nprobe <= nlist && k > 0 && k <= SELECT_MAX_K &&
@@ -696,19 +820,28 @@ extern "C" int nrb_ivf_scan_small(const float* xq, int64_t ldq, int32_t nq, int3
     const int64_t ld = ivf_small_ld(nprobe, max_list_len, lists->n);
     const int B = select_slices(ld);
     const SmallWs w = carve_small(workspace, nq, ld, B, k);
-    const dim3 grid((max_list_len + IVF_CHUNK - 1) / IVF_CHUNK, nq * nprobe);
-    const size_t sh = lists->kp * sizeof(float);
     const int l2 = metric == NRB_METRIC_L2 ? 1 : 0;
-    if (l2)
-        ivf_small_scores_kernel<true><<<grid, SMALL_THREADS, sh, st>>>(xq, ldq, d, lists->raw, lists->kp, offsets, coarse, nprobe,
-                                                                       w.scores, ld);
-    else
-        ivf_small_scores_kernel<false><<<grid, SMALL_THREADS, sh, st>>>(xq, ldq, d, lists->raw, lists->kp, offsets, coarse, nprobe,
-                                                                        w.scores, ld);
-    NRB_LAUNCH_CHECK();
-    ivf_small_select1_kernel<<<dim3(B, nq), 1024, 0, st>>>(w.scores, ld, offsets, coarse, nprobe, k, l2, w.cands);
-    NRB_LAUNCH_CHECK();
-    ivf_small_select2_kernel<<<nq, B * k <= 2048 ? 256 : 1024, 0, st>>>(w.cands, B, offsets, coarse, nprobe, ids, k, l2, D, I);
-    NRB_LAUNCH_CHECK();
-    return NRB_OK;
+    if (member)
+        return ivf_small_launch<true>(xq, ldq, nq, d, lists, offsets, max_list_len, ids, coarse, nprobe, l2, k, D, I, w, ld,
+                                      B, member, keep, st);
+    return ivf_small_launch<false>(xq, ldq, nq, d, lists, offsets, max_list_len, ids, coarse, nprobe, l2, k, D, I, w, ld, B,
+                                   nullptr, 0, st);
+}
+
+extern "C" int nrb_ivf_scan_small(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* lists,
+                                  const int32_t* offsets, int32_t nlist, int32_t max_list_len, const int64_t* ids,
+                                  const int64_t* coarse, int32_t nprobe, int32_t metric, int32_t k, float* D, int64_t* I,
+                                  void* workspace, size_t workspace_bytes, void* stream) {
+    return ivf_scan_small_impl(xq, ldq, nq, d, lists, offsets, nlist, max_list_len, ids, coarse, nprobe, metric, k, D, I,
+                               workspace, workspace_bytes, nullptr, 0, stream);
+}
+
+extern "C" int nrb_ivf_scan_small_sel(const float* xq, int64_t ldq, int32_t nq, int32_t d, const nrb_matrix* lists,
+                                      const int32_t* offsets, int32_t nlist, int32_t max_list_len, const int64_t* ids,
+                                      const int64_t* coarse, int32_t nprobe, int32_t metric, int32_t k, float* D, int64_t* I,
+                                      void* workspace, size_t workspace_bytes, void* stream, const int64_t* member,
+                                      int64_t keep) {
+    NRB_REQUIRE(member, "ivf_scan_small_sel: null member");
+    return ivf_scan_small_impl(xq, ldq, nq, d, lists, offsets, nlist, max_list_len, ids, coarse, nprobe, metric, k, D, I,
+                               workspace, workspace_bytes, member, keep, stream);
 }

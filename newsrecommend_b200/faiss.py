@@ -4,8 +4,18 @@ Mirrors exactly the symbols /root/reference/Retrieval.py uses (Retrieval.py:12-3
 IndexHNSWFlat, IndexFlatL2, vector_float_to_array, index.search) plus the index surface
 BASELINE.json's north_star names (IndexFlatIP, IndexIVFFlat with train/add/search, nlist /
 nprobe / k semantics, METRIC_*, normalize_L2). Semantics follow SURVEY.md section 8b. External
-ids (IndexIDMap, IndexIVFFlat.add_with_ids, remove_ids with IDSelectorBatch / IDSelectorRange) stand
-in for the article-id array that Retrieval.py:7,23 keeps beside the index.
+ids (IndexIDMap, IndexIVFFlat.add_with_ids, remove_ids with IDSelectorBatch / IDSelectorRange /
+IDSelectorNot) stand in for the article-id array that Retrieval.py:7,23 keeps beside the index.
+
+Search-time selectors follow faiss: `index.search(x, k, params=SearchParameters(sel=...))` on the flat
+indexes and IndexIDMap, `SearchParametersIVF(sel=..., nprobe=...)` on IndexIVFFlat. The selector
+tests row positions on a plain flat index, external ids on IndexIDMap and stored ids on IndexIVFFlat
+(whose coarse search still ranks every centroid; only the list scan skips unselected rows). Rows
+that are not selected never appear in a result; when fewer than k rows qualify the tail is padded
+with I = -1 as for k > ntotal. Small batches (the HBM-regime kernels) scan with a row mask; larger
+ones search a compacted copy of the selected rows, built like one add() of those rows, and map the
+labels back on the device, so such a search returns what the same search of an index built from
+only the selected rows returns.
 
 Host code only: every array lives in HBM as torch tensors and all arithmetic is done by
 libnrb200.so (hand-written sm_100a CUDA) through the C-ABI in include/nrb200.h. numpy in ->
@@ -28,8 +38,8 @@ from ._lib import (METRIC_INNER_PRODUCT, METRIC_L2, PATH_AUTO, PATH_SIMT, PATH_T
 
 __all__ = [
     "METRIC_INNER_PRODUCT", "METRIC_L2", "IndexFlat", "IndexFlatL2", "IndexFlatIP", "IndexHNSWFlat",
-    "IndexIVFFlat", "IndexIDMap", "IDSelectorBatch", "IDSelectorRange", "Clustering", "ClusteringParameters",
-    "vector_float_to_array", "normalize_L2",
+    "IndexIVFFlat", "IndexIDMap", "IDSelectorBatch", "IDSelectorRange", "IDSelectorNot", "SearchParameters",
+    "SearchParametersIVF", "Clustering", "ClusteringParameters", "vector_float_to_array", "normalize_L2",
 ]
 
 _FLT_MAX = 3.4028234663852886e38
@@ -283,6 +293,54 @@ class IDSelectorBatch:
         return bool(np.any(self.ids == i))
 
 
+class IDSelectorNot:
+    """faiss.IDSelectorNot: selects the ids `sel` does not. Evaluated as sel's own test with the keep
+    sense flipped (nrb_id_select marks sel's members, the search keeps the others): no extra pass."""
+
+    def __init__(self, sel):
+        if not isinstance(sel, (IDSelectorRange, IDSelectorBatch, IDSelectorNot)):
+            raise TypeError(f"IDSelectorNot wraps an IDSelectorRange, IDSelectorBatch or IDSelectorNot, not {type(sel)}")
+        self.sel = sel
+
+    def is_member(self, i: int) -> bool:
+        return not self.sel.is_member(i)
+
+
+class SearchParameters:
+    """faiss.SearchParameters: per-call search options. sel (an IDSelector, or None) restricts the
+    search to the rows it selects."""
+
+    def __init__(self, sel=None, **fields):
+        if fields:
+            raise TypeError(f"{type(self).__name__}: unsupported field(s) {sorted(fields)}")
+        if sel is not None and not isinstance(sel, (IDSelectorRange, IDSelectorBatch, IDSelectorNot)):
+            raise TypeError(f"sel must be an IDSelectorRange, IDSelectorBatch or IDSelectorNot, not {type(sel)}")
+        self.sel = sel
+
+
+class SearchParametersIVF(SearchParameters):
+    """faiss.SearchParametersIVF: sel as SearchParameters; nprobe, when set, replaces index.nprobe for
+    the call. max_codes (a cap on scanned rows) is not supported: anything but 0 raises."""
+
+    def __init__(self, sel=None, nprobe=None, max_codes=0, **fields):
+        super().__init__(sel, **fields)
+        if max_codes:
+            raise NotImplementedError("SearchParametersIVF.max_codes is not supported (the scan is exhaustive)")
+        self.nprobe = None if nprobe is None else int(nprobe)
+        self.max_codes = 0
+
+
+def _search_sel(params, ivf: bool):
+    """(selector or None, nprobe override or None) of a search's params argument."""
+    if params is None:
+        return None, None
+    if ivf and not isinstance(params, SearchParametersIVF):
+        raise RuntimeError("IndexIVF params have incorrect type")
+    if not isinstance(params, SearchParameters):
+        raise TypeError(f"params must be a SearchParameters, not {type(params)}")
+    return params.sel, getattr(params, "nprobe", None)
+
+
 def _int64_ids(a, what: str) -> np.ndarray:
     """A 1-D host array of integer ids as int64 (floats are refused, not truncated)."""
     if isinstance(a, torch.Tensor):
@@ -296,36 +354,79 @@ def _int64_ids(a, what: str) -> np.ndarray:
 def _selector(sel):
     """remove_ids' argument: an IDSelector, or an id array wrapped in IDSelectorBatch (faiss's
     Python layer does the same)."""
-    if isinstance(sel, (IDSelectorBatch, IDSelectorRange)):
+    if isinstance(sel, (IDSelectorBatch, IDSelectorRange, IDSelectorNot)):
         return sel
     if isinstance(sel, (np.ndarray, torch.Tensor)):
         return IDSelectorBatch(sel)
-    raise TypeError(f"remove_ids takes an IDSelectorBatch, an IDSelectorRange or an int64 id array, not {type(sel)}")
+    raise TypeError("remove_ids takes an IDSelectorBatch, an IDSelectorRange, an IDSelectorNot or an int64 id array, "
+                    f"not {type(sel)}")
 
 
-def _keep_partition(sel, ids, n: int, dev):
-    """Stable keep / remove partition of n rows whose ids are ids (i64 CUDA tensor) or, when ids
-    is None, the row positions: nrb_id_select marks the selected rows, nrb_ivf_build_lists with two
-    buckets puts the rest first in their old order. Returns (order i32 CUDA tensor of the kept rows,
-    number of removed rows); reads one count back, so it synchronises the stream."""
+def _unwrap_not(sel):
+    """(innermost Range / Batch selector, keep): a row is selected when nrb_id_select's member value
+    for that inner selector equals keep (1, or 0 under an odd number of IDSelectorNot)."""
+    keep = 1
+    while isinstance(sel, IDSelectorNot):
+        sel, keep = sel.sel, 1 - keep
+    if not isinstance(sel, (IDSelectorRange, IDSelectorBatch)):
+        raise TypeError(f"expected an IDSelectorRange, IDSelectorBatch or IDSelectorNot, not {type(sel)}")
+    return sel, keep
+
+
+def _select(sel, ids, n: int, dev):
+    """Row mask of a selector over n rows whose ids are ids (i64 CUDA tensor) or, when ids is None,
+    the row positions: (member i64 CUDA tensor from nrb_id_select, keep); row i is selected when
+    member[i] == keep. Queued on the current stream, no synchronisation."""
+    base, keep = _unwrap_not(sel)
     member = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
-    if isinstance(sel, IDSelectorRange):
-        batch, nb, imin, imax = None, 0, sel.imin, sel.imax
+    if isinstance(base, IDSelectorRange):
+        batch, nb, imin, imax = None, 0, base.imin, base.imax
     else:
-        batch = torch.from_numpy(sel.ids).to(dev) if sel.ids.size else None
-        nb, imin, imax = sel.ids.size, 0, 0
+        batch = torch.from_numpy(base.ids).to(dev) if base.ids.size else None
+        nb, imin, imax = base.ids.size, 0, 0
     wsb = lib.nrb_id_select_workspace(nb)
     ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device=dev)
     check(lib.nrb_id_select(_ptr(ids), n, _ptr(batch), nb, imin, imax, member.data_ptr(), ws.data_ptr(), wsb,
                             _stream()), "id_select")
+    return member, keep
+
+
+def _selected_rows(sel, ids, n: int, dev, selected: bool = True) -> torch.Tensor:
+    """The rows a selector picks (selected=True) or leaves (False), in their old order, as an i32
+    CUDA tensor: nrb_id_select marks the rows, nrb_ivf_build_lists with two buckets partitions them
+    stably (member 0 first). Reads one count back, so it synchronises the stream."""
+    member, keep = _select(sel, ids, n, dev)
     offsets = torch.empty(3, dtype=torch.int32, device=dev)
     order = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
     wsb = lib.nrb_ivf_build_lists_workspace(n, 2)
     ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
     check(lib.nrb_ivf_build_lists(member.data_ptr(), n, 2, offsets.data_ptr(), order.data_ptr(), ws.data_ptr(), wsb,
                                   _stream()), "ivf_build_lists")
-    nkeep = int(_to_host(offsets[1:2])[0])
-    return order[:nkeep], n - nkeep
+    n0 = int(_to_host(offsets[1:2])[0])
+    return order[:n0] if (keep if selected else 1 - keep) == 0 else order[n0:n]
+
+
+def _keep_partition(sel, ids, n: int, dev):
+    """remove_ids' stable partition: (order i32 CUDA tensor of the rows sel does not select, number
+    of rows it selects); synchronises the stream once."""
+    order = _selected_rows(sel, ids, n, dev, selected=False)
+    return order, n - order.shape[0]
+
+
+def _positions_kept(sel, n: int):
+    """Number of row positions 0..n-1 a selector keeps, worked out on the host (no device work)."""
+    base, keep = _unwrap_not(sel)
+    if isinstance(base, IDSelectorRange):
+        c = max(0, min(base.imax, n) - max(base.imin, 0))
+    else:
+        c = np.unique(base.ids[(base.ids >= 0) & (base.ids < n)]).size
+    return c if keep else n - c
+
+
+def _padding(nq: int, k: int, metric: int, dev):
+    """The result of a search with no row to return: I = -1, D = -FLT_MAX (IP) / +FLT_MAX (L2)."""
+    D = torch.full((nq, k), _FLT_MAX if metric == METRIC_L2 else -_FLT_MAX, dtype=torch.float32, device=dev)
+    return D, torch.full((nq, k), -1, dtype=torch.int64, device=dev)
 
 
 def _gather_i64(src: torch.Tensor, order: torch.Tensor) -> torch.Tensor:
@@ -410,9 +511,10 @@ class IndexFlat:
             self._struct_cache = self._packed().struct()
         return self._struct_cache
 
-    def _search_small_host(self, a: np.ndarray, k: int, D=None, I=None):
+    def _search_small_host(self, a: np.ndarray, k: int, D=None, I=None, member=None, keep: int = 1):
         """nq < 20, numpy in / numpy out (the call Retrieval.py:32 makes 50,000 times with nq = 1):
-        ONE C-ABI call -- staged H2D, the row-per-warp fp32 kernels, D2H, one sync."""
+        ONE C-ABI call -- staged H2D, the row-per-warp fp32 kernels, D2H, one sync. member / keep:
+        the row mask of a selector (_select), scanned by the masked kernels."""
         nq = a.shape[0]
         if D is None:
             D = np.empty((nq, k), dtype=np.float32)
@@ -420,19 +522,30 @@ class IndexFlat:
             I = np.empty((nq, k), dtype=np.int64)
         assert D.shape == (nq, k) and I.shape == (nq, k) and D.dtype == np.float32 and I.dtype == np.int64
         assert D.flags.c_contiguous and I.flags.c_contiguous, "bad output array"
-        check(lib.nrb_search_small_host(C.byref(self._struct()), a.ctypes.data, nq, self.d, self.metric_type, k, 0,
-                                        D.ctypes.data, I.ctypes.data, _stream()), "search_small_host")
+        if member is None:
+            check(lib.nrb_search_small_host(C.byref(self._struct()), a.ctypes.data, nq, self.d, self.metric_type, k, 0,
+                                            D.ctypes.data, I.ctypes.data, _stream()), "search_small_host")
+        else:
+            check(lib.nrb_search_small_host_sel(C.byref(self._struct()), a.ctypes.data, nq, self.d, self.metric_type, k,
+                                                0, D.ctypes.data, I.ctypes.data, _stream(), member.data_ptr(), keep),
+                  "search_small_host_sel")
         return D, I
 
-    def _search_small_dev(self, t: torch.Tensor, k: int, id_base: int = 0):
+    def _search_small_dev(self, t: torch.Tensor, k: int, id_base: int = 0, member=None, keep: int = 1):
         """The same route for a CUDA tensor batch: asynchronous on the current stream."""
         nq = t.shape[0]
         D = torch.empty((nq, k), dtype=torch.float32, device=t.device)
         I = torch.empty((nq, k), dtype=torch.int64, device=t.device)
         wsb = lib.nrb_search_small_workspace(nq, self.ntotal, k)
         ws = torch.empty(wsb, dtype=torch.uint8, device=t.device)
-        check(lib.nrb_search_small(t.data_ptr(), t.stride(0), nq, self.d, C.byref(self._struct()), self.metric_type, k,
-                                   id_base, D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb, _stream()), "search_small")
+        if member is None:
+            check(lib.nrb_search_small(t.data_ptr(), t.stride(0), nq, self.d, C.byref(self._struct()), self.metric_type,
+                                       k, id_base, D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb, _stream()),
+                  "search_small")
+        else:
+            check(lib.nrb_search_small_sel(t.data_ptr(), t.stride(0), nq, self.d, C.byref(self._struct()),
+                                           self.metric_type, k, id_base, D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb,
+                                           _stream(), member.data_ptr(), keep), "search_small_sel")
         return D, I
 
     def _packed(self) -> PackedMatrix:
@@ -469,10 +582,64 @@ class IndexFlat:
         self._xb = _gather_packed(self._xb, order)
         self._struct_cache = None
 
-    def search(self, x, k: int, D=None, I=None):
+    def search(self, x, k: int, D=None, I=None, *, params=None):
         """(D, I) = search(x, k). Like faiss, optional preallocated numpy outputs D f32[nq,k],
-        I i64[nq,k] are filled and returned (page-locked buffers avoid a staging copy)."""
+        I i64[nq,k] are filled and returned (page-locked buffers avoid a staging copy).
+        params: SearchParameters (or SearchParametersIVF) whose sel selects row positions."""
+        sel, _ = _search_sel(params, False)
+        if sel is not None:
+            return self._search_filtered(x, k, D, I, None, sel)
         return self._search(x, k, D, I, None)
+
+    def _search_filtered(self, x, k: int, D, I, id_map: torch.Tensor | None, sel):
+        """search() over the rows sel selects; sel tests id_map[row] (IndexIDMap) or the row position.
+        Batches that would take the low-latency route (nq < small_nq) scan the whole index with the
+        row mask (the masked HBM-regime kernels). Every other batch searches a compacted subset: the
+        selected rows in their order, re-packed as one add() of those rows (own max_norm and fp16
+        scale), on the unchanged route, and its labels go back through one nrb_map_ids."""
+        assert k > 0
+        if k > _lib.MAX_K:
+            raise RuntimeError(f"k={k} > {_lib.MAX_K} is not supported by the selection stage")
+        k, n = int(k), self.ntotal
+        nq = x.shape[0] if isinstance(x, torch.Tensor) else np.asarray(x).shape[0]
+        if n == 0 or nq == 0:
+            _unwrap_not(sel)
+            return self._search(x, k, D, I, id_map)
+        dev = self._xb.device
+        if self.small_nq and self.path == PATH_AUTO and nq < self.small_nq:
+            if id_map is None and _positions_kept(sel, n) == 0:
+                subset, labels = None, None
+            else:
+                member, keep = _select(sel, id_map, n, dev)
+                if not isinstance(x, torch.Tensor) and id_map is None:
+                    a = np.ascontiguousarray(x, dtype=np.float32)
+                    assert a.ndim == 2 and a.shape[1] == self.d
+                    return self._search_small_host(a, k, D, I, member, keep)
+                t, from_np = _to_device_f32(x)
+                assert t.shape[1] == self.d
+                Dd, Id = self._search_small_dev(t, k, member=member, keep=keep)
+                _map_ids(id_map, Id)
+                if from_np or D is not None or I is not None:
+                    return _to_host_pair(Dd, Id, D, I)
+                return Dd, Id
+        else:
+            rows = _selected_rows(sel, id_map, n, dev)
+            if rows.shape[0] == n:  # every row: the index itself
+                subset, labels = self, id_map
+            elif rows.shape[0] == 0:
+                subset, labels = None, None
+            else:
+                subset = IndexFlat(self.d, self.metric_type)
+                subset.path, subset.small_nq = self.path, self.small_nq
+                subset._xb = _gather_packed(self._xb, rows)
+                labels = rows.long() if id_map is None else _gather_i64(id_map, rows)
+        if subset is not None:
+            return subset._search(x, k, D, I, labels)
+        # no row selected: no search
+        Dd, Id = _padding(nq, k, self.metric_type, dev)
+        if not isinstance(x, torch.Tensor) or D is not None or I is not None:
+            return _to_host_pair(Dd, Id, D, I)
+        return Dd, Id
 
     def _search(self, x, k: int, D, I, id_map: torch.Tensor | None):
         """search(); id_map (IndexIDMap): labels are translated on the device before any copy back."""
@@ -619,7 +786,11 @@ class IndexIDMap:
         self.index.add(t)
         self.id_map = ids_d if self.id_map is None or self.id_map.numel() == 0 else torch.cat([self.id_map, ids_d])
 
-    def search(self, x, k: int, D=None, I=None):
+    def search(self, x, k: int, D=None, I=None, *, params=None):
+        """params: SearchParameters whose sel selects external ids (faiss's IDSelectorTranslated)."""
+        sel, _ = _search_sel(params, False)
+        if sel is not None:
+            return self.index._search_filtered(x, k, D, I, self.id_map if self.ntotal else None, sel)
         return self.index._search(x, k, D, I, self.id_map if self.ntotal else None)
 
     def remove_ids(self, sel) -> int:
@@ -898,21 +1069,41 @@ class IndexIVFFlat:
         self._lists = None
 
     def _build_lists(self):
-        if self._lists is not None:
-            return self._lists
+        if self._lists is None:
+            self._lists = self._pack_lists(self._assign, self.nlist)
+        return self._lists
+
+    def _filtered_lists(self, sel):
+        """The lists of the rows sel selects (by stored id), not cached: nrb_sel_keys sends every
+        other row to an extra bucket nlist that is never packed. The counting sort is stable, so
+        each list holds its selected rows in the order of the unfiltered list, and the planes come
+        out as those of an index built from the selected rows alone."""
         n, dev = self.ntotal, self._x.device
-        offsets = torch.empty(self.nlist + 1, dtype=torch.int32, device=dev)
+        member, keep = _select(sel, self._ids, n, dev)
+        key = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+        check(lib.nrb_sel_keys(member.data_ptr(), keep, self._assign.data_ptr(), n, self.nlist, key.data_ptr(),
+                               _stream()), "sel_keys")
+        return self._pack_lists(key, self.nlist + 1)
+
+    def _pack_lists(self, key: torch.Tensor, nbuckets: int):
+        """List-contiguous planes of the rows whose key (i64[ntotal], in [0, nbuckets)) is below
+        nlist: a stable counting sort by key, a gather of those rows, hi / lo / norms and the
+        scaled fp16 plane. nbuckets > nlist: the rows of the extra buckets are left out."""
+        n, dev = self.ntotal, self._x.device
+        offsets = torch.empty(nbuckets + 1, dtype=torch.int32, device=dev)
         order = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
-        wsb = lib.nrb_ivf_build_lists_workspace(n, self.nlist)
+        wsb = lib.nrb_ivf_build_lists_workspace(n, nbuckets)
         ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-        check(lib.nrb_ivf_build_lists(self._assign.data_ptr(), n, self.nlist, offsets.data_ptr(),
+        check(lib.nrb_ivf_build_lists(key.data_ptr(), n, nbuckets, offsets.data_ptr(),
                                       order.data_ptr(), ws.data_ptr(), wsb, _stream()), "ivf_build_lists")
+        off_h = _to_host(offsets[: self.nlist + 1]).astype(np.int64)
+        n = int(off_h[-1])  # rows in lists 0 .. nlist-1
         kp = self._x.kp
         raw = torch.empty((max(n, 1), kp), dtype=torch.float32, device=dev)
         check(lib.nrb_gather_rows(self._x.raw.data_ptr(), kp, order.data_ptr(), n, raw.data_ptr(), _stream()),
               "gather_rows")
         packed = PackedMatrix(self.d, dev)
-        packed._reserve(n)
+        packed._reserve(max(n, 1))  # a filter may keep no row
         packed.raw = raw  # already list-ordered and padded; derive hi / lo / norms from it
         check(lib.nrb_pack_rows(raw.data_ptr(), n, self.d, kp, kp, 0, packed.hi.data_ptr(), packed.lo.data_ptr(),
                                 packed.norms.data_ptr(), _stream()), "pack_rows")
@@ -927,22 +1118,24 @@ class IndexIVFFlat:
                 check(lib.nrb_pack_rows_h16(raw.data_ptr(), n, self.d, kp, kp, packed.h16_scale,
                                             packed.h16.data_ptr(), 0, _stream()), "pack_rows_h16")
         ids = _gather_i64(self._ids, order[:n])
-        off_h = _to_host(offsets).astype(np.int64)
         sizes = np.diff(off_h)
-        self._lists = dict(packed=packed, ids=ids, offsets=offsets, offsets_host=off_h,
-                           max_len=int(sizes.max()) if sizes.size else 0)
-        return self._lists
+        return dict(packed=packed, ids=ids, offsets=offsets[: self.nlist + 1], offsets_host=off_h,
+                    max_len=int(sizes.max()) if sizes.size else 0)
 
     def list_sizes(self) -> np.ndarray:
         return np.diff(self._build_lists()["offsets_host"])
 
-    def search(self, x, k: int):
+    def search(self, x, k: int, *, params=None):
+        """params: SearchParametersIVF. Its sel selects stored ids: the coarse search still ranks
+        every centroid, and the scan of the nprobe lists skips the rows sel does not select. Its
+        nprobe, when set, replaces index.nprobe for this call."""
+        sel, nprobe_p = _search_sel(params, True)
         if not self.is_trained:
             raise RuntimeError("Error: 'is_trained' failed")
         t, from_np = _to_device_f32(x)
         assert t.shape[1] == self.d
         assert k > 0
-        nprobe = min(int(self.nprobe), self.nlist)
+        nprobe = min(int(self.nprobe if nprobe_p is None else nprobe_p), self.nlist)
         if k > _lib.MAX_K or nprobe > _lib.MAX_K:
             raise RuntimeError(f"k / nprobe > {_lib.MAX_K} is not supported by the selection stage")
         nq, dev = t.shape[0], t.device
@@ -952,7 +1145,14 @@ class IndexIVFFlat:
             D.fill_(3.4028234663852886e38 if self.metric_type == METRIC_L2 else -3.4028234663852886e38)
             I.fill_(-1)
         elif nq:
-            L = self._build_lists()
+            small = self.path == PATH_AUTO and nq <= IVF_SMALL_NQ and nq * nprobe <= 65535 and self.quantizer.ntotal
+            # a selector: the small route masks the cached lists, the batch route scans lists of the
+            # selected rows only
+            L = self._build_lists() if sel is None or small else self._filtered_lists(sel)
+            if L["packed"].n == 0:  # the selector keeps no row: no search
+                D.fill_(3.4028234663852886e38 if self.metric_type == METRIC_L2 else -3.4028234663852886e38)
+                I.fill_(-1)
+                nq = 0
             # PATH_AUTO: fp16 filter + exact refine over the lists when eligible (raw, norms, h16 for
             # the filter; hi, lo for the queries it flags), else the 3xTF32 scan
             filt = self.path in (PATH_AUTO, PATH_TC16) and L["packed"].h16 is not None and k <= 112 and \
@@ -962,16 +1162,20 @@ class IndexIVFFlat:
                                          (("raw", "norms", "h16") if filt else ()) +
                                          (("norms",) if self.metric_type == METRIC_L2 else ())))
             ls = L["packed"].struct()
-            if self.path == PATH_AUTO and nq <= IVF_SMALL_NQ and nq * nprobe <= 65535 and self.quantizer.ntotal:
+            if small and nq:
                 # HBM-regime route for small batches: exact fp32 coarse search + row-per-warp list scan
                 _, coarse = self.quantizer._search_small_dev(t, nprobe) if nq < SMALL_NQ else \
                     self.quantizer.search(t, nprobe)
                 wsb = lib.nrb_ivf_scan_small_workspace(nq, nprobe, L["max_len"], self.ntotal, int(k))
                 ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-                check(lib.nrb_ivf_scan_small(t.data_ptr(), t.stride(0), nq, self.d, C.byref(ls), L["offsets"].data_ptr(),
-                                             self.nlist, L["max_len"], L["ids"].data_ptr(), coarse.data_ptr(), nprobe,
-                                             self.metric_type, int(k), D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb,
-                                             _stream()), "ivf_scan_small")
+                args = (t.data_ptr(), t.stride(0), nq, self.d, C.byref(ls), L["offsets"].data_ptr(), self.nlist,
+                        L["max_len"], L["ids"].data_ptr(), coarse.data_ptr(), nprobe, self.metric_type, int(k),
+                        D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb, _stream())
+                if sel is None:
+                    check(lib.nrb_ivf_scan_small(*args), "ivf_scan_small")
+                else:
+                    member, keep = _select(sel, L["ids"], self.ntotal, dev)  # list order, like the scan
+                    check(lib.nrb_ivf_scan_small_sel(*args, member.data_ptr(), keep), "ivf_scan_small_sel")
                 nq = 0  # done
             for q0 in range(0, nq, IVF_QUERY_BATCH):
                 q1 = min(nq, q0 + IVF_QUERY_BATCH)
