@@ -315,6 +315,14 @@ int nrb_pack_topk(const float* D, const int64_t* I, int64_t id_base, int64_t n, 
  * packed with) -> global top-k D f32[nq, k], I i64[nq, k]. Exact ties resolve by part order. */
 int nrb_merge_topk_packed(const uint64_t* P, const int64_t* bases, int32_t nparts, int64_t nq, int32_t k,
                           int32_t metric, float* D, int64_t* I, void* stream);
+/* The wire format of the id-carrying sharded indexes, whose ids are arbitrary int64 values rather
+ * than offsets from a shard base: 16 bytes per candidate, still one collective per chunk.
+ * P u64[n, 2]: P[t][0] = fp32 bits of D[t] << 32 | (I[t] < 0 ? 0xffffffff : 0), P[t][1] = I[t]. */
+int nrb_pack_topk_ids(const float* D, const int64_t* I, int64_t n, uint64_t* P, void* stream);
+/* P u64[nparts, nq, k, 2] (each part best-first) -> D f32[nq, k], I i64[nq, k]. Exact ties resolve by
+ * part order, then list position, as nrb_merge_topk_packed does. */
+int nrb_merge_topk_packed_ids(const uint64_t* P, int32_t nparts, int64_t nq, int32_t k, int32_t metric,
+                              float* D, int64_t* I, void* stream);
 
 #ifdef __cplusplus
 }

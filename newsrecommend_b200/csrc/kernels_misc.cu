@@ -602,6 +602,22 @@ struct PackedShardSource {
     }
 };
 
+// The same with caller-given 64-bit ids (id-carrying sharded indexes), 16 bytes per candidate:
+// P[s, q, pos] = {(fp32 bits of D) << 32 | (0xffffffff = no result, else 0), id}. Word 0 is all
+// the merge reads; the output step reads word 1.
+struct PackedIdShardSource {
+    const uint64_t* P;
+    int64_t nq;
+    int S, k, metric;
+    __device__ __forceinline__ int row(int64_t, int s) const { return s; }
+    __device__ __forceinline__ uint64_t load(int64_t q, int s, int, int pos) const {
+        const uint64_t e = P[(((int64_t)s * nq + q) * k + pos) * 2];
+        if ((uint32_t)e == 0xffffffffu) return empty_cand();
+        const float d = __uint_as_float((uint32_t)(e >> 32));
+        return pack_cand(metric == NRB_METRIC_L2 ? -d : d, s * k + pos);  // ties: part order, then position
+    }
+};
+
 template <int MAXL, typename Source>
 __device__ __forceinline__ void warp_kway_merge(const Source& S, int64_t q, int k, int lane,
                                                 uint64_t (&res)[4]) {
@@ -726,12 +742,46 @@ __global__ void shard_merge_packed_kernel(PackedShardSource S, const int64_t* __
     }
 }
 
+template <int MAXL>
+__global__ void shard_merge_packed_ids_kernel(PackedIdShardSource S, float* __restrict__ D, int64_t* __restrict__ I) {
+    const int lane = threadIdx.x & 31;
+    const int64_t q = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (q >= S.nq) return;
+    uint64_t res[4];
+    warp_kway_merge<MAXL>(S, q, S.k, lane, res);
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+        const int r = i * 32 + lane;
+        if (r < S.k) {
+            const int e = cand_idx(res[i]);
+            if (e < 0) {
+                I[q * S.k + r] = -1;
+                D[q * S.k + r] = (S.metric == NRB_METRIC_L2) ? FLT_MAX : -FLT_MAX;
+            } else {
+                const int s = e / S.k, pos = e - s * S.k;
+                const uint64_t* w = S.P + (((int64_t)s * S.nq + q) * S.k + pos) * 2;
+                I[q * S.k + r] = (int64_t)w[1];
+                D[q * S.k + r] = __uint_as_float((uint32_t)(w[0] >> 32));
+            }
+        }
+    }
+}
+
 __global__ void pack_topk_kernel(const float* __restrict__ D, const int64_t* __restrict__ I, int64_t id_base,
                                  int64_t n, uint64_t* __restrict__ P) {
     for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) {
         const int64_t id = I[t];
         const uint32_t lo = id < 0 ? 0xffffffffu : (uint32_t)(id - id_base);
         P[t] = ((uint64_t)__float_as_uint(D[t]) << 32) | lo;
+    }
+}
+
+__global__ void pack_topk_ids_kernel(const float* __restrict__ D, const int64_t* __restrict__ I, int64_t n,
+                                     uint64_t* __restrict__ P) {
+    for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n; t += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t id = I[t];
+        P[2 * t] = ((uint64_t)__float_as_uint(D[t]) << 32) | (id < 0 ? 0xffffffffu : 0u);
+        P[2 * t + 1] = (uint64_t)id;
     }
 }
 
@@ -1421,6 +1471,42 @@ extern "C" int nrb_merge_topk_packed(const uint64_t* P, const int64_t* bases, in
         shard_merge_packed_kernel<4><<<blocks, wpb * 32, 0, st>>>(ss, bases, D, I);
     else
         shard_merge_packed_kernel<8><<<blocks, wpb * 32, 0, st>>>(ss, bases, D, I);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}
+
+extern "C" int nrb_pack_topk_ids(const float* D, const int64_t* I, int64_t n, uint64_t* P, void* stream) {
+    NRB_REQUIRE(n >= 0 && (n == 0 || (D && I && P)), "pack_topk_ids: bad arguments");
+    if (n == 0) return NRB_OK;
+    int rc = require_device();
+    if (rc) return rc;
+    int64_t blocks = (n + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    pack_topk_ids_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(D, I, n, P);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}
+
+extern "C" int nrb_merge_topk_packed_ids(const uint64_t* P, int32_t nparts, int64_t nq, int32_t k, int32_t metric,
+                                         float* D, int64_t* I, void* stream) {
+    NRB_REQUIRE(nparts > 0 && nparts <= 256 && nq >= 0 && k > 0 && k <= 128, "merge_topk_packed_ids: bad sizes");
+    NRB_REQUIRE((int64_t)nparts * k < (1LL << 31), "merge_topk_packed_ids: nparts*k too large");
+    if (nq == 0) return NRB_OK;
+    NRB_REQUIRE(P && D && I, "merge_topk_packed_ids: null argument");
+    int rc = require_device();
+    if (rc) return rc;
+    PackedIdShardSource ss{P, nq, nparts, k, metric};
+    const int wpb = 8;
+    const unsigned blocks = (unsigned)((nq + wpb - 1) / wpb);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (nparts <= 32)
+        shard_merge_packed_ids_kernel<1><<<blocks, wpb * 32, 0, st>>>(ss, D, I);
+    else if (nparts <= 64)
+        shard_merge_packed_ids_kernel<2><<<blocks, wpb * 32, 0, st>>>(ss, D, I);
+    else if (nparts <= 128)
+        shard_merge_packed_ids_kernel<4><<<blocks, wpb * 32, 0, st>>>(ss, D, I);
+    else
+        shard_merge_packed_ids_kernel<8><<<blocks, wpb * 32, 0, st>>>(ss, D, I);
     NRB_LAUNCH_CHECK();
     return NRB_OK;
 }

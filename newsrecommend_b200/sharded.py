@@ -16,8 +16,20 @@ runs the exact top-k kernel on its shard. The exchange step comes in two forms:
 The merged result equals the single-index answer up to the order of exact ties. The reference has
 no distributed code at all (SURVEY 2.2); this is the north star's extension of IndexFlat.search.
 
-Host logic only; `make_index` (per-rank index) and `codec` (pack / merge) are injectable so that
-the same code runs under gloo on CPU with the oracle index and numpy stand-ins (tests/).
+External ids, removal and search-time selectors (faiss's IndexIDMap / add_with_ids / remove_ids /
+SearchParameters): an index is either id-carrying (built with add_with_ids*) or plain (built with
+add_global / add_local), fixed by its first add. The rank-local work is the single-GPU index's own
+(IndexIDMap over IndexFlat, IndexIVFFlat.add_with_ids, their remove_ids and search(params=...));
+the sharded layer only moves a plain index's selectors into the rank's local numbering and
+all-reduces counts. Id-carrying results travel as 16-byte (score bits, int64 id) words
+(nrb_pack_topk_ids / nrb_merge_topk_packed_ids), plain ones keep the 8-byte format. Exact score
+ties merge in rank order: after one add_with_ids call that is row order, as in the single index;
+after several calls rank 0's later rows come before rank 1's earlier ones, where the single index
+keeps insertion order.
+
+Host logic only; `make_index` / `make_idmap` (per-rank index) and `codec` (pack / merge) are
+injectable so that the same code runs under gloo on CPU with the oracle index and numpy stand-ins
+(tests/).
 """
 from __future__ import annotations
 
@@ -75,6 +87,42 @@ class GpuCodec:
                                         torch.cuda.current_stream().cuda_stream), "merge_topk_packed")
         return D, I
 
+    @staticmethod
+    def pack_ids(D: torch.Tensor, I: torch.Tensor) -> torch.Tensor:
+        """16-byte words i64[..., 2] of an id-carrying index's results (nrb_pack_topk_ids)."""
+        from ._lib import check, lib
+        P = torch.empty(tuple(D.shape) + (2,), dtype=torch.int64, device=D.device)
+        check(lib.nrb_pack_topk_ids(D.data_ptr(), I.data_ptr(), D.numel(), P.data_ptr(),
+                                    torch.cuda.current_stream().cuda_stream), "pack_topk_ids")
+        return P
+
+    @staticmethod
+    def merge_ids(P: torch.Tensor, metric: int):
+        from ._lib import check, lib
+        G, nq, k, _ = P.shape
+        D = torch.empty((nq, k), dtype=torch.float32, device=P.device)
+        I = torch.empty((nq, k), dtype=torch.int64, device=P.device)
+        check(lib.nrb_merge_topk_packed_ids(P.data_ptr(), G, nq, k, metric, D.data_ptr(), I.data_ptr(),
+                                            torch.cuda.current_stream().cuda_stream), "merge_topk_packed_ids")
+        return D, I
+
+
+_I64_MIN, _I64_MAX = -(1 << 63), (1 << 63) - 1
+
+
+def shift_selector(sel, base: int):
+    """A selector over global row positions moved into a shard's local numbering (position - base):
+    IDSelectorRange(imin - base, imax - base), IDSelectorBatch(ids - base) of the ids >= base (the
+    rest cannot name a local row), IDSelectorNot of the shifted inner selector."""
+    from .faiss import IDSelectorBatch, IDSelectorNot, IDSelectorRange
+    if isinstance(sel, IDSelectorNot):
+        return IDSelectorNot(shift_selector(sel.sel, base))
+    if isinstance(sel, IDSelectorRange):
+        return IDSelectorRange(min(max(sel.imin - base, _I64_MIN), _I64_MAX), min(max(sel.imax - base, _I64_MIN), _I64_MAX))
+    if isinstance(sel, IDSelectorBatch):
+        return IDSelectorBatch(sel.ids[sel.ids >= base] - base)
+    raise TypeError(f"expected an IDSelectorRange, IDSelectorBatch or IDSelectorNot, not {type(sel)}")
+
 
 class _ShardedSearch:
     """The exchange machinery shared by the sharded indexes: chunking, packing, all-to-all by query
@@ -93,6 +141,85 @@ class _ShardedSearch:
         self.bases = None  # i64[G]: first global id of every shard
         self._bases_host = [0]
         self.chunk_queries = chunk_queries
+        self.with_ids = None  # True: id-carrying (add_with_ids*), False: plain (add_global / add_local), None: empty
+
+    def _start_add(self, with_ids: bool, what: str) -> bool:
+        """Fixes the index's kind at its first add (True is returned then) and refuses the other kind
+        afterwards, as faiss's IndexIDMap refuses add()."""
+        if self.with_ids is None:
+            self.with_ids = with_ids
+            return True
+        if self.with_ids != with_ids:
+            raise RuntimeError(f"{what} on an index built with " +
+                               ("add_with_ids: use add_with_ids / add_with_ids_local" if self.with_ids else
+                                "add_global / add_local: it carries no ids"))
+        return False
+
+    def _gather_counts(self, *vals: int) -> np.ndarray:
+        """i64[G, len(vals)]: the given per-rank counts of every rank (one all-gather)."""
+        t = torch.tensor(vals, dtype=torch.int64, device=self._dev())
+        if self.world == 1:
+            return t.cpu().numpy().reshape(1, -1)
+        out = torch.empty(self.world * len(vals), dtype=torch.int64, device=self._dev())
+        dist.all_gather_into_tensor(out, t, group=self.group)
+        return out.cpu().numpy().reshape(self.world, -1)
+
+    def add_with_ids(self, x, ids):
+        """Every rank passes the SAME full batch and int64 ids; each keeps its shard_range slice.
+        Appends to what the ranks hold already; the index carries ids from its first add on."""
+        nb = x.shape[0]
+        if len(ids) != nb:
+            raise TypeError(f"add_with_ids: {len(ids)} ids for {nb} rows")
+        lo, hi = shard_range(nb, self.world, self.rank)
+        self.add_with_ids_local(x[lo:hi], ids[lo:hi])
+
+    def add_with_ids_local(self, x_local, ids_local):
+        """Each rank passes only ITS rows and their int64 ids. ntotal is all-reduced afterwards."""
+        self._start_add(True, "add_with_ids")
+        self.local.add_with_ids(x_local, ids_local)
+        self.ntotal = int(self._gather_counts(self.local.ntotal).sum())
+
+    def remove_ids(self, sel) -> int:
+        """Removes the rows sel selects (IDSelectorRange / IDSelectorBatch / IDSelectorNot or an int64
+        id array) from every shard; returns the number removed across all ranks, on every rank.
+        sel tests the external ids of an id-carrying index, the global row positions of a plain
+        ShardedIndexFlat (later rows move up, as in IndexFlat.remove_ids) and the stored ids of a plain
+        ShardedIndexIVFFlat (the global positions given at add time; survivors keep them)."""
+        from .faiss import _selector
+        sel = _selector(sel)
+        removed = self.local.remove_ids(sel if self.with_ids else shift_selector(sel, self.id_base))
+        counts = self._gather_counts(self.local.ntotal, removed)
+        self.ntotal = int(counts[:, 0].sum())
+        self._after_remove(counts[:, 0])
+        return int(counts[:, 1].sum())
+
+    def _after_remove(self, local_counts: np.ndarray):
+        pass
+
+    def _local_params(self, params):
+        """The params the rank-local index searches with: a plain index's selector moves into the
+        shard's local numbering. Checked on every rank before any collective."""
+        raise NotImplementedError
+
+    def _pack(self, D: torch.Tensor, I: torch.Tensor) -> torch.Tensor:
+        return self.codec.pack_ids(D, I) if self.with_ids else self.codec.pack(D, I, self.id_base)
+
+    def _merge(self, recv: torch.Tensor):
+        if self.with_ids:
+            return self.codec.merge_ids(recv, self.metric_type)
+        return self.codec.merge(recv, self._bases(), self.metric_type)
+
+    def _local_search(self, xq, k: int, params):
+        """The rank-local index's search (CUDA tensors, or ndarrays on the CPU test path) as tensors,
+        labels made global: external ids as they are, local positions + id_base."""
+        if self._cuda_index:
+            D, I = self.local.search(xq, k, params=params)
+        else:
+            D, I = self.local.search(np.ascontiguousarray(xq), k, **({} if params is None else {"params": params}))
+            D, I = torch.as_tensor(D), torch.as_tensor(I)
+        if self.with_ids:
+            return D, I
+        return D, torch.where(I >= 0, I + self.id_base, I)
 
     def _set_bases_global(self, nb: int):
         self._bases_host = [shard_range(nb, self.world, r)[0] for r in range(self.world)]
@@ -127,33 +254,37 @@ class _ShardedSearch:
         return 1 << 17
 
     # ------------------------------------------------------------------ search pieces
-    def search_local(self, xq, k: int):
-        """Per-shard top-k of a raw query chunk with GLOBAL ids: (D f32[n,k], I i64[n,k]) tensors."""
+    def search_local(self, xq, k: int, params=None):
+        """Per-shard top-k of a raw query chunk with GLOBAL ids: (D f32[n,k], I i64[n,k]) tensors.
+        params: what _local_params made of the caller's search parameters."""
         raise NotImplementedError
 
     def _exchange_start(self, P: torch.Tensor, per: int):
-        """Starts the exchange of one chunk's packed per-shard results P i64[cn, k]. Returns
-        (recv i64[G, rows, k], work handle or None): alltoall -> rows = this rank's slice of the
-        chunk, allgather -> rows = the whole chunk."""
-        cn, k = P.shape
+        """Starts the exchange of one chunk's packed per-shard results P i64[cn, k] (i64[cn, k, 2]
+        with ids). Returns (recv i64[G, rows, ...], work handle or None): alltoall -> rows = this
+        rank's slice of the chunk, allgather -> rows = the whole chunk."""
+        cn, tail = P.shape[0], tuple(P.shape[1:])
         G, r = self.world, self.rank
         if G == 1:
             return P.unsqueeze(0), None
         if self.exchange_mode == "allgather":
-            recv = torch.empty((G * cn, k), dtype=P.dtype, device=P.device)
+            recv = torch.empty((G * cn,) + tail, dtype=P.dtype, device=P.device)
             work = dist.all_gather_into_tensor(recv, P, group=self.group, async_op=True)
-            return recv.view(G, cn, k), work
+            return recv.view((G, cn) + tail), work
         in_rows = [max(0, min(cn, (j + 1) * per) - min(cn, j * per)) for j in range(G)]
         mine = in_rows[r]
-        recv = torch.empty((G * mine, k), dtype=P.dtype, device=P.device)
+        recv = torch.empty((G * mine,) + tail, dtype=P.dtype, device=P.device)
         work = dist.all_to_all_single(recv, P, [mine] * G, in_rows, group=self.group, async_op=True)
-        return recv.view(G, mine, k), work
+        return recv.view((G, mine) + tail), work
 
-    def search(self, xq, k: int, gather: bool = True):
+    def search(self, xq, k: int, gather: bool = True, *, params=None):
         """xq: the FULL query batch on every rank (CUDA tensor fp32 [nq, d]; ndarray on the CPU test
         path). gather=True: (D, I) of all queries on every rank (a final all-gather of the merged
         slices). gather=False: the merged results of this rank's own rows only, as
-        (D, I, spans) with spans = owned_rows(nq, ...)."""
+        (D, I, spans) with spans = owned_rows(nq, ...). params: as the single index of the same kind
+        takes them (SearchParameters / SearchParametersIVF); when fewer than k rows qualify across
+        all shards the tail is I = -1, D = -FLT_MAX (IP) / +FLT_MAX (L2)."""
+        lp = self._local_params(params)
         nq = xq.shape[0]
         G = self.world
         chunk = self._chunk()
@@ -164,11 +295,11 @@ class _ShardedSearch:
             recv, work = p
             if work is not None:
                 work.wait()
-            parts.append(self.codec.merge(recv, self._bases(), self.metric_type))
+            parts.append(self._merge(recv))
 
         for c0, c1, per in chunk_slices(nq, G, chunk):
-            D, I = self.search_local(xq[c0:c1], k)
-            P = self.codec.pack(D, I, self.id_base)
+            D, I = self.search_local(xq[c0:c1], k, lp)
+            P = self._pack(D, I)
             nxt = self._exchange_start(P, per)
             if pending is not None:
                 finish(pending[:2])  # merged after the NEXT chunk's search was queued: its exchange overlaps that search
@@ -212,13 +343,15 @@ class _ShardedSearch:
         return D, I
 
     # ------------------------------------------------------------------ end to end from host memory
-    def search_host(self, xq_host: np.ndarray, k: int, D_out: np.ndarray, I_out: np.ndarray):
+    def search_host(self, xq_host: np.ndarray, k: int, D_out: np.ndarray, I_out: np.ndarray, *, params=None):
         """The call a user of the sharded index makes with HOST arrays: every rank passes the same
         page-locked fp32 [nq, d] batch and the same-shaped output arrays; each rank copies only ITS
         rows host-to-device (1/G of the batch), the ranks all-gather the query rows over NVLink,
         search, exchange, merge, and each rank copies the results of its own rows back into
-        D_out / I_out (rows owned by other ranks are left untouched). Returns the owned spans."""
+        D_out / I_out (rows owned by other ranks are left untouched). Returns the owned spans.
+        params: as search() takes them."""
         assert self._cuda_index, "search_host is the CUDA path"
+        lp = self._local_params(params)
         nq, d = xq_host.shape
         G, r = self.world, self.rank
         dev = self._dev()
@@ -234,7 +367,7 @@ class _ShardedSearch:
                 work.wait()
             if self.exchange_mode == "allgather" and G > 1:
                 recv = recv[:, lo - c0:hi - c0].contiguous()  # merge (and return) only the owned rows
-            Dm, Im = self.codec.merge(recv, self._bases(), self.metric_type)
+            Dm, Im = self._merge(recv)
             if hi > lo:
                 Dt[lo:hi].copy_(Dm, non_blocking=True)
                 It[lo:hi].copy_(Im, non_blocking=True)
@@ -253,8 +386,8 @@ class _ShardedSearch:
                 dist.all_gather_into_tensor(full, mine, group=self.group)
             else:
                 full = mine
-            D, I = self.search_local(full[: c1 - c0], k)
-            P = self.codec.pack(D, I, self.id_base)
+            D, I = self.search_local(full[: c1 - c0], k, lp)
+            P = self._pack(D, I)
             recv, work = self._exchange_start(P, per)
             if pending is not None:
                 keep.append(finish(pending[:5]))
@@ -269,18 +402,23 @@ class ShardedIndexFlat(_ShardedSearch):
     """Row-sharded exact index (IndexFlatIP / IndexFlatL2 semantics over the whole catalog)."""
 
     def __init__(self, d: int, metric: int = 1, group=None, make_index=None, codec=None, exchange: str = "alltoall",
-                 chunk_queries: int | None = None):
+                 chunk_queries: int | None = None, make_idmap=None):
         self._init_sharding(metric, group, codec, exchange, chunk_queries, cuda_index=make_index is None)
         self.d = d
         if make_index is None:
             from .faiss import IndexFlat
             make_index = IndexFlat
+        if make_idmap is None:
+            from .faiss import IndexIDMap
+            make_idmap = IndexIDMap
         self.local = make_index(d, metric)
+        self._make_idmap = make_idmap  # wraps the empty local index at the first add_with_ids*
 
     # ------------------------------------------------------------------ build
     def add_global(self, x):
         """Every rank passes the SAME full matrix; each keeps only its own row range."""
         nb = x.shape[0]
+        self._start_add(False, "add_global")
         assert self.ntotal == 0, "add_global is a one-shot build"
         lo, hi = shard_range(nb, self.world, self.rank)
         self.id_base = lo
@@ -291,20 +429,37 @@ class ShardedIndexFlat(_ShardedSearch):
     def add_local(self, x_local, id_base: int, ntotal: int):
         """Each rank passes only ITS rows (global ids id_base ... id_base + len - 1): for catalogs
         that no single process ever holds whole (10M x 256 sharded: BASELINE configs[4])."""
+        self._start_add(False, "add_local")
         assert self.ntotal == 0, "add_local is a one-shot build"
         self.id_base = int(id_base)
         self.local.add(x_local)
         self.ntotal = int(ntotal)
         self._set_bases_gathered()
 
-    def search_local(self, xq, k: int):
-        if self._cuda_index:
+    def add_with_ids_local(self, x_local, ids_local):
+        if self.with_ids is None:
+            self.local = self._make_idmap(self.local)
+        super().add_with_ids_local(x_local, ids_local)
+
+    def _after_remove(self, local_counts: np.ndarray):
+        if not self.with_ids:  # positions renumber: every shard's first global position moves up
+            self._bases_host = [0] + np.cumsum(local_counts)[:-1].tolist()
+            self.id_base = int(self._bases_host[self.rank])
+            self.bases = None
+
+    def _local_params(self, params):
+        from .faiss import SearchParameters, _search_sel
+        sel, _ = _search_sel(params, False)
+        if sel is None:
+            return None
+        return SearchParameters(sel=sel if self.with_ids else shift_selector(sel, self.id_base))
+
+    def search_local(self, xq, k: int, params=None):
+        if self._cuda_index and params is None and not self.with_ids:
             from .faiss import PackedMatrix
             q = PackedMatrix.from_tensor(xq, planes=self.local._query_planes(k))  # K0 on the fresh chunk
             return self.local.search_packed(q, k, self.id_base)
-        D, I = self.local.search(np.ascontiguousarray(xq), k)
-        I = torch.as_tensor(I)
-        return torch.as_tensor(D), torch.where(I >= 0, I + self.id_base, I)
+        return self._local_search(xq, k, params)
 
 
 # ------------------------------------------------------------------------------------ sharded IVF
@@ -517,6 +672,7 @@ class ShardedIndexIVFFlat(_ShardedSearch):
 
     def add_global(self, x):
         nb = x.shape[0]
+        self._start_add(False, "add_global")
         assert self.ntotal == 0, "add_global is a one-shot build"
         lo, hi = shard_range(nb, self.world, self.rank)
         self.id_base = lo
@@ -525,17 +681,22 @@ class ShardedIndexIVFFlat(_ShardedSearch):
         self._set_bases_global(nb)
 
     def add_local(self, x_local, id_base: int, ntotal: int):
+        self._start_add(False, "add_local")
         assert self.ntotal == 0, "add_local is a one-shot build"
         self.id_base = int(id_base)
         self.local.add(x_local)
         self.ntotal = int(ntotal)
         self._set_bases_gathered()
 
-    def search_local(self, xq, k: int):
+    def _local_params(self, params):
+        from .faiss import SearchParametersIVF, _search_sel
+        sel, nprobe = _search_sel(params, True)
+        if params is None:
+            return None
+        if sel is not None and not self.with_ids:
+            sel = shift_selector(sel, self.id_base)  # stored ids are local positions
+        return SearchParametersIVF(sel=sel, nprobe=nprobe)
+
+    def search_local(self, xq, k: int, params=None):
         self.local.nprobe = self.nprobe
-        if self._cuda_index:
-            D, I = self.local.search(xq, k)  # ids = local insertion rows
-            return D, torch.where(I >= 0, I + self.id_base, I)
-        D, I = self.local.search(np.ascontiguousarray(xq), k)
-        I = torch.as_tensor(I)
-        return torch.as_tensor(D), torch.where(I >= 0, I + self.id_base, I)
+        return self._local_search(xq, k, params)  # plain: stored ids = local insertion rows
