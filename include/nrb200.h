@@ -324,6 +324,15 @@ int nrb_pack_topk_ids(const float* D, const int64_t* I, int64_t n, uint64_t* P, 
 int nrb_merge_topk_packed_ids(const uint64_t* P, int32_t nparts, int64_t nq, int32_t k, int32_t metric,
                               float* D, int64_t* I, void* stream);
 
+/* Per-query exclusion after an over-fetched search. Row r of Din/Iin (f32/i64 [nrows, kin], best-first,
+ * labels already translated) belongs to query q = qidx ? qidx[r] : r. Entries whose label is >= 0 and
+ * occurs in excl_ids[excl_off[q] .. excl_off[q+1]) are dropped; the first k survivors, in order, go to
+ * D[q, :], I[q, :] (f32/i64 [*, k]); the rest of the row is padding (I = -1, D = -FLT_MAX for IP,
+ * +FLT_MAX for L2). 1 <= k <= kin <= 128. A warp per row; the cost is O(kin * list length / 32). */
+int nrb_exclude_topk(const float* Din, const int64_t* Iin, int64_t nrows, int32_t kin, const int64_t* qidx,
+                     const int64_t* excl_off, const int64_t* excl_ids, int32_t metric, int32_t k,
+                     float* D, int64_t* I, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

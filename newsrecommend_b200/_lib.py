@@ -36,7 +36,7 @@ SYMBOLS = [
     "nrb_ivf_scan_small_workspace", "nrb_ivf_scan_small", "nrb_split_table_f64",
     "nrb_id_select_workspace", "nrb_id_select", "nrb_map_ids",
     "nrb_search_small_sel", "nrb_search_small_host_sel", "nrb_ivf_scan_small_sel", "nrb_sel_keys",
-    "nrb_pack_topk_ids", "nrb_merge_topk_packed_ids",
+    "nrb_pack_topk_ids", "nrb_merge_topk_packed_ids", "nrb_exclude_topk",
 ]
 
 
@@ -115,6 +115,7 @@ lib.nrb_ivf_scan_small_sel.argtypes = lib.nrb_ivf_scan_small.argtypes + [_vp, _i
 lib.nrb_sel_keys.argtypes = [_vp, _i64, _vp, _i64, _i64, _vp, _vp]
 lib.nrb_pack_topk_ids.argtypes = [_vp, _vp, _i64, _vp, _vp]
 lib.nrb_merge_topk_packed_ids.argtypes = [_vp, _i32, _i64, _i32, _i32, _vp, _vp, _vp]
+lib.nrb_exclude_topk.argtypes = [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]
 
 
 def last_error() -> str:

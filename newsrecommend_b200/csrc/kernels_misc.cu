@@ -1735,3 +1735,77 @@ extern "C" int nrb_sel_keys(const int64_t* member, int64_t keep, const int64_t* 
     NRB_LAUNCH_CHECK();
     return NRB_OK;
 }
+
+// ------------------------------------------------------------------- per-query exclusion lists
+// After a search at kin = k + (longest list of the batch), drop from row r (query q = qidx[r], or r)
+// every candidate whose label is in q's list and keep the first k survivors in order. A warp per row:
+// slot s = lane + 32 * j (j < 4) lives in lane `lane`'s registers, the list is read 32 ids at a time
+// and broadcast lane by lane, and one ballot per j gives each survivor its output position.
+constexpr int EX_WPB = 8;
+
+__global__ void __launch_bounds__(EX_WPB * 32)
+exclude_topk_kernel(const float* __restrict__ Din, const int64_t* __restrict__ Iin, int64_t nrows, int kin,
+                    const int64_t* __restrict__ qidx, const int64_t* __restrict__ excl_off,
+                    const int64_t* __restrict__ excl_ids, float pad, int k, float* __restrict__ D,
+                    int64_t* __restrict__ I) {
+    const int lane = threadIdx.x & 31;
+    const int64_t r = (int64_t)blockIdx.x * EX_WPB + (threadIdx.x >> 5);
+    if (r >= nrows) return;
+    const int64_t q = qidx ? qidx[r] : r;
+    float dv[4];
+    int64_t iv[4];
+    bool keep[4];
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        const int s = lane + 32 * j;
+        keep[j] = s < kin;
+        iv[j] = keep[j] ? Iin[r * kin + s] : -1;
+        dv[j] = keep[j] ? Din[r * kin + s] : 0.0f;
+    }
+    const int64_t b = excl_off[q], e = excl_off[q + 1];
+    for (int64_t c = b; c < e; c += 32) {
+        const int64_t v = c + lane < e ? excl_ids[c + lane] : -1;
+        const int cnt = e - c < 32 ? (int)(e - c) : 32;
+        for (int t = 0; t < cnt; t++) {
+            const int64_t x = __shfl_sync(0xffffffffu, v, t);
+            if (x < 0) continue;  // warp-uniform: a negative list entry removes nothing
+#pragma unroll
+            for (int j = 0; j < 4; j++) keep[j] = keep[j] && iv[j] != x;
+        }
+    }
+    float* Dq = D + q * k;
+    int64_t* Iq = I + q * k;
+    const unsigned below = (1u << lane) - 1u;
+    int base = 0;
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        const unsigned m = __ballot_sync(0xffffffffu, keep[j]);
+        const int pos = base + __popc(m & below);
+        if (keep[j] && pos < k) {
+            Dq[pos] = dv[j];
+            Iq[pos] = iv[j];
+        }
+        base += __popc(m);
+    }
+    for (int p = base + lane; p < k; p += 32) {
+        Dq[p] = pad;
+        Iq[p] = -1;
+    }
+}
+
+extern "C" int nrb_exclude_topk(const float* Din, const int64_t* Iin, int64_t nrows, int32_t kin, const int64_t* qidx,
+                                const int64_t* excl_off, const int64_t* excl_ids, int32_t metric, int32_t k, float* D,
+                                int64_t* I, void* stream) {
+    NRB_REQUIRE(nrows >= 0 && kin >= 1 && kin <= 128 && k >= 1 && k <= kin,
+                "exclude_topk: bad sizes nrows=%lld kin=%d k=%d", (long long)nrows, kin, k);
+    NRB_REQUIRE(metric == NRB_METRIC_INNER_PRODUCT || metric == NRB_METRIC_L2, "exclude_topk: bad metric %d", metric);
+    NRB_REQUIRE(nrows == 0 || (Din && Iin && excl_off && excl_ids && D && I), "exclude_topk: null argument");
+    if (nrows == 0) return NRB_OK;
+    int rc = require_device();
+    if (rc) return rc;
+    const float pad = metric == NRB_METRIC_L2 ? FLT_MAX : -FLT_MAX;
+    exclude_topk_kernel<<<(unsigned)((nrows + EX_WPB - 1) / EX_WPB), EX_WPB * 32, 0, (cudaStream_t)stream>>>(
+        Din, Iin, nrows, kin, qidx, excl_off, excl_ids, pad, k, D, I);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}

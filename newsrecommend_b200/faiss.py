@@ -17,6 +17,11 @@ ones search a compacted copy of the selected rows, built like one add() of those
 labels back on the device, so such a search returns what the same search of an index built from
 only the selected rows returns.
 
+Per-query exclusion lists: `search(x, k, exclude=(offsets, ids))` on the same three index types keeps
+query q from returning any label in ids[offsets[q]:offsets[q+1]] (labels as for selectors; combines
+with params). Each query is searched at k plus its list length and the listed labels are dropped on
+the device by nrb_exclude_topk (_search_excluded).
+
 Host code only: every array lives in HBM as torch tensors and all arithmetic is done by
 libnrb200.so (hand-written sm_100a CUDA) through the C-ABI in include/nrb200.h. numpy in ->
 numpy out (synchronous, like faiss); CUDA torch tensors in -> CUDA torch tensors out
@@ -467,6 +472,105 @@ def _map_ids(id_map: torch.Tensor | None, I: torch.Tensor):
         check(lib.nrb_map_ids(id_map.data_ptr(), I.data_ptr(), I.numel(), _stream()), "map_ids")
 
 
+# ------------------------------------------------------------------------------------ exclusion lists
+_FILTER_MAX_K = 112  # the fp16 filter's k bound (_query_planes, IndexIVFFlat.search's eligibility check)
+
+
+def _exclude_arg(exclude, nq: int):
+    """search()'s exclude=(offsets, ids): a CSR pair of int64 numpy arrays or tensors, checked before any
+    device work. Returns (offsets as a host int64 array, offsets, ids)."""
+    if not isinstance(exclude, (tuple, list)) or len(exclude) != 2:
+        raise TypeError("exclude must be a pair (offsets, ids) of int64 arrays")
+    arrs = []
+    for a, what in zip(exclude, ("offsets", "ids")):
+        if isinstance(a, torch.Tensor):
+            ok = a.dtype == torch.int64
+        elif isinstance(a, np.ndarray):
+            ok = a.dtype == np.int64
+        else:
+            ok = False
+        if not ok:
+            raise TypeError(f"exclude: {what} must be an int64 numpy array or tensor, not {getattr(a, 'dtype', type(a))}")
+        if a.ndim != 1:
+            raise ValueError(f"exclude: {what} must be 1-D, got shape {tuple(a.shape)}")
+        arrs.append(a)
+    off, ids = arrs
+    off_h = off.detach().cpu().numpy() if isinstance(off, torch.Tensor) else off
+    if off_h.shape[0] != nq + 1:
+        raise ValueError(f"exclude: offsets has {off_h.shape[0]} entries for {nq} queries (needs nq + 1)")
+    if off_h[0] != 0 or off_h[-1] != ids.shape[0]:
+        raise ValueError(f"exclude: offsets must run from 0 to len(ids) = {ids.shape[0]}, "
+                         f"not {int(off_h[0])} .. {int(off_h[-1])}")
+    if (np.diff(off_h) < 0).any():
+        raise ValueError("exclude: offsets decrease")
+    return off_h, off, ids
+
+
+def _exclude_to_device(off_h, off, ids, dev):
+    """The checked CSR pair as i64 CUDA tensors (offsets, ids)."""
+    off_d = off.to(dev) if isinstance(off, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(off_h)).to(dev)
+    ids_d = ids.to(dev) if isinstance(ids, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(ids)).to(dev)
+    if ids_d.numel() == 0:
+        ids_d = torch.empty(1, dtype=torch.int64, device=dev)  # never read; keeps the pointer valid
+    return off_d.contiguous(), ids_d.contiguous()
+
+
+def _list_member(row_ids, n: int, ids_d: torch.Tensor, lo: int, hi: int, sel_mask, dev):
+    """Row mask of one query's exclusion list ids_d[lo:hi] over n rows whose labels are row_ids (i64
+    CUDA tensor, or None for row positions), ANDed with a selector's mask sel_mask = _select(...) or None:
+    (member, keep = 0) in the form the masked kernels take. The AND is nrb_sel_keys with the list's
+    member as key and 1 as the drop value: a row scans when the selector keeps it and the list misses it."""
+    nb = hi - lo
+    member = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+    wsb = lib.nrb_id_select_workspace(nb)
+    ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device=dev)
+    check(lib.nrb_id_select(_ptr(row_ids), n, ids_d.data_ptr() + 8 * lo if nb else None, nb, 0, 0, member.data_ptr(),
+                            ws.data_ptr(), wsb, _stream()), "id_select")
+    if sel_mask is not None:
+        both = torch.empty_like(member)
+        check(lib.nrb_sel_keys(sel_mask[0].data_ptr(), sel_mask[1], member.data_ptr(), n, 1, both.data_ptr(),
+                               _stream()), "sel_keys")
+        member = both
+    return member, 0
+
+
+def _search_excluded(t: torch.Tensor, k: int, metric: int, exclude, group_search, long_search):
+    """search(..., exclude=(offsets, ids)) over the CUDA query batch t -> (D, I) CUDA tensors; exclude is
+    what _exclude_arg returned.
+
+    Query q's list holds E_q = offsets[q+1] - offsets[q] labels (duplicates counted). At most E_q of its
+    top k + E_q rows are excluded, so the survivors hold the exact top k of the rows it may see. The
+    queries with k + E_q <= 112 (the fp16 filter's bound) form one group and those with 112 < k + E_q <=
+    128 another; each group is gathered and searched once by group_search(x, k') at k' = k + its longest
+    list, and nrb_exclude_topk drops the listed labels and scatters the group's first k survivors into
+    its rows of D, I. A query with k + E_q > 128 (MAX_K) cannot over-fetch: long_search(x_q, lo, hi)
+    scans it alone with its list as a row mask."""
+    nq, dev = t.shape[0], t.device
+    off_h = exclude[0]
+    off_d, ids_d = _exclude_to_device(*exclude, dev)
+    D = torch.empty((nq, k), dtype=torch.float32, device=dev)
+    I = torch.empty((nq, k), dtype=torch.int64, device=dev)
+    need = k + np.diff(off_h)
+    for group in (need <= _FILTER_MAX_K, (need > _FILTER_MAX_K) & (need <= _lib.MAX_K)):
+        rows = np.nonzero(group)[0]
+        if rows.size == 0:
+            continue
+        kq = int(need[rows].max())
+        if rows.size == nq:
+            qidx, xg = None, t
+        else:
+            qidx = torch.from_numpy(rows.astype(np.int64)).to(dev)
+            xg = t.index_select(0, qidx)
+        Dg, Ig = group_search(xg, kq)
+        check(lib.nrb_exclude_topk(Dg.data_ptr(), Ig.data_ptr(), rows.size, kq, _ptr(qidx), off_d.data_ptr(),
+                                   ids_d.data_ptr(), metric, k, D.data_ptr(), I.data_ptr(), _stream()), "exclude_topk")
+    for q in np.nonzero(need > _lib.MAX_K)[0]:
+        Dq, Iq = long_search(t[q:q + 1], int(off_h[q]), int(off_h[q + 1]), ids_d)
+        D[q].copy_(Dq[0])
+        I[q].copy_(Iq[0])
+    return D, I
+
+
 # ------------------------------------------------------------------------------------ flat
 class IndexFlat:
     """IndexFlatL2 / IndexFlatIP (Retrieval.py:25-26,32; SURVEY 8b). add() copies into HBM."""
@@ -582,14 +686,53 @@ class IndexFlat:
         self._xb = _gather_packed(self._xb, order)
         self._struct_cache = None
 
-    def search(self, x, k: int, D=None, I=None, *, params=None):
+    def search(self, x, k: int, D=None, I=None, *, params=None, exclude=None):
         """(D, I) = search(x, k). Like faiss, optional preallocated numpy outputs D f32[nq,k],
         I i64[nq,k] are filled and returned (page-locked buffers avoid a staging copy).
-        params: SearchParameters (or SearchParametersIVF) whose sel selects row positions."""
+        params: SearchParameters (or SearchParametersIVF) whose sel selects row positions.
+        exclude: (offsets i64[nq+1], ids i64) CSR lists, numpy or tensors; query q returns no row
+        position in ids[offsets[q]:offsets[q+1]] (a -1 or an absent id excludes nothing)."""
         sel, _ = _search_sel(params, False)
+        if exclude is not None:
+            return self._search_exclude(x, k, D, I, None, sel, exclude)
         if sel is not None:
             return self._search_filtered(x, k, D, I, None, sel)
         return self._search(x, k, D, I, None)
+
+    def _search_exclude(self, x, k: int, D, I, id_map: torch.Tensor | None, sel, exclude):
+        """search() with per-query exclusion lists (_search_excluded): the lists and sel test
+        id_map[row] (IndexIDMap) or the row position. Numpy batches take one copy in and one copy back;
+        the pipelined host route is not used."""
+        assert k > 0
+        if k > _lib.MAX_K:
+            raise RuntimeError(f"k={k} > {_lib.MAX_K} is not supported by the selection stage")
+        k, n = int(k), self.ntotal
+        nq = x.shape[0] if isinstance(x, torch.Tensor) else np.asarray(x).shape[0]
+        ex = _exclude_arg(exclude, nq)
+        if n == 0 or nq == 0:
+            return self._search_filtered(x, k, D, I, id_map, sel) if sel is not None else self._search(x, k, D, I, id_map)
+        t, from_np = _to_device_f32(x)
+        assert t.shape[1] == self.d
+        dev = t.device
+        sel_mask = []
+
+        def group_search(xg, kq):
+            if sel is not None:
+                return self._search_filtered(xg, kq, None, None, id_map, sel)
+            return self._search(xg, kq, None, None, id_map)
+
+        def long_search(xq, lo, hi, ids_d):
+            if sel is not None and not sel_mask:
+                sel_mask.append(_select(sel, id_map, n, dev))
+            member, keep = _list_member(id_map, n, ids_d, lo, hi, sel_mask[0] if sel_mask else None, dev)
+            Dq, Iq = self._search_small_dev(xq, k, member=member, keep=keep)
+            _map_ids(id_map, Iq)
+            return Dq, Iq
+
+        Dd, Id = _search_excluded(t, k, self.metric_type, ex, group_search, long_search)
+        if from_np or D is not None or I is not None:
+            return _to_host_pair(Dd, Id, D, I)
+        return Dd, Id
 
     def _search_filtered(self, x, k: int, D, I, id_map: torch.Tensor | None, sel):
         """search() over the rows sel selects; sel tests id_map[row] (IndexIDMap) or the row position.
@@ -786,9 +929,12 @@ class IndexIDMap:
         self.index.add(t)
         self.id_map = ids_d if self.id_map is None or self.id_map.numel() == 0 else torch.cat([self.id_map, ids_d])
 
-    def search(self, x, k: int, D=None, I=None, *, params=None):
-        """params: SearchParameters whose sel selects external ids (faiss's IDSelectorTranslated)."""
+    def search(self, x, k: int, D=None, I=None, *, params=None, exclude=None):
+        """params: SearchParameters whose sel selects external ids (faiss's IDSelectorTranslated).
+        exclude: (offsets, ids) CSR lists of external ids, as IndexFlat.search takes them."""
         sel, _ = _search_sel(params, False)
+        if exclude is not None:
+            return self.index._search_exclude(x, k, D, I, self.id_map if self.ntotal else None, sel, exclude)
         if sel is not None:
             return self.index._search_filtered(x, k, D, I, self.id_map if self.ntotal else None, sel)
         return self.index._search(x, k, D, I, self.id_map if self.ntotal else None)
@@ -1125,11 +1271,14 @@ class IndexIVFFlat:
     def list_sizes(self) -> np.ndarray:
         return np.diff(self._build_lists()["offsets_host"])
 
-    def search(self, x, k: int, *, params=None):
+    def search(self, x, k: int, *, params=None, exclude=None):
         """params: SearchParametersIVF. Its sel selects stored ids: the coarse search still ranks
         every centroid, and the scan of the nprobe lists skips the rows sel does not select. Its
-        nprobe, when set, replaces index.nprobe for this call."""
+        nprobe, when set, replaces index.nprobe for this call.
+        exclude: (offsets, ids) CSR lists of stored ids, as IndexFlat.search takes them."""
         sel, nprobe_p = _search_sel(params, True)
+        if exclude is not None:
+            return self._search_exclude(x, k, params, sel, nprobe_p, exclude)
         if not self.is_trained:
             raise RuntimeError("Error: 'is_trained' failed")
         t, from_np = _to_device_f32(x)
@@ -1163,19 +1312,8 @@ class IndexIVFFlat:
                                          (("norms",) if self.metric_type == METRIC_L2 else ())))
             ls = L["packed"].struct()
             if small and nq:
-                # HBM-regime route for small batches: exact fp32 coarse search + row-per-warp list scan
-                _, coarse = self.quantizer._search_small_dev(t, nprobe) if nq < SMALL_NQ else \
-                    self.quantizer.search(t, nprobe)
-                wsb = lib.nrb_ivf_scan_small_workspace(nq, nprobe, L["max_len"], self.ntotal, int(k))
-                ws = torch.empty(wsb, dtype=torch.uint8, device=dev)
-                args = (t.data_ptr(), t.stride(0), nq, self.d, C.byref(ls), L["offsets"].data_ptr(), self.nlist,
-                        L["max_len"], L["ids"].data_ptr(), coarse.data_ptr(), nprobe, self.metric_type, int(k),
-                        D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb, _stream())
-                if sel is None:
-                    check(lib.nrb_ivf_scan_small(*args), "ivf_scan_small")
-                else:
-                    member, keep = _select(sel, L["ids"], self.ntotal, dev)  # list order, like the scan
-                    check(lib.nrb_ivf_scan_small_sel(*args, member.data_ptr(), keep), "ivf_scan_small_sel")
+                self._scan_small(t, int(k), nprobe, L, D, I,
+                                 None if sel is None else _select(sel, L["ids"], self.ntotal, dev))  # list order
                 nq = 0  # done
             for q0 in range(0, nq, IVF_QUERY_BATCH):
                 q1 = min(nq, q0 + IVF_QUERY_BATCH)
@@ -1188,6 +1326,58 @@ class IndexIVFFlat:
                                          L["max_len"], L["ids"].data_ptr(), coarse.data_ptr(), nprobe,
                                          self.metric_type, int(k), D[q0:q1].data_ptr(), I[q0:q1].data_ptr(),
                                          ws.data_ptr(), wsb, self.path, _stream()), "ivf_search")
+        if from_np:
+            return _to_host_pair(D, I)
+        return D, I
+
+    def _scan_small(self, t: torch.Tensor, k: int, nprobe: int, L, D: torch.Tensor, I: torch.Tensor, mask=None):
+        """HBM-regime route for small batches: exact fp32 coarse search + row-per-warp list scan of the
+        lists L into D, I. mask: (member, keep) over the packed list rows, or None (every row)."""
+        nq = t.shape[0]
+        _, coarse = self.quantizer._search_small_dev(t, nprobe) if nq < SMALL_NQ else self.quantizer.search(t, nprobe)
+        wsb = lib.nrb_ivf_scan_small_workspace(nq, nprobe, L["max_len"], self.ntotal, k)
+        ws = torch.empty(wsb, dtype=torch.uint8, device=t.device)
+        ls = L["packed"].struct()
+        args = (t.data_ptr(), t.stride(0), nq, self.d, C.byref(ls), L["offsets"].data_ptr(), self.nlist,
+                L["max_len"], L["ids"].data_ptr(), coarse.data_ptr(), nprobe, self.metric_type, k,
+                D.data_ptr(), I.data_ptr(), ws.data_ptr(), wsb, _stream())
+        if mask is None:
+            check(lib.nrb_ivf_scan_small(*args), "ivf_scan_small")
+        else:
+            check(lib.nrb_ivf_scan_small_sel(*args, mask[0].data_ptr(), mask[1]), "ivf_scan_small_sel")
+
+    def _search_exclude(self, x, k: int, params, sel, nprobe_p, exclude):
+        """search() with per-query exclusion lists (_search_excluded) of stored ids. The long group
+        scans the cached lists with the list's row mask (and sel's) on the small route."""
+        nq = x.shape[0] if isinstance(x, torch.Tensor) else np.asarray(x).shape[0]
+        ex = _exclude_arg(exclude, nq)
+        if not self.is_trained:
+            raise RuntimeError("Error: 'is_trained' failed")
+        assert k > 0
+        k = int(k)
+        nprobe = min(int(self.nprobe if nprobe_p is None else nprobe_p), self.nlist)
+        if k > _lib.MAX_K or nprobe > _lib.MAX_K:
+            raise RuntimeError(f"k / nprobe > {_lib.MAX_K} is not supported by the selection stage")
+        t, from_np = _to_device_f32(x)
+        assert t.shape[1] == self.d
+        dev = t.device
+        if self.ntotal == 0 or nq == 0:
+            D, I = self.search(t, k, params=params)
+        else:
+            sel_mask = []
+
+            def long_search(xq, lo, hi, ids_d):
+                L = self._build_lists()
+                if sel is not None and not sel_mask:
+                    sel_mask.append(_select(sel, L["ids"], self.ntotal, dev))
+                mask = _list_member(L["ids"], self.ntotal, ids_d, lo, hi, sel_mask[0] if sel_mask else None, dev)
+                Dq = torch.empty((1, k), dtype=torch.float32, device=dev)
+                Iq = torch.empty((1, k), dtype=torch.int64, device=dev)
+                self._scan_small(xq, k, nprobe, L, Dq, Iq, mask)
+                return Dq, Iq
+
+            D, I = _search_excluded(t, k, self.metric_type, ex,
+                                    lambda xg, kq: self.search(xg, kq, params=params), long_search)
         if from_np:
             return _to_host_pair(D, I)
         return D, I

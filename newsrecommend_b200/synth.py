@@ -35,10 +35,12 @@ def g_skew(n: int, d: int, seed: int, n_topics: int = 461, r: int = 16, zipf: fl
 
 
 def user_profiles(items: np.ndarray, topics: np.ndarray | None, n_users: int, seed: int,
-                  mean_clicks: float = 6.5, max_clicks: int = 64) -> np.ndarray:
+                  mean_clicks: float = 6.5, max_clicks: int = 64, return_clicks: bool = False):
     """Mean of L clicked item rows, L ~ clip(Geometric(1/mean_clicks), 1, max_clicks); 70 % of a
     user's clicks come from one topic, 30 % uniformly (the dataset has ~6.5 clicks per user,
-    others/data_analysis.ipynb:1868,1981)."""
+    others/data_analysis.ipynb:1868,1981). return_clicks: also return the click history as CSR,
+    (offsets i64[n_users+1], clicked rows i64), user u's clicks being rows[offsets[u]:offsets[u+1]]
+    (a row clicked twice appears twice); the profiles are the same either way."""
     rng = np.random.default_rng(seed)
     n = items.shape[0]
     L = np.clip(rng.geometric(1.0 / mean_clicks, size=n_users), 1, max_clicks)
@@ -60,4 +62,8 @@ def user_profiles(items: np.ndarray, topics: np.ndarray | None, n_users: int, se
     out = np.zeros((n_users, items.shape[1]), dtype=np.float32)
     np.add.at(out, owner, items[picks])
     out /= L[:, None].astype(np.float32)
+    if return_clicks:
+        offsets = np.zeros(n_users + 1, dtype=np.int64)
+        np.cumsum(L, out=offsets[1:])
+        return out, (offsets, picks.astype(np.int64, copy=False))
     return out
