@@ -333,6 +333,18 @@ int nrb_exclude_topk(const float* Din, const int64_t* Iin, int64_t nrows, int32_
                      const int64_t* excl_off, const int64_t* excl_ids, int32_t metric, int32_t k,
                      float* D, int64_t* I, void* stream);
 
+/* Stable compaction of CSR lists: off i64[nrows+1] (off[0] = 0, off[nrows] = nids) over ids i64[nids].
+ * Entry i is kept when member[i] == 1 (what nrb_id_select wrote over the list ids) and written as
+ * ids[i] - shift; out_off i64[nrows+1] are the kept lists' offsets, out_ids (room for nids) their
+ * entries, in the input order within each row. Deterministic. ids, member and out_ids may be NULL
+ * when nids == 0; nrows == 0 writes out_off[0] = 0. The sharded indexes use it to keep the part of
+ * per-query exclusion lists a shard holds, in the shard's label space.
+ * Workspace: nrb_csr_compact_workspace(nrows) bytes. */
+size_t nrb_csr_compact_workspace(int64_t nrows);
+int nrb_csr_compact(const int64_t* off, const int64_t* ids, int64_t nrows, int64_t nids, const int64_t* member,
+                    int64_t shift, int64_t* out_off, int64_t* out_ids, void* workspace, size_t workspace_bytes,
+                    void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -37,6 +37,7 @@ SYMBOLS = [
     "nrb_id_select_workspace", "nrb_id_select", "nrb_map_ids",
     "nrb_search_small_sel", "nrb_search_small_host_sel", "nrb_ivf_scan_small_sel", "nrb_sel_keys",
     "nrb_pack_topk_ids", "nrb_merge_topk_packed_ids", "nrb_exclude_topk",
+    "nrb_csr_compact_workspace", "nrb_csr_compact",
 ]
 
 
@@ -116,6 +117,9 @@ lib.nrb_sel_keys.argtypes = [_vp, _i64, _vp, _i64, _i64, _vp, _vp]
 lib.nrb_pack_topk_ids.argtypes = [_vp, _vp, _i64, _vp, _vp]
 lib.nrb_merge_topk_packed_ids.argtypes = [_vp, _i32, _i64, _i32, _i32, _vp, _vp, _vp]
 lib.nrb_exclude_topk.argtypes = [_vp, _vp, _i64, _i32, _vp, _vp, _vp, _i32, _i32, _vp, _vp, _vp]
+lib.nrb_csr_compact_workspace.restype = _sz
+lib.nrb_csr_compact_workspace.argtypes = [_i64]
+lib.nrb_csr_compact.argtypes = [_vp, _vp, _i64, _i64, _vp, _i64, _vp, _vp, _vp, _sz, _vp]
 
 
 def last_error() -> str:

@@ -1809,3 +1809,142 @@ extern "C" int nrb_exclude_topk(const float* Din, const int64_t* Iin, int64_t nr
     NRB_LAUNCH_CHECK();
     return NRB_OK;
 }
+
+// ------------------------------------------------------------------- CSR list compaction
+// The part of per-query exclusion lists that one shard holds: entry i of row r survives when
+// member[i] == 1 (what nrb_id_select wrote over the list ids) and is written as ids[i] - shift, in
+// order. Three launches, no atomics, so the result is deterministic: (1) a warp per row counts its
+// survivors by ballot and each block sums its CC_ROWS rows, (2) one block scans the block sums,
+// (3) each block scans its rows' counts into offsets and a warp per row scatters its survivors with a
+// ballot prefix.
+constexpr int CC_WARPS = 8;
+constexpr int CC_ROWS = CC_WARPS * 32;  // rows per block; the scatter kernel scans one count per thread
+
+// Exclusive scan of one int64 per thread over a block of NT threads; *total = the block's sum.
+template <int NT>
+__device__ __forceinline__ int64_t cc_block_scan(int64_t v, int64_t* wsum, int64_t* total) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    int64_t x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int64_t y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= o) x += y;
+    }
+    if (lane == 31) wsum[w] = x;
+    __syncthreads();
+    if (w == 0) {
+        int64_t s = lane < NT / 32 ? wsum[lane] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int64_t y = __shfl_up_sync(0xffffffffu, s, o);
+            if (lane >= o) s += y;
+        }
+        if (lane < NT / 32) wsum[lane] = s;
+    }
+    __syncthreads();
+    const int64_t excl = (w ? wsum[w - 1] : 0) + x - v;
+    *total = wsum[NT / 32 - 1];
+    __syncthreads();  // wsum is reused by the next call
+    return excl;
+}
+
+// out_off[r + 1] = kept entries of row r; block_sum[b] = kept entries of block b's rows
+__global__ void __launch_bounds__(CC_ROWS)
+csr_compact_count_kernel(const int64_t* __restrict__ off, const int64_t* __restrict__ member, int64_t nrows,
+                         int64_t* __restrict__ out_off, int64_t* __restrict__ block_sum) {
+    __shared__ int64_t wsum[CC_WARPS];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t r0 = (int64_t)blockIdx.x * CC_ROWS;
+    int64_t tot = 0;
+    for (int j = w; j < CC_ROWS && r0 + j < nrows; j += CC_WARPS) {
+        const int64_t b = off[r0 + j], e = off[r0 + j + 1];
+        int64_t c = 0;
+        for (int64_t i = b; i < e; i += 32) c += __popc(__ballot_sync(0xffffffffu, i + lane < e && member[i + lane] == 1));
+        if (lane == 0) out_off[r0 + j + 1] = c;
+        tot += c;
+    }
+    if (lane == 0) wsum[w] = tot;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int64_t s = 0;
+        for (int i = 0; i < CC_WARPS; i++) s += wsum[i];
+        block_sum[blockIdx.x] = s;
+    }
+}
+
+// block_sum[0 .. nblocks) -> its exclusive prefix sums, in place (one block)
+__global__ void __launch_bounds__(1024) csr_compact_scan_kernel(int64_t* __restrict__ block_sum, int64_t nblocks) {
+    __shared__ int64_t wsum[32];
+    int64_t carry = 0;
+    for (int64_t t0 = 0; t0 < nblocks; t0 += 1024) {
+        const int64_t i = t0 + threadIdx.x;
+        int64_t tot;
+        const int64_t p = cc_block_scan<1024>(i < nblocks ? block_sum[i] : 0, wsum, &tot);
+        if (i < nblocks) block_sum[i] = carry + p;
+        carry += tot;
+    }
+}
+
+__global__ void __launch_bounds__(CC_ROWS)
+csr_compact_scatter_kernel(const int64_t* __restrict__ off, const int64_t* __restrict__ ids,
+                           const int64_t* __restrict__ member, int64_t nrows, int64_t shift,
+                           const int64_t* __restrict__ block_base, int64_t* __restrict__ out_off,
+                           int64_t* __restrict__ out_ids) {
+    __shared__ int64_t wsum[CC_WARPS];
+    __shared__ int64_t start[CC_ROWS];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t r0 = (int64_t)blockIdx.x * CC_ROWS, r = r0 + threadIdx.x;
+    const int64_t c = r < nrows ? out_off[r + 1] : 0;  // this row's count, from the count kernel
+    int64_t tot;
+    const int64_t s = block_base[blockIdx.x] + cc_block_scan<CC_ROWS>(c, wsum, &tot);
+    start[threadIdx.x] = s;
+    if (r < nrows) out_off[r + 1] = s + c;
+    if (r == 0) out_off[0] = 0;
+    __syncthreads();
+    const unsigned below = (1u << lane) - 1u;
+    for (int j = w; j < CC_ROWS && r0 + j < nrows; j += CC_WARPS) {
+        const int64_t b = off[r0 + j], e = off[r0 + j + 1];
+        int64_t pos = start[j];
+        for (int64_t i = b; i < e; i += 32) {
+            const bool keep = i + lane < e && member[i + lane] == 1;
+            const unsigned m = __ballot_sync(0xffffffffu, keep);
+            if (keep) out_ids[pos + __popc(m & below)] = ids[i + lane] - shift;
+            pos += __popc(m);
+        }
+    }
+}
+
+extern "C" size_t nrb_csr_compact_workspace(int64_t nrows) {
+    return nrows > 0 ? (size_t)((nrows + CC_ROWS - 1) / CC_ROWS) * sizeof(int64_t) : 0;
+}
+
+extern "C" int nrb_csr_compact(const int64_t* off, const int64_t* ids, int64_t nrows, int64_t nids,
+                               const int64_t* member, int64_t shift, int64_t* out_off, int64_t* out_ids,
+                               void* workspace, size_t workspace_bytes, void* stream) {
+    NRB_REQUIRE(nrows >= 0 && nrows < (1LL << 38) && nids >= 0, "csr_compact: bad sizes nrows=%lld nids=%lld", (long long)nrows,
+                (long long)nids);
+    NRB_REQUIRE(off && out_off, "csr_compact: null offsets");
+    NRB_REQUIRE(nids == 0 || (ids && member && out_ids), "csr_compact: null argument");
+    const size_t need = nrb_csr_compact_workspace(nrows);
+    if (workspace_bytes < need || (need && !workspace)) {
+        set_error("csr_compact: workspace %zu < %zu", workspace_bytes, need);
+        return NRB_ERR_WORKSPACE;
+    }
+    int rc = require_device();
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (nrows == 0) {
+        NRB_CUDA_CHECK(cudaMemsetAsync(out_off, 0, sizeof(int64_t), st));
+        return NRB_OK;
+    }
+    const int64_t nblocks = (nrows + CC_ROWS - 1) / CC_ROWS;
+    int64_t* block_sum = (int64_t*)workspace;
+    csr_compact_count_kernel<<<(unsigned)nblocks, CC_ROWS, 0, st>>>(off, member, nrows, out_off, block_sum);
+    NRB_LAUNCH_CHECK();
+    csr_compact_scan_kernel<<<1, 1024, 0, st>>>(block_sum, nblocks);
+    NRB_LAUNCH_CHECK();
+    csr_compact_scatter_kernel<<<(unsigned)nblocks, CC_ROWS, 0, st>>>(off, ids, member, nrows, shift, block_sum,
+                                                                       out_off, out_ids);
+    NRB_LAUNCH_CHECK();
+    return NRB_OK;
+}

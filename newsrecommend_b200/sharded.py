@@ -27,8 +27,14 @@ ties merge in rank order: after one add_with_ids call that is row order, as in t
 after several calls rank 0's later rows come before rank 1's earlier ones, where the single index
 keeps insertion order.
 
-Host logic only; `make_index` / `make_idmap` (per-rank index) and `codec` (pack / merge) are
-injectable so that the same code runs under gloo on CPU with the oracle index and numpy stand-ins
+Per-query exclusion lists (search(..., exclude=(offsets, ids)), labels as for selectors): every rank
+passes the same lists, keeps only the entries that name its own rows, moved into its local label
+space (`localize`: nrb_id_select + nrb_csr_compact, once per call), and runs the single-GPU excluded
+search on its shard. A shard then over-fetches by the listed ids it holds, not by the whole list.
+The per-shard results are exact, so the merge is unchanged.
+
+Host logic only; `make_index` / `make_idmap` (per-rank index) and `codec` (pack / merge / localize)
+are injectable so that the same code runs under gloo on CPU with the oracle index and numpy stand-ins
 (tests/).
 """
 from __future__ import annotations
@@ -106,8 +112,47 @@ class GpuCodec:
                                             torch.cuda.current_stream().cuda_stream), "merge_topk_packed_ids")
         return D, I
 
+    @staticmethod
+    def localize(ex, held, shift: int, dev):
+        """The part of the exclusion lists ex (what faiss._exclude_arg returned) that this rank holds, in
+        its local label space. held: (lo, hi), the range of labels the rank's rows carry, or an i64
+        tensor of its stored ids (None when it has none). An entry held names is kept, as ids[i] - shift,
+        in order (nrb_id_select, then nrb_csr_compact). Returns (offsets as a host i64 array, ids as a
+        device tensor); the offsets' copy to the host is the call's one synchronisation."""
+        from ._lib import check, lib
+        from .faiss import _exclude_to_device
+        off_h = ex[0]
+        nq, n = off_h.shape[0] - 1, int(off_h[-1])
+        st = torch.cuda.current_stream().cuda_stream
+        off_d, ids_d = _exclude_to_device(*ex, dev)
+        member = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+        if isinstance(held, tuple):
+            check(lib.nrb_id_select(ids_d.data_ptr(), n, None, 0, held[0], held[1], member.data_ptr(), None, 0, st),
+                  "id_select")
+        else:
+            nb = 0 if held is None else held.numel()
+            wsb = lib.nrb_id_select_workspace(nb)
+            ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device=dev)
+            check(lib.nrb_id_select(ids_d.data_ptr(), n, held.data_ptr() if nb else None, nb, 0, 0, member.data_ptr(),
+                                    ws.data_ptr(), wsb, st), "id_select")
+        out_off = torch.empty(nq + 1, dtype=torch.int64, device=dev)
+        out_ids = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
+        wsb = lib.nrb_csr_compact_workspace(nq)
+        ws = torch.empty(max(wsb, 1), dtype=torch.uint8, device=dev)
+        check(lib.nrb_csr_compact(off_d.data_ptr(), ids_d.data_ptr(), nq, n, member.data_ptr(), shift, out_off.data_ptr(),
+                                  out_ids.data_ptr(), ws.data_ptr(), wsb, st), "csr_compact")
+        loc_off = out_off.cpu().numpy()
+        return loc_off, out_ids[: int(loc_off[-1])]
+
 
 _I64_MIN, _I64_MAX = -(1 << 63), (1 << 63) - 1
+
+
+def chunk_lists(lists, c0: int, c1: int):
+    """Queries [c0, c1) of localized CSR lists (host offsets, ids): offsets rebased to 0, a view of the ids."""
+    off, ids = lists
+    a, b = int(off[c0]), int(off[c1])
+    return off[c0:c1 + 1] - a, ids[a:b]
 
 
 def shift_selector(sel, base: int):
@@ -204,18 +249,38 @@ class _ShardedSearch:
     def _pack(self, D: torch.Tensor, I: torch.Tensor) -> torch.Tensor:
         return self.codec.pack_ids(D, I) if self.with_ids else self.codec.pack(D, I, self.id_base)
 
+    def _held(self):
+        """(held, shift) for codec.localize: which exclusion-list entries name this rank's rows, and
+        what moves them into its local label space."""
+        raise NotImplementedError
+
+    def _localize(self, exclude, nq: int):
+        """exclude=(offsets, ids) checked and cut down to this rank's entries (codec.localize), or None.
+        Every rank passes the same lists, so a malformed pair raises the same error on every rank,
+        before any device work or collective."""
+        if exclude is None:
+            return None
+        from .faiss import _exclude_arg
+        ex = _exclude_arg(exclude, nq)
+        held, shift = self._held()
+        return self.codec.localize(ex, held, shift, self._dev())
+
     def _merge(self, recv: torch.Tensor):
         if self.with_ids:
             return self.codec.merge_ids(recv, self.metric_type)
         return self.codec.merge(recv, self._bases(), self.metric_type)
 
-    def _local_search(self, xq, k: int, params):
+    def _local_search(self, xq, k: int, params, exclude=None):
         """The rank-local index's search (CUDA tensors, or ndarrays on the CPU test path) as tensors,
-        labels made global: external ids as they are, local positions + id_base."""
+        labels made global: external ids as they are, local positions + id_base. exclude: this chunk's
+        localized lists, or None."""
+        kw = {} if exclude is None else {"exclude": exclude}
         if self._cuda_index:
-            D, I = self.local.search(xq, k, params=params)
+            D, I = self.local.search(xq, k, params=params, **kw)
         else:
-            D, I = self.local.search(np.ascontiguousarray(xq), k, **({} if params is None else {"params": params}))
+            if params is not None:
+                kw["params"] = params
+            D, I = self.local.search(np.ascontiguousarray(xq), k, **kw)
             D, I = torch.as_tensor(D), torch.as_tensor(I)
         if self.with_ids:
             return D, I
@@ -254,9 +319,10 @@ class _ShardedSearch:
         return 1 << 17
 
     # ------------------------------------------------------------------ search pieces
-    def search_local(self, xq, k: int, params=None):
+    def search_local(self, xq, k: int, params=None, exclude=None):
         """Per-shard top-k of a raw query chunk with GLOBAL ids: (D f32[n,k], I i64[n,k]) tensors.
-        params: what _local_params made of the caller's search parameters."""
+        params: what _local_params made of the caller's search parameters. exclude: the chunk's
+        exclusion lists already localized to this rank (local labels), as (offsets, ids)."""
         raise NotImplementedError
 
     def _exchange_start(self, P: torch.Tensor, per: int):
@@ -277,15 +343,18 @@ class _ShardedSearch:
         work = dist.all_to_all_single(recv, P, [mine] * G, in_rows, group=self.group, async_op=True)
         return recv.view((G, mine) + tail), work
 
-    def search(self, xq, k: int, gather: bool = True, *, params=None):
+    def search(self, xq, k: int, gather: bool = True, *, params=None, exclude=None):
         """xq: the FULL query batch on every rank (CUDA tensor fp32 [nq, d]; ndarray on the CPU test
         path). gather=True: (D, I) of all queries on every rank (a final all-gather of the merged
         slices). gather=False: the merged results of this rank's own rows only, as
         (D, I, spans) with spans = owned_rows(nq, ...). params: as the single index of the same kind
         takes them (SearchParameters / SearchParametersIVF); when fewer than k rows qualify across
-        all shards the tail is I = -1, D = -FLT_MAX (IP) / +FLT_MAX (L2)."""
+        all shards the tail is I = -1, D = -FLT_MAX (IP) / +FLT_MAX (L2). exclude: (offsets i64[nq+1],
+        ids i64) CSR lists, numpy or tensors, the same on every rank; query q returns no label in
+        ids[offsets[q]:offsets[q+1]] (labels as params' selectors test them)."""
         lp = self._local_params(params)
         nq = xq.shape[0]
+        lists = self._localize(exclude, nq)
         G = self.world
         chunk = self._chunk()
         pending = None
@@ -298,7 +367,7 @@ class _ShardedSearch:
             parts.append(self._merge(recv))
 
         for c0, c1, per in chunk_slices(nq, G, chunk):
-            D, I = self.search_local(xq[c0:c1], k, lp)
+            D, I = self.search_local(xq[c0:c1], k, lp, None if lists is None else chunk_lists(lists, c0, c1))
             P = self._pack(D, I)
             nxt = self._exchange_start(P, per)
             if pending is not None:
@@ -343,16 +412,18 @@ class _ShardedSearch:
         return D, I
 
     # ------------------------------------------------------------------ end to end from host memory
-    def search_host(self, xq_host: np.ndarray, k: int, D_out: np.ndarray, I_out: np.ndarray, *, params=None):
+    def search_host(self, xq_host: np.ndarray, k: int, D_out: np.ndarray, I_out: np.ndarray, *, params=None,
+                    exclude=None):
         """The call a user of the sharded index makes with HOST arrays: every rank passes the same
         page-locked fp32 [nq, d] batch and the same-shaped output arrays; each rank copies only ITS
         rows host-to-device (1/G of the batch), the ranks all-gather the query rows over NVLink,
         search, exchange, merge, and each rank copies the results of its own rows back into
         D_out / I_out (rows owned by other ranks are left untouched). Returns the owned spans.
-        params: as search() takes them."""
+        params, exclude: as search() takes them; every rank copies the whole list pair to its device."""
         assert self._cuda_index, "search_host is the CUDA path"
         lp = self._local_params(params)
         nq, d = xq_host.shape
+        lists = self._localize(exclude, nq)
         G, r = self.world, self.rank
         dev = self._dev()
         chunk = self._chunk()
@@ -386,7 +457,7 @@ class _ShardedSearch:
                 dist.all_gather_into_tensor(full, mine, group=self.group)
             else:
                 full = mine
-            D, I = self.search_local(full[: c1 - c0], k, lp)
+            D, I = self.search_local(full[: c1 - c0], k, lp, None if lists is None else chunk_lists(lists, c0, c1))
             P = self._pack(D, I)
             recv, work = self._exchange_start(P, per)
             if pending is not None:
@@ -454,12 +525,17 @@ class ShardedIndexFlat(_ShardedSearch):
             return None
         return SearchParameters(sel=sel if self.with_ids else shift_selector(sel, self.id_base))
 
-    def search_local(self, xq, k: int, params=None):
-        if self._cuda_index and params is None and not self.with_ids:
+    def _held(self):
+        if self.with_ids:
+            return self.local.id_map, 0
+        return (self.id_base, self.id_base + self.local.ntotal), self.id_base  # global row positions
+
+    def search_local(self, xq, k: int, params=None, exclude=None):
+        if self._cuda_index and params is None and exclude is None and not self.with_ids:
             from .faiss import PackedMatrix
             q = PackedMatrix.from_tensor(xq, planes=self.local._query_planes(k))  # K0 on the fresh chunk
             return self.local.search_packed(q, k, self.id_base)
-        return self._local_search(xq, k, params)
+        return self._local_search(xq, k, params, exclude)
 
 
 # ------------------------------------------------------------------------------------ sharded IVF
@@ -621,6 +697,7 @@ class ShardedIndexIVFFlat(_ShardedSearch):
         self.cp = self.local.cp
         self._kmeans_ops = kmeans_ops
         self.iteration_stats = []
+        self._pos_end = 0  # plain index: end of the global positions this rank was given at add time
 
     @property
     def is_trained(self) -> bool:
@@ -677,6 +754,7 @@ class ShardedIndexIVFFlat(_ShardedSearch):
         lo, hi = shard_range(nb, self.world, self.rank)
         self.id_base = lo
         self.local.add(x[lo:hi])
+        self._pos_end = hi
         self.ntotal = nb
         self._set_bases_global(nb)
 
@@ -685,8 +763,15 @@ class ShardedIndexIVFFlat(_ShardedSearch):
         assert self.ntotal == 0, "add_local is a one-shot build"
         self.id_base = int(id_base)
         self.local.add(x_local)
+        self._pos_end = self.id_base + self.local.ntotal
         self.ntotal = int(ntotal)
         self._set_bases_gathered()
+
+    def _held(self):
+        if self.with_ids:
+            return self.local._ids, 0
+        # stored ids are the positions given at add time; a removed row's position matches nothing
+        return (self.id_base, self._pos_end), self.id_base
 
     def _local_params(self, params):
         from .faiss import SearchParametersIVF, _search_sel
@@ -697,6 +782,6 @@ class ShardedIndexIVFFlat(_ShardedSearch):
             sel = shift_selector(sel, self.id_base)  # stored ids are local positions
         return SearchParametersIVF(sel=sel, nprobe=nprobe)
 
-    def search_local(self, xq, k: int, params=None):
+    def search_local(self, xq, k: int, params=None, exclude=None):
         self.local.nprobe = self.nprobe
-        return self._local_search(xq, k, params)  # plain: stored ids = local insertion rows
+        return self._local_search(xq, k, params, exclude)  # plain: stored ids = local insertion rows
